@@ -6,6 +6,7 @@
 
     python bench.py --config 4 --gpus N ...                        # BASELINE.json configs[3]: 1 M envs + imitation reward
     python bench.py --config 5 --gpus N ...                        # BASELINE.json configs[4]: 8 x (1024 x 4), 512 Ki envs/GPU
+    python bench.py ... --dump-outputs DIR                         # also write the last timed step's outputs as DIR/*.npy
 
 One "step" = one pass of the hot path over one batch of synthetic input.  The default workload (--config 2) is
 BASELINE.json configs[1], the MILO rollout batch of samples_per_step = 40 000 learned-dynamics env-steps per GPU
@@ -20,6 +21,12 @@ same work through the host-buffer API with pinned H2D/D2H copies inside the time
 ensemble layer GEMM against the measured tensor peak (burst AND sustained denominators), `sustained` repeats the
 timed loop for >= 2 s, `cpu_baseline` is the oracle port of the reference's PyTorch CPU path timed on this box's
 host cores on a bounded sample.
+
+--dump-outputs DIR writes what the timed path handed its caller in the last timed step (rank 0's envs): next_state,
+disc, done, cost, ipm, bonus and the updated num_steps of the env step, imitation_reward with --config 3 / 4, and with
+--config 4 / 5 disc_quantile, the global 0.9 quantile of that step's disc (taken after the timed loop).  Inputs are
+seeded, so two builds run with the same arguments can be compared array for array.  See dump_outputs for the format and
+the 64 MB cap.
 """
 import argparse
 import json
@@ -430,6 +437,32 @@ def pcie_probe(device, nbytes=36 << 20, reps=10):
     return nbytes * reps / (time.perf_counter() - t0) / 1e9
 
 
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, per_env, scalars=None, limit=DUMP_LIMIT_BYTES):
+    """Writes per_env's tensors (first dimension = env) as out_dir/<name>.npy: floating outputs as float32, integer
+    ones (done, num_steps) as float64.  When they exceed `limit` bytes together, every array keeps the same rows, a
+    sorted sample drawn with a fixed seed, and rows.npy holds their indices.  scalars are written as 1-element float64
+    arrays."""
+    import numpy as np
+    import torch
+    n = next(iter(per_env.values())).shape[0]
+    row_bytes = sum((t[0].numel() if t.dim() > 1 else 1) * (4 if t.is_floating_point() else 8) for t in per_env.values())
+    os.makedirs(out_dir, exist_ok=True)
+    rows = None
+    if n * row_bytes > limit:
+        keep = (limit - 65536) // (row_bytes + 8)   # rows.npy and the .npy headers fit in the 64 KiB kept back
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        np.save(os.path.join(out_dir, "rows.npy"), rows.numpy().astype(np.float64))
+    for name, t in per_env.items():
+        t = t.detach() if rows is None else t.detach()[rows.to(t.device)]
+        t = t.float() if t.is_floating_point() else t.double()
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+    for name, v in (scalars or {}).items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.array([v], dtype=np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -586,6 +619,19 @@ def run_ours(args):
     t_wall1 = time.time()
     launches = _lib.launch_count() - launches0
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
+    if args.dump_outputs:   # now: the passes below write into the same output buffers
+        o = (args.warmup + args.steps - 1) % oring
+        scalars = {}
+        if q_every and step_on:   # a collective: every rank takes part
+            scalars["disc_quantile"] = float(parallel.global_quantile(disc[o], 0.9, engine=eng))
+        if rank == 0:
+            per_env = {}
+            if step_on:
+                per_env.update(next_state=nxt, disc=disc[o], done=done, cost=cst[o], ipm=ipm, bonus=bonus,
+                               num_steps=steps)
+            if imit is not None:
+                per_env["imitation_reward"] = rew
+            dump_outputs(args.dump_outputs, per_env, scalars)
     e_total = torch.tensor([float(E)], device=device, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(e_total, op=dist.ReduceOp.SUM)
@@ -937,8 +983,9 @@ def plugin_single_env(ens, ds, device, n=200):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=500)
-    ap.add_argument("--warmup", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 500; 30 with --config 4 / 5)")
+    ap.add_argument("--warmup", type=int, default=None, help="untimed steps first, at least 3 (default: 20; 5 with "
+                                                              "--config 4 / 5)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", type=int, default=2, choices=sorted(CONFIGS),
                     help="BASELINE.json workload, 1-based: 2 = configs[1] (default, the headline), 3 = imitation only, "
@@ -953,11 +1000,20 @@ def main():
     ap.add_argument("--rff-split", default="auto", choices=["auto", "on", "off"],
                     help="hi/lo operand pairs in the cost-feature GEMM: measured decision (auto), always, never")
     ap.add_argument("--graph-check", action="store_true", help="also time the steps replayed from CUDA graphs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (at most 64 MB in all)")
     args = ap.parse_args()
+    long_steps = args.config in (4, 5)  # a step is 20-60 ms here
+    if args.steps is None:
+        args.steps = 30 if long_steps else 500
+    if args.warmup is None:
+        args.warmup = 5 if long_steps else 20
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
-    if args.config in (4, 5) and args.steps == 500:
-        args.steps, args.warmup = 30, max(3, min(args.warmup, 5))  # a step is 20-60 ms here
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA path's outputs (--impl ours)")
     # The contract is ONE JSON line on stdout.  Libraries write there too (NCCL prints its version banner on
     # stdout when NCCL_DEBUG is set on the box), so file descriptor 1 is pointed at stderr for the duration of the
     # run and the JSON line goes to the original stdout.

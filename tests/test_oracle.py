@@ -8,6 +8,21 @@ import torch
 from oracle import milo_oracle as mo
 from tests import helpers as H
 
+GOLDEN_THREADS = 8
+
+
+@pytest.fixture(autouse=True, scope="module")
+def golden_thread_count():
+    """The float32 golden vectors were written with GOLDEN_THREADS torch intra-op threads.  The CPU GEMM (MKL) splits
+    its sums by thread count, so the same ops reproduce the stored bits only with that count, whatever the host's
+    number of cores.  The bits also depend on the MKL build and on the instruction set its kernels use (they are
+    reproduced by the MKL that torch 2.11 ships, on AVX-512); pinning the thread count removes only the core-count
+    dependence."""
+    before = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(before)
+
 
 @pytest.mark.parametrize("tag", ["tiny_dense", "tiny_plain_tanh"])
 def test_forward_and_discrepancy_match_reference(tag):

@@ -126,6 +126,16 @@ _SIGNATURES = {
     "simstep_train_loss": (C.c_int, [_c_void_p, _c_void_p, _c_void_p, _c_void_p, C.c_int32, _c_void_p, _c_void_p]),
     "simstep_train_grads": (C.c_int, [_c_void_p, _c_void_p, _c_void_p, _c_void_p, C.c_int32, _c_void_p, _c_void_p]),
     "simstep_train_export": (C.c_int, [_c_void_p, C.c_int32, C.POINTER(_c_void_p), C.POINTER(_c_void_p)]),
+    "simstep_npg_init": (C.c_int, [_c_void_p, C.c_float, C.POINTER(C.c_int64)]),
+    "simstep_npg_params": (C.c_int, [_c_void_p, C.c_int32, _c_void_p, _c_void_p]),
+    "simstep_npg_grad": (C.c_int, [_c_void_p, _c_void_p, _c_void_p, _c_void_p, _c_void_p, C.c_int64, _c_void_p, _c_void_p]),
+    "simstep_npg_prepare": (C.c_int, [_c_void_p, _c_void_p, C.c_int64, _c_void_p, C.c_int64, _c_void_p]),
+    "simstep_npg_fvp": (C.c_int, [_c_void_p, _c_void_p, _c_void_p, C.c_int64, _c_void_p, C.c_int64, _c_void_p, _c_void_p,
+                                  _c_void_p]),
+    "simstep_npg_cg": (C.c_int, [_c_void_p, C.c_int32, _c_void_p, C.c_double, _c_void_p]),
+    "simstep_npg_apply": (C.c_int, [_c_void_p, C.c_double, C.c_int32, _c_void_p]),
+    "simstep_npg_diag": (C.c_int, [_c_void_p, _c_void_p, _c_void_p, _c_void_p, _c_void_p, C.c_int64, _c_void_p, _c_void_p]),
+    "simstep_npg_scalars": (C.c_int, [_c_void_p, _c_void_p, _c_void_p]),
     "simstep_histogram": (C.c_int, [_c_void_p, _c_void_p, C.c_int64, C.c_double, C.c_double, C.c_int32, _c_void_p,
                                     _c_void_p]),
     "simstep_quantile_op": (C.c_int, [_c_void_p, C.c_int32, _c_void_p, C.c_int64, C.c_int32, _c_void_p, _c_void_p,

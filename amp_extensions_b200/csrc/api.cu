@@ -20,6 +20,7 @@
 #include "chain_launch.h"
 #include "imitation.cuh"
 #include "imitation_h3d.cuh"
+#include "npg.cuh"
 #include "policy.cuh"
 #include "post_tma.cuh"
 #include "train.cuh"
@@ -106,6 +107,7 @@ struct simstep_handle {
   ImitConst* imit_dev = nullptr;
   void* policy = nullptr;  // PolicyStore (policy_api.inc)
   void* train = nullptr;   // TrainStore (train_api.inc)
+  void* npg = nullptr;     // NpgStore (npg_api.inc)
   bool train_raw = false;  // tf32 handle in training: parameters keep all fp32 bits (they are the master copy)
   bool have_clip = false;
   int dof = 0;
@@ -975,6 +977,7 @@ int upload_layer(simstep_handle* h, int l, const float* const* weights_host, con
 void free_clip(simstep_handle* h);
 void free_policy(simstep_handle* h);
 void free_train(simstep_handle* h);
+void free_npg(simstep_handle* h);
 
 // A handle's buffers, tensor maps and kernel attributes belong to the device it was created on; work can only be
 // enqueued from a thread whose current device is that one (one process per GPU does this by construction).
@@ -1114,6 +1117,7 @@ int simstep_destroy(simstep_handle* h) {
   cudaFree(h->rff_wpad);
   cudaFree(h->colsum_partial);
   free_clip(h);
+  free_npg(h);
   free_policy(h);
   free_train(h);
   delete h;
@@ -1690,3 +1694,4 @@ int simstep_debug_gemm(int32_t precision, int32_t groups, int64_t m, int32_t n, 
 #include "imitation_api.inc"
 #include "policy_api.inc"
 #include "train_api.inc"
+#include "npg_api.inc"

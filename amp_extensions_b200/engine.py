@@ -134,6 +134,8 @@ class Engine:
         # bumped by every call that re-allocates device parameters or changes what the step's launches bake in
         # (load_* / set_*): captured CUDA graphs of an older generation must not be replayed
         self.generation = 0
+        # bumped by load_policy only: it replaces the policy's device parameters and discards the NPG state
+        self.policy_generation = 0
 
     # -- lifetime -----------------------------------------------------------------------
     def close(self):
@@ -435,6 +437,7 @@ class Engine:
             self._check(self.lib.simstep_load_policy(self._h, nl, lin, lout, wp, bp, int(nonlinearity == "tanh"),
                                                      *[_ptr(x) for x in extra]))
             self.generation += 1
+            self.policy_generation += 1
         self.policy_obs_dim, self.policy_act_dim = int(ws[0].shape[1]), int(ws[-1].shape[0])
 
     def policy_act(self, obs, noise=None, action=None, mean=None, want_mean=True):
@@ -480,6 +483,84 @@ class Engine:
         out = torch.empty_like(x) if out is None else out
         self._check(self.lib.simstep_whiten(self._h, _ptr(x), _ptr(valid), x.numel(), _ptr(stats), float(eps), _ptr(out),
                                             _stream(self.device)))
+        return out
+
+    # -- natural policy gradient step of the loaded policy (simstep_npg_*) ----------------
+    NPG_CG_START, NPG_CG_STEP = 0, 1
+
+    def npg_init(self, min_log_std=-3.0):
+        """Allocate the NPG state of the loaded policy; returns P, the length of its parameter vector."""
+        n = C.c_int64(0)
+        with torch.cuda.device(self.device):
+            self._check(self.lib.simstep_npg_init(self._h, float(min_log_std), C.byref(n)))
+        self.npg_n_params = int(n.value)
+        return self.npg_n_params
+
+    def _npg_rows(self, t, name, dtype=torch.float32):
+        """Row tensors of the simstep_npg_* calls cross the ABI as raw device pointers: refuse anything else."""
+        if t is None:
+            return
+        if not (torch.is_tensor(t) and t.dtype == dtype and t.device == self.device and t.is_contiguous()):
+            raise TypeError(f"{name} must be a contiguous {dtype} tensor on {self.device}, got "
+                            f"{getattr(t, 'dtype', type(t))} on {getattr(t, 'device', '?')}")
+
+    def npg_params(self, theta=None):
+        """Set the parameters from a CUDA fp32 [P] tensor (mjrl's flat order), or return a copy of them."""
+        if theta is not None:
+            theta = theta.to(self.device, torch.float32).contiguous()
+            self._check(self.lib.simstep_npg_params(self._h, 1, _ptr(theta), _stream(self.device)))
+            return theta
+        out = torch.empty((self.npg_n_params,), device=self.device, dtype=torch.float32)
+        self._check(self.lib.simstep_npg_params(self._h, 0, _ptr(out), _stream(self.device)))
+        return out
+
+    def npg_grad(self, obs, act, adv, valid=None, out=None):
+        n = obs.shape[0]
+        for t, nm in ((obs, "obs"), (act, "act"), (adv, "adv")):
+            self._npg_rows(t, nm)
+        self._npg_rows(valid, "valid", torch.uint8)
+        out = torch.empty((self.npg_n_params + 2,), device=self.device, dtype=torch.float64) if out is None else out
+        self._check(self.lib.simstep_npg_grad(self._h, _ptr(obs), _ptr(act), _ptr(adv), _ptr(valid), n, _ptr(out),
+                                              _stream(self.device)))
+        return out
+
+    def npg_prepare(self, obs, idx=None):
+        n = obs.shape[0]
+        self._npg_rows(obs, "obs")
+        self._npg_rows(idx, "idx", torch.int64)
+        self._check(self.lib.simstep_npg_prepare(self._h, _ptr(obs), n, _ptr(idx), 0 if idx is None else idx.numel(),
+                                                 _stream(self.device)))
+
+    def npg_fvp(self, obs, valid=None, idx=None, v=None, out=None):
+        n = obs.shape[0]
+        self._npg_rows(obs, "obs")
+        self._npg_rows(valid, "valid", torch.uint8)
+        self._npg_rows(idx, "idx", torch.int64)
+        self._npg_rows(v, "v", torch.float64)
+        out = torch.empty((self.npg_n_params + 2,), device=self.device, dtype=torch.float64) if out is None else out
+        self._check(self.lib.simstep_npg_fvp(self._h, _ptr(obs), _ptr(valid), n, _ptr(idx),
+                                             0 if idx is None else idx.numel(), _ptr(v), _ptr(out), _stream(self.device)))
+        return out
+
+    def npg_cg(self, op, sums, damping=0.0):
+        self._check(self.lib.simstep_npg_cg(self._h, int(op), _ptr(sums), float(damping), _stream(self.device)))
+
+    def npg_apply(self, step, const_lr=False):
+        self._check(self.lib.simstep_npg_apply(self._h, float(step), int(bool(const_lr)), _stream(self.device)))
+
+    def npg_diag(self, obs, act, adv, valid=None):
+        for t, nm in ((obs, "obs"), (act, "act"), (adv, "adv")):
+            self._npg_rows(t, nm)
+        self._npg_rows(valid, "valid", torch.uint8)
+        out = torch.empty((3,), device=self.device, dtype=torch.float64)
+        self._check(self.lib.simstep_npg_diag(self._h, _ptr(obs), _ptr(act), _ptr(adv), _ptr(valid), obs.shape[0],
+                                              _ptr(out), _stream(self.device)))
+        return out
+
+    def npg_scalars(self):
+        """{r.r, g.x, alpha, gradient rows, mean advantage, CG iterations run} as a CUDA fp64 [6] tensor."""
+        out = torch.empty((6,), device=self.device, dtype=torch.float64)
+        self._check(self.lib.simstep_npg_scalars(self._h, _ptr(out), _stream(self.device)))
         return out
 
     # -- training (tf32 handles only) ---------------------------------------------------

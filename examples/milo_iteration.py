@@ -1,5 +1,5 @@
 """One MILO iteration on a B200 with the reference's objects swapped for amp_extensions_b200's (reference run.py:60-170
-and mjrl/mjrl/algos/batch_reinforce.py:85-170, without the NPG update itself):
+and mjrl/mjrl/algos/batch_reinforce.py:85-170, with the NPG update as an option):
 
   1. train the dynamics ensemble on an offline dataset            (run.py:80-93   -> DynamicsEnsemble.train)
   2. discrepancy threshold over the dataset                        (run.py:108     -> compute_threshold)
@@ -7,6 +7,8 @@ and mjrl/mjrl/algos/batch_reinforce.py:85-170, without the NPG update itself):
   4. roll the policy out in the learned-dynamics env               (sampler.py     -> DeviceRollout.collect)
   5. fit the cost on the rollout, recompute the rewards            (batch_reinforce.py:113-144)
   6. returns, GAE advantages, whitening, rollout statistics        (process_samples.py, batch_reinforce.py:135-141)
+  7. with npg_steps > 0: that many rounds of collect -> advantages -> NPG policy step on the device (npg_cg.py,
+     DeviceNPG.update)
 
 Synthetic offline / expert data stand in for data/offline.pt and data/expert.pt (a download in the reference);
 initial states come from the spin-kick clip without the simulator.  Run:  python examples/milo_iteration.py
@@ -42,7 +44,7 @@ class GaussianMLP:
         self.log_std = torch.full((act_dim,), float(init_log_std))
 
 
-def main(num_envs=512, horizon=40, epochs=3, n_offline=4096, hidden=(128, 128), num_models=4, verbose=True):
+def main(num_envs=512, horizon=40, epochs=3, n_offline=4096, hidden=(128, 128), num_models=4, verbose=True, npg_steps=0):
     from amp_extensions_b200 import (AmpDataset, DynamicsEnsemble, ImitationReward, RBFLinearCost, VecSimEnv)
     from amp_extensions_b200.rollout import DeviceRollout
     S, A = 226, 28
@@ -80,6 +82,18 @@ def main(num_envs=512, horizon=40, epochs=3, n_offline=4096, hidden=(128, 128), 
                env_steps=int(batch.rewards.numel()), trajectories=len(stats["ep_len"]), complete_paths=len(paths),
                mean_cost=stats["mean_cost"], adv_mean=float(adv.mean()), adv_std=float(adv.std(unbiased=False)),
                mean_return=float(ret[0].mean()), expert_cost=float(cost.get_expert_cost()))
+    if npg_steps > 0:                                                                  # 7
+        from amp_extensions_b200.npg import DeviceNPG
+        npg = DeviceNPG(ro, policy)
+        out["npg"] = []
+        for _ in range(npg_steps):
+            res = npg.update(batch, adv)
+            out["npg"].append({k: float(v) for k, v in res.items()})
+            env.reset()
+            batch = ro.collect(horizon, graph=True)                                     # replays with the new policy
+            ret = batch.returns(0.995)
+            adv = batch.normalize(batch.advantages(torch.zeros_like(ret), 0.995, 0.97))
+        npg.export_params()
     if verbose:
         for k, v in out.items():
             print(f"{k:18s} {v}")

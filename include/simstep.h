@@ -351,6 +351,49 @@ int simstep_moments(simstep_handle* h, const float* x_dev, const uint8_t* valid_
 int simstep_whiten(simstep_handle* h, const float* x_dev, const uint8_t* valid_dev, int64_t n, const double* stats_dev,
                    float eps, float* out_dev, void* stream);
 
+/* ---- natural policy gradient step of the loaded policy (mjrl/mjrl/algos/npg_cg.py: NPG.train_from_paths) ---- */
+
+/* One NPG update of the policy loaded with simstep_load_policy, computed from rows of (obs, action, advantage) in
+ * device memory, written in place into the handle's policy (nothing is re-allocated: graphs that captured
+ * simstep_policy_act stay valid).  The calls only enqueue work; the "sums" they return are un-normalised, with their
+ * row counts, so that a multi-GPU caller can all-reduce them between calls.  P is the length of the parameter vector
+ * in mjrl's get_param_values order: per linear layer the weight [out][in] then the bias [out], then log_std [act].
+ *   init:    allocates the NPG state for the loaded policy (*n_params_out = P); EINVAL when the parameter vector does
+ *            not fit the per-CTA gradient accumulator.  min_log_std is MLP.min_log_std (the clamp of set_param_values).
+ *            simstep_load_policy discards this state.
+ *   params:  set != 0: theta_dev [P] fp32 becomes the parameters (and is written into the policy); set == 0: copies
+ *            the current parameters to theta_dev.
+ *   grad:    out_dev [P + 2] fp64 = { sum_i adv_i dLL_i/dtheta, rows, sum_i adv_i } over the rows with valid_dev[i] != 0
+ *            (NULL: all n rows); LL is MLP.log_likelihood.
+ *   prepare: caches the hidden activations of the Fisher rows: obs rows idx_dev[0 .. n_idx) (int64), or all n rows when
+ *            idx_dev is NULL.  Call again whenever the rows or the parameters change.
+ *   fvp:     out_dev [P + 2] fp64 = { sum over Fisher rows of H_i v, rows, 0 }, H_i the Hessian of MLP.mean_kl at new =
+ *            old for row i (rows with valid_dev[idx] == 0 do not count); v_dev [P] fp64, or NULL for the direction
+ *            of the CG solve, in which case nothing is computed once the solve has converged.
+ *   cg:      SIMSTEP_NPG_CG_START with the grad sums: g = sum / rows, x = 0, r = p = g (cg_solve.py);
+ *            SIMSTEP_NPG_CG_STEP with the fvp sums of the direction: one cg_solve iteration with
+ *            F p = sum / rows + damping * p; converged (remaining steps are no-ops) once r.r < 1e-10.
+ *   apply:   theta += alpha * x with alpha = const_lr ? step : sqrt(|step / (g.x + 1e-10)|), log_std clamped at
+ *            min_log_std, written into the policy; the previous parameters are kept for diag.
+ *   diag:    out_dev [3] fp64 = { rows, sum_i exp(LL_new - LL_old) adv_i, sum_i KL_i(new, old) } (CPI_surrogate and
+ *            kl_old_new of the step just applied).
+ *   scalars: out_dev [6] fp64 = { r.r, g.x, alpha, gradient rows, mean advantage, CG iterations run }. */
+#define SIMSTEP_NPG_CG_START 0
+#define SIMSTEP_NPG_CG_STEP 1
+int simstep_npg_init(simstep_handle* h, float min_log_std, int64_t* n_params_out);
+int simstep_npg_params(simstep_handle* h, int32_t set, float* theta_dev, void* stream);
+int simstep_npg_grad(simstep_handle* h, const float* obs_dev, const float* act_dev, const float* adv_dev,
+                     const uint8_t* valid_dev, int64_t n, double* out_dev, void* stream);
+int simstep_npg_prepare(simstep_handle* h, const float* obs_dev, int64_t n, const int64_t* idx_dev, int64_t n_idx,
+                        void* stream);
+int simstep_npg_fvp(simstep_handle* h, const float* obs_dev, const uint8_t* valid_dev, int64_t n, const int64_t* idx_dev,
+                    int64_t n_idx, const double* v_dev, double* out_dev, void* stream);
+int simstep_npg_cg(simstep_handle* h, int32_t op, const double* sums_dev, double damping, void* stream);
+int simstep_npg_apply(simstep_handle* h, double step, int32_t const_lr, void* stream);
+int simstep_npg_diag(simstep_handle* h, const float* obs_dev, const float* act_dev, const float* adv_dev,
+                     const uint8_t* valid_dev, int64_t n, double* out_dev, void* stream);
+int simstep_npg_scalars(simstep_handle* h, double* out_dev, void* stream);
+
 /* ---- ensemble training (milo/milo/dynamics.py:236-250, DynamicsModel.train_step) ------------------- */
 
 /* All n_models members take one optimisation step per call, each on its own batch of batch_rows

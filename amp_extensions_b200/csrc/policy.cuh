@@ -265,8 +265,8 @@ __global__ void whiten_kernel(const float* __restrict__ x, const uint8_t* __rest
     out[i] = (valid == nullptr || valid[i]) ? (x[i] - m) * inv : 0.f;
 }
 
-// Fixed-range histogram for the multi-GPU quantile (parallel.global_quantile): counts[b] += #{i : x[i] in [lo, hi],
-// bin(x[i]) == b}, bin = clamp(floor((x - lo) / width), 0, bins - 1) evaluated in fp64 like the host code.  Integer
+// Fixed-range histogram (simstep_histogram): counts[b] += #{i : x[i] in [lo, hi],
+// bin(x[i]) == b}, bin = clamp(floor((x - lo) / width), 0, bins - 1) evaluated in fp64.  Integer
 // counts: the result does not depend on scheduling.  Shared-memory bins per block, then one atomic per non-empty bin.
 constexpr int kHistMaxBins = 8192;
 
@@ -293,120 +293,135 @@ histogram_kernel(const float* __restrict__ x, long long n, double lo, double hi,
 
 
 // ---- device-side steps of the distributed quantile (parallel.global_quantile) --------------------------------
-// qstate: per order statistic i in {0, 1}: [4i] window lo, [4i + 1] window hi, [4i + 2] samples below the window,
-// [4i + 3] rank k of the order statistic (all doubles, resident on the device: no host round trip per refinement).
+// Exact radix selection on the order-preserving key of the fp32 bit pattern,
+//     key(u) = u ^ (sign(u) ? 0xFFFFFFFF : 0x80000000)      (unsigned order of keys = order of the floats),
+// NaN (detected on the bits before keying) counted in a slot of its own.  Three histogram passes of 12, 12 and 8
+// key bits fix all 32 bits of the two order statistics that bracket the quantile.
+// qstate (doubles, resident on the device): [0] q (set by the caller), [1] result (written by the SELECT that fixes
+// the last bits), [2] n, [3] NaN count; order statistic i in {0, 1}: [4 + 4i] key prefix, [5 + 4i] key bits fixed
+// (32 = done), [6 + 4i] samples whose key is below the prefix, [7 + 4i] rank k.  Start: q, then zeros.
+constexpr int kQuantileBins = 4096;                      // widest digit: 12 bits
+constexpr int kQuantileNanSlot = 2 * kQuantileBins;      // counts: [2][kQuantileBins] + NaN count
+constexpr int kQuantileDigit = 12;
 
-// out[0] = -min(x), out[1] = max(x): one MAX all-reduce makes both global.  Single block, deterministic.
-__global__ void __launch_bounds__(1024)
-quantile_minmax_kernel(const float* __restrict__ x, long long n, double* __restrict__ out) {
-  __shared__ float s_mn[32], s_mx[32];
-  float mn = INFINITY, mx = -INFINITY;
-  for (long long i = threadIdx.x; i < n; i += blockDim.x) {
-    const float v = x[i];
-    mn = fminf(mn, v);
-    mx = fmaxf(mx, v);
-  }
-  for (int off = 16; off > 0; off >>= 1) {
-    mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, off));
-    mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, off));
-  }
-  if ((threadIdx.x & 31) == 0) { s_mn[threadIdx.x >> 5] = mn; s_mx[threadIdx.x >> 5] = mx; }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    for (int w = 1; w < (blockDim.x + 31) / 32; ++w) { mn = fminf(mn, s_mn[w]); mx = fmaxf(mx, s_mx[w]); }
-    out[0] = -static_cast<double>(mn);
-    out[1] = static_cast<double>(mx);
-  }
-}
+__device__ __forceinline__ int quantile_digit_bits(int fixed) { return min(kQuantileDigit, 32 - fixed); }
 
-// counts[i * bins + b] += samples of window i in bin b (both windows in one pass over x)
+// counts[i * kQuantileBins + d] += samples whose key matches prefix i and has next digit d; while both order
+// statistics share their prefix (always in the first pass) only window 0 is counted.  The first pass also counts NaN.
+// Equal digits of a warp are combined with __match_any_sync before the shared-memory atomic (heavy ties, e.g.
+// exact zeros, would otherwise serialise a warp on one bin).
 __global__ void __launch_bounds__(256)
-quantile_hist_kernel(const float* __restrict__ x, long long n, const double* __restrict__ qstate, int bins,
+quantile_hist_kernel(const float* __restrict__ x, long long n, const double* __restrict__ qstate,
                      unsigned long long* __restrict__ counts) {
-  extern __shared__ unsigned int sh_bins[];  // [2][bins]
-  for (int b = threadIdx.x; b < 2 * bins; b += blockDim.x) sh_bins[b] = 0u;
-  __syncthreads();
-  double lo[2], hi[2], inv[2];
+  __shared__ unsigned int sh_bins[2 * kQuantileBins + 1];
+  int fixed[2];
+  unsigned prefix[2];
 #pragma unroll
   for (int i = 0; i < 2; ++i) {
-    lo[i] = qstate[4 * i];
-    hi[i] = qstate[4 * i + 1];
-    inv[i] = hi[i] > lo[i] ? bins / (hi[i] - lo[i]) : 0.0;
+    prefix[i] = static_cast<unsigned>(qstate[4 + 4 * i]);
+    fixed[i] = static_cast<int>(qstate[5 + 4 * i]);
   }
-  for (long long j = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; j < n;
-       j += static_cast<long long>(gridDim.x) * blockDim.x) {
-    const double v = x[j];
-#pragma unroll
-    for (int i = 0; i < 2; ++i) {
-      if (v >= lo[i] && v <= hi[i]) {
-        int b = static_cast<int>(floor((v - lo[i]) * inv[i]));
-        b = b < 0 ? 0 : (b >= bins ? bins - 1 : b);
-        atomicAdd(&sh_bins[i * bins + b], 1u);
+  if (fixed[0] >= 32 && fixed[1] >= 32) return;
+  const int windows = (fixed[0] == fixed[1] && prefix[0] == prefix[1]) ? 1 : 2;
+  const bool count_nan = fixed[0] == 0;
+  for (int b = threadIdx.x; b < 2 * kQuantileBins + 1; b += blockDim.x) sh_bins[b] = 0u;
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  // every thread of a block runs the same number of iterations: the warp votes below need all lanes
+  for (long long base = blockIdx.x * static_cast<long long>(blockDim.x); base < n;
+       base += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long j = base + threadIdx.x;
+    const bool valid = j < n;
+    const unsigned u = valid ? __float_as_uint(x[j]) : 0u;
+    const bool nan = valid && (u & 0x7fffffffu) > 0x7f800000u;
+    const unsigned key = u ^ ((u >> 31) ? 0xffffffffu : 0x80000000u);
+    if (count_nan) {
+      const unsigned m = __ballot_sync(0xffffffffu, nan);
+      if (lane == 0 && m) atomicAdd(&sh_bins[kQuantileNanSlot], static_cast<unsigned>(__popc(m)));
+    }
+    for (int i = 0; i < windows; ++i) {
+      int bin = -1;
+      if (valid && !nan && fixed[i] < 32 && (fixed[i] == 0 || (key >> (32 - fixed[i])) == prefix[i])) {
+        const int w = quantile_digit_bits(fixed[i]);
+        bin = static_cast<int>((key >> (32 - fixed[i] - w)) & ((1u << w) - 1u));
       }
+      const unsigned peers = __match_any_sync(0xffffffffu, bin);
+      if (bin >= 0 && lane == __ffs(peers) - 1) atomicAdd(&sh_bins[i * kQuantileBins + bin], static_cast<unsigned>(__popc(peers)));
     }
   }
   __syncthreads();
-  for (int b = threadIdx.x; b < 2 * bins; b += blockDim.x)
+  for (int b = threadIdx.x; b < 2 * kQuantileBins + 1; b += blockDim.x)
     if (sh_bins[b]) atomicAdd(&counts[b], static_cast<unsigned long long>(sh_bins[b]));
 }
 
-// Narrows window i to the bin that holds its order statistic: the first bin whose cumulative count (plus the samples
-// below the window) exceeds k.  One block; thread t scans a contiguous run of bins, then a serial pass over the runs.
+__device__ __forceinline__ double quantile_key_value(unsigned key) {
+  return static_cast<double>(__uint_as_float((key & 0x80000000u) ? (key ^ 0x80000000u) : ~key));
+}
+
+// Given the (all-reduced) counts of one HIST pass: in the first pass n, the NaN count and the ranks
+// k0 = floor(q (n - 1)), k1 = min(k0 + 1, n - 1); then appends to each prefix the digit whose cumulative count
+// (plus the samples below the prefix) first exceeds k.  When the last bits are fixed, qstate[1] = the
+// quantile, interpolated in fp64 with torch.lerp's formula; NaN when there are no samples or any NaN.
+// One block; thread t sums a contiguous run of bins, thread 0 walks the runs, then the bins of the run.
 __global__ void __launch_bounds__(256)
-quantile_select_kernel(const long long* __restrict__ counts, int bins, double* __restrict__ qstate) {
+quantile_select_kernel(const long long* __restrict__ counts, double* __restrict__ qstate) {
   __shared__ long long run_sum[256];
+  const bool same = qstate[4] == qstate[8] && qstate[5] == qstate[9];
+  bool finished = false;
   for (int i = 0; i < 2; ++i) {
-    const long long* c = counts + static_cast<long long>(i) * bins;
-    const int per = (bins + 255) / 256;
-    const int b0 = threadIdx.x * per, b1 = min(bins, b0 + per);
+    double* st = qstate + 4 + 4 * i;
+    const int fixed = static_cast<int>(st[1]);  // the same in every thread: written by thread 0 before a barrier
+    if (fixed >= 32) continue;
+    const int w = quantile_digit_bits(fixed);
+    const int nb = 1 << w;
+    const int per = nb / 256;
+    const long long* c = counts + (same ? 0 : i * kQuantileBins);
     long long s = 0;
-    for (int b = b0; b < b1; ++b) s += c[b];
+    for (int b = threadIdx.x * per; b < (threadIdx.x + 1) * per; ++b) s += c[b];
     run_sum[threadIdx.x] = s;
     __syncthreads();
     if (threadIdx.x == 0) {
-      const double lo = qstate[4 * i], hi = qstate[4 * i + 1];
-      const long long k = static_cast<long long>(qstate[4 * i + 3]);
-      long long cum = static_cast<long long>(qstate[4 * i + 2]);
-      if (hi > lo) {
+      bool active = true;
+      if (fixed == 0 && i == 0) {
+        long long valid = 0;
+        for (int t = 0; t < 256; ++t) valid += run_sum[t];
+        const long long nan = counts[kQuantileNanSlot];
+        const long long n = valid + nan;
+        qstate[2] = static_cast<double>(n);
+        qstate[3] = static_cast<double>(nan);
+        if (nan > 0 || n == 0) {
+          qstate[1] = NAN;
+          qstate[5] = qstate[9] = 32.0;
+          active = false;
+        } else {
+          const double k0 = floor(qstate[0] * static_cast<double>(n - 1));
+          qstate[7] = k0;
+          qstate[11] = fmin(k0 + 1.0, static_cast<double>(n - 1));
+        }
+      }
+      if (active) {
+        const long long k = static_cast<long long>(st[3]);
+        long long cum = static_cast<long long>(st[2]);
         int t = 0;
         while (t < 255 && cum + run_sum[t] <= k) cum += run_sum[t++];
         int b = t * per;
-        const int bend = min(bins, b + per);
-        while (b < bend - 1 && cum + c[b] <= k) cum += c[b++];
-        if (b >= bins) b = bins - 1;
-        const double width = (hi - lo) / bins;
-        qstate[4 * i] = lo + b * width;
-        qstate[4 * i + 1] = lo + (b + 1) * width;
-        qstate[4 * i + 2] = static_cast<double>(cum);
+        while (b < (t + 1) * per - 1 && cum + c[b] <= k) cum += c[b++];
+        st[0] = st[0] * nb + b;
+        st[1] = fixed + w;
+        st[2] = static_cast<double>(cum);
+        finished = fixed + w == 32;
       }
     }
     __syncthreads();
   }
-}
-
-// out[i] = -min{x in window i} (-(+inf) when the window holds none of this rank's samples); single block
-__global__ void __launch_bounds__(1024)
-quantile_winmin_kernel(const float* __restrict__ x, long long n, const double* __restrict__ qstate,
-                       double* __restrict__ out) {
-  __shared__ float s_mn[2][32];
-  float mn[2] = {INFINITY, INFINITY};
-  const double lo0 = qstate[0], hi0 = qstate[1], lo1 = qstate[4], hi1 = qstate[5];
-  for (long long i = threadIdx.x; i < n; i += blockDim.x) {
-    const float v = x[i];
-    const double d = v;
-    if (d >= lo0 && d <= hi0) mn[0] = fminf(mn[0], v);
-    if (d >= lo1 && d <= hi1) mn[1] = fminf(mn[1], v);
-  }
-#pragma unroll
-  for (int i = 0; i < 2; ++i) {
-    for (int off = 16; off > 0; off >>= 1) mn[i] = fminf(mn[i], __shfl_xor_sync(0xffffffffu, mn[i], off));
-    if ((threadIdx.x & 31) == 0) s_mn[i][threadIdx.x >> 5] = mn[i];
-  }
-  __syncthreads();
-  if (threadIdx.x < 2) {
-    float m = INFINITY;
-    for (int w = 0; w < (blockDim.x + 31) / 32; ++w) m = fminf(m, s_mn[threadIdx.x][w]);
-    out[threadIdx.x] = -static_cast<double>(m);
+  if (threadIdx.x == 0 && finished) {  // both order statistics advance together: window 1 fixed its last bits
+    const double v0 = quantile_key_value(static_cast<unsigned>(qstate[4]));
+    const double v1 = quantile_key_value(static_cast<unsigned>(qstate[8]));
+    const double pos = qstate[0] * (qstate[2] - 1.0);
+    const double wt = pos - floor(pos);
+    const double d = v1 - v0;
+    // torch.lerp: self + w (end - self) for w < 0.5, else end - (end - self)(1 - w); w == 0 is sorted[k0] exactly
+    qstate[1] = wt == 0.0 ? v0 : (wt < 0.5 ? fma(wt, d, v0) : fma(-d, 1.0 - wt, v1));
   }
 }
 

@@ -340,13 +340,14 @@ class Engine:
                                                _stream(self.device)))
         return out
 
-    QOP_MINMAX, QOP_HIST, QOP_SELECT, QOP_WINMIN = 0, 1, 2, 3
+    QOP_HIST, QOP_SELECT, QUANTILE_BINS = 1, 2, 4096
 
-    def quantile_op(self, op, x=None, bins=0, qstate=None, counts=None, out=None):
-        """One device-side step of the distributed quantile (simstep_quantile_op); x: contiguous fp32 CUDA vector."""
+    def quantile_op(self, op, x=None, qstate=None, counts=None):
+        """One device-side round step of the distributed quantile (simstep_quantile_op); x: contiguous fp32 CUDA
+        vector, qstate: 12 fp64, counts: 2 * QUANTILE_BINS + 1 int64, both on this device."""
         n = 0 if x is None else x.numel()
-        self._check(self.lib.simstep_quantile_op(self._h, int(op), _ptr(x), n, int(bins), _ptr(qstate), _ptr(counts),
-                                                 _ptr(out), _stream(self.device)))
+        self._check(self.lib.simstep_quantile_op(self._h, int(op), _ptr(x), n, self.QUANTILE_BINS, _ptr(qstate),
+                                                 _ptr(counts), None, _stream(self.device)))
 
     def reduce_max_sum(self, x, out=None):
         """[max, sum] of a device vector as fp64 (written into `out` when given)."""

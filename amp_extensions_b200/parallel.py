@@ -4,13 +4,16 @@ The env step itself needs no data-path collective (every env is independent; SUR
 torch.distributed (NCCL on GPUs, gloo in the CPU tests) carries only small reductions:
 
   * the discrepancy threshold = dataset maximum (reference milo/milo/dynamics.py:145-152) -> all-reduce MAX,
-    or, as an extension, a global quantile of the per-row discrepancies via a two-pass histogram all-reduce;
+    or, as an extension, a global quantile of the per-row discrepancies via radix-select histogram all-reduces;
   * fit_cost's feature mean (reference milo/milo/linear_cost.py:84-94) -> all-reduce SUM of [D] sums + count;
   * rollout cost / return statistics (reference mjrl/mjrl/algos/batch_reinforce.py:135-141, 288-295);
   * normalisation statistics of a sharded offline dataset (reference milo/milo/datasets.py:23-43).
 
 Every function works un-initialised (world size 1) and on CPU tensors (gloo) as well as CUDA tensors (NCCL).
 """
+import math
+import struct
+
 import torch
 import torch.distributed as dist
 
@@ -155,92 +158,97 @@ def rollout_stats(cost, ipm, bonus, done, num_steps):
     }
 
 
-def _global_quantile_device(x32, q, bins, refine, engine):
-    """Device-resident variant: the windows around the two bracketing order statistics live in device memory
-    (simstep_quantile_op), so the call issues 1 all-gather of [-min, max, count], refine + 1 all-reduces of the
-    two histograms and 1 all-reduce of the window minima - and synchronises with the host ONCE, for the result."""
-    dev = x32.device
-    f64 = dict(device=dev, dtype=torch.float64)
-    bins = min(int(bins), 4096)
-    head = torch.empty(3, **f64)
-    engine.quantile_op(engine.QOP_MINMAX, x32, out=head)
-    head[2] = float(x32.numel())
-    if is_dist():
-        allh = torch.empty(world_size() * 3, **f64)
-        dist.all_gather_into_tensor(allh, head)
-        allh = allh.view(-1, 3)
-        mm, n = allh[:, :2].max(dim=0).values, allh[:, 2].sum()
-    else:
-        mm, n = head[:2], head[2]
-    lo, hi = -mm[0], mm[1]
-    pos = q * (n - 1.0)
-    k0 = torch.floor(pos).clamp_min(0.0)
-    frac = (pos - k0).clamp(0.0, 1.0)
-    k1 = torch.minimum(k0 + 1.0, (n - 1.0).clamp_min(0.0))
-    zero = torch.zeros((), **f64)
-    qstate = torch.stack([lo, hi, zero, k0, lo, hi, zero, k1]).contiguous()
-    counts = torch.empty(2 * bins, device=dev, dtype=torch.int64)
-    for _ in range(int(refine) + 1):
-        engine.quantile_op(engine.QOP_HIST, x32, bins=bins, qstate=qstate, counts=counts)
+def _global_quantile_device(x32, q, engine):
+    """Device-resident variant of the radix selection (simstep_quantile_op): the prefixes, ranks and result live in
+    device memory, so the call issues 3 all-reduces of the counts and synchronises with the host ONCE, for the
+    result."""
+    qstate = torch.zeros(12, device=x32.device, dtype=torch.float64)
+    qstate[0] = q
+    counts = torch.empty(2 * engine.QUANTILE_BINS + 1, device=x32.device, dtype=torch.int64)
+    for _ in range(3):  # 12 + 12 + 8 key bits
+        engine.quantile_op(engine.QOP_HIST, x32, qstate=qstate, counts=counts)
         _all_reduce(counts, dist.ReduceOp.SUM)
-        engine.quantile_op(engine.QOP_SELECT, None, bins=bins, qstate=qstate, counts=counts)
-    out = torch.empty(2, **f64)
-    engine.quantile_op(engine.QOP_WINMIN, x32, qstate=qstate, out=out)
-    _all_reduce(out, dist.ReduceOp.MAX)
-    v0, v1 = -out[0], -out[1]
-    res = torch.where(n > 0, v0 + frac * (v1 - v0), torch.full((), float("nan"), **f64))
-    return float(res.item())
+        engine.quantile_op(engine.QOP_SELECT, None, qstate=qstate, counts=counts)
+    return float(qstate[1].item())
 
 
-def global_quantile(x_local, q, bins=4096, refine=2, engine=None):
-    """q-quantile (linear interpolation between order statistics, as torch.quantile) of the union of every
-    rank's x_local, without gathering the samples: all-reduce of min/max and of fixed-range histograms, refined
-    `refine` times around the two order statistics that bracket the quantile.  Exact up to the final bin width
-    (range / bins**(refine+1)); used for threshold_mode='quantile', an extension over the reference's dataset
-    maximum.  With `engine` and a CUDA fp32 vector everything but the final read stays on the device
-    (_global_quantile_device); CPU tensors (the gloo tests) take the torch path below."""
-    xt = torch.as_tensor(x_local)
+# dtype -> (integer view, key bits, digit widths of the passes, struct formats of the integer and the float)
+_KEYS = {torch.float32: (torch.int32, 32, (12, 12, 8), "<i", "<f"),
+         torch.float64: (torch.int64, 64, (16, 16, 16, 16), "<q", "<d")}
+
+
+def _order_stats(x, q):
+    """Torch path of global_quantile: (v0, v1, w) with v0, v1 the order statistics k0 = floor(q (n - 1)) and
+    min(k0 + 1, n - 1) of the union of every rank's x (fp32 or fp64) and w = q (n - 1) - k0, or None when there are no
+    samples or any NaN.  Radix selection on the signed order-preserving key of the bit pattern,
+    key = s ^ ((s >> (B - 1)) & (2^(B-1) - 1)); digit d of a pass counts the samples that share the prefix fixed so
+    far (top digit offset by 2^(w-1) to make it unsigned); one all-reduce of the counts per pass."""
+    view, nbits, widths, ifmt, ffmt = _KEYS[x.dtype]
+    nan = torch.isnan(x)
+    s = x[~nan].view(view).to(torch.int64)
+    key = s ^ ((s >> (nbits - 1)) & ((1 << (nbits - 1)) - 1))
+    keys, below, prefix = [key, key], [0, 0], [0, 0]
+    fixed = 0
+    for p, w in enumerate(widths):
+        shift = nbits - fixed - w
+        same = prefix[0] == prefix[1]  # both order statistics still share their prefix: one histogram serves both
+        digits = [((k >> shift) & ((1 << w) - 1)) ^ ((1 << (w - 1)) if p == 0 else 0) for k in keys[:1 if same else 2]]
+        hists = [torch.bincount(d, minlength=1 << w) for d in digits]
+        head = [nan.sum().reshape(1)] if p == 0 else []
+        packed = all_reduce_sum(torch.cat(hists + head))
+        if p == 0:
+            n_nan = int(packed[-1])
+            n = int(packed[:-1].sum()) + n_nan
+            if n_nan or n == 0:
+                return None
+            pos = q * (n - 1)
+            k0 = math.floor(pos)
+            ks, wt = (k0, min(k0 + 1, n - 1)), pos - k0
+        for i in range(2):
+            j = 0 if same else i
+            cum = torch.cumsum(packed[j << w:(j + 1) << w], 0) + below[i]
+            b = int(torch.searchsorted(cum, torch.tensor([ks[i]], device=cum.device), right=True))
+            below[i] = int(cum[b - 1]) if b > 0 else below[i]
+            prefix[i] = (prefix[i] << w) | b
+            keys.append(keys[j][digits[j] == b])
+        keys = keys[2:]
+        fixed += w
+
+    def value(ukey):
+        key = ukey - (1 << (nbits - 1))
+        s = key ^ ((key >> (nbits - 1)) & ((1 << (nbits - 1)) - 1))
+        return struct.unpack(ffmt, struct.pack(ifmt, s))[0]
+
+    return value(prefix[0]), value(prefix[1]), wt
+
+
+def global_quantile(x_local, q, engine=None):
+    """q-quantile of the union of every rank's x_local, without gathering the samples: the linear interpolation
+    between the order statistics k0 = floor(q (n - 1)) and k0 + 1 of torch.quantile, used for
+    threshold_mode='quantile' (an extension over the reference's dataset maximum).
+
+    The order statistics are exact: radix selection on the order-preserving integer key of the bit pattern, one
+    all-reduce of a histogram of the next key digit per pass (fp32: 12 + 12 + 8 bits, fp64: 4 x 16 bits; other dtypes
+    go through fp64).  Semantics:
+      * any NaN in the union of the samples, or no samples at all, gives NaN; q outside [0, 1] raises ValueError;
+      * w = q (n - 1) - k0 == 0 gives sorted[k0] exactly.  This deliberately differs from torch.quantile where it
+        returns NaN for lerp(inf, inf, 0), e.g. at q = 1 when the maximum is +inf;
+      * otherwise torch.lerp's formula in fp64, v0 + w (v1 - v0) for w < 0.5 and v1 - (v1 - v0)(1 - w) above.
+    With `engine` and a CUDA fp32 vector everything but the final read stays on the device (_global_quantile_device);
+    other tensors (CPU ones in the gloo tests, CUDA fp64) take the torch path."""
+    q = float(q)
+    if not 0.0 <= q <= 1.0:
+        raise ValueError(f"quantile q must be in [0, 1], got {q}")
+    xt = torch.as_tensor(x_local).reshape(-1)
     if engine is not None and xt.is_cuda and xt.dtype == torch.float32:
-        return _global_quantile_device(xt.reshape(-1).contiguous(), float(q), bins, refine, engine)
-    x32 = torch.as_tensor(x_local).reshape(-1) if engine is not None else None
-    x = torch.as_tensor(x_local).to(torch.float64).reshape(-1)
-    dev = x.device
-    n = all_reduce_sum(torch.tensor([float(x.numel())], device=dev, dtype=torch.float64))[0]
-    if n.item() == 0:
+        return _global_quantile_device(xt.contiguous(), q, engine)
+    if xt.dtype not in _KEYS:
+        xt = xt.to(torch.float64)
+    stats = _order_stats(xt.contiguous(), q)
+    if stats is None:
         return float("nan")
-    inf = float("inf")
-    lo = -all_reduce_max(torch.tensor([-(x.min().item() if x.numel() else inf)], device=dev, dtype=torch.float64))[0]
-    hi = all_reduce_max(torch.tensor([x.max().item() if x.numel() else -inf], device=dev, dtype=torch.float64))[0]
-    pos = q * (n.item() - 1)
-    k0 = int(pos)
-    frac = pos - k0
-
-    def order_stat(k):
-        a, b = float(lo), float(hi)
-        below = 0  # samples strictly below the current window
-        for _ in range(refine + 1):
-            if b <= a:
-                return a
-            width = (b - a) / bins
-            if engine is not None and x32.is_cuda and x32.dtype == torch.float32:
-                hist = engine.histogram(x32, a, b, bins).to(torch.float64)
-            else:
-                idx = torch.clamp(((x - a) / width).floor(), 0, bins - 1).long()
-                sel = (x >= a) & (x <= b)
-                hist = torch.bincount(idx[sel], minlength=bins).to(torch.float64)
-            hist = all_reduce_sum(hist)
-            cum = torch.cumsum(hist, 0) + below
-            bin_i = int(torch.searchsorted(cum, torch.tensor([float(k) + 0.5], device=dev, dtype=torch.float64)).item())
-            bin_i = min(bin_i, bins - 1)
-            below = int(cum[bin_i - 1].item()) if bin_i > 0 else below
-            a, b = a + bin_i * width, a + (bin_i + 1) * width
-        # all samples left in the window are within one final bin width: take the window's lower edge + local min
-        in_win = x[(x >= a) & (x <= b)]
-        cand = torch.tensor([-(in_win.min().item() if in_win.numel() else inf)], device=dev, dtype=torch.float64)
-        return float(-all_reduce_max(cand)[0])
-
-    v0 = order_stat(k0)
-    if frac == 0.0 or k0 + 1 >= int(n.item()):
+    v0, v1, w = stats
+    if w == 0.0:
         return v0
-    v1 = order_stat(k0 + 1)
-    return v0 + frac * (v1 - v0)
+    f64 = torch.float64
+    return float(torch.lerp(torch.tensor(v0, dtype=f64), torch.tensor(v1, dtype=f64), w))

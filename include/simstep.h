@@ -427,23 +427,27 @@ int simstep_train_export(simstep_handle* h, int32_t what, float* const* weights_
 /* ---- reductions used by the multi-GPU host code ------------------------- */
 
 /* counts_dev[b] (int64, bins entries, overwritten) = number of x_dev[i] in [lo, hi] whose bin
- * clamp(floor((x - lo) / ((hi - lo) / bins)), 0, bins - 1) is b; 1 <= bins <= 8192.  The all-reduced
- * histograms of the ranks give the global discrepancy quantile without gathering samples. */
+ * clamp(floor((x - lo) / ((hi - lo) / bins)), 0, bins - 1) is b; 1 <= bins <= 8192.  Integer counts:
+ * the all-reduced histograms of the ranks do not depend on scheduling. */
 int simstep_histogram(simstep_handle* h, const float* x_dev, int64_t n, double lo, double hi, int32_t bins,
                       int64_t* counts_dev, void* stream);
 
-/* Device-side steps of the distributed q-quantile (amp_extensions_b200.parallel.global_quantile): the windows that
- * bracket the two order statistics live in device memory, so a refinement costs no host round trip.
- * qstate_dev: 8 doubles, for order statistic i in {0, 1}: [4i] window lo, [4i+1] window hi, [4i+2] number of
- * samples below the window, [4i+3] rank k of the order statistic.  Every op only enqueues work on `stream`.
- *   MINMAX: out_dev[0] = -min(x), out_dev[1] = max(x)              (one all-reduce MAX makes both global)
- *   HIST:   counts_dev[i*bins + b] (int64, overwritten) = samples of window i in bin b, 1 <= bins <= 4096
- *   SELECT: narrows both windows to the bin that holds their order statistic, given the (all-reduced) counts
- *   WINMIN: out_dev[i] = -min{x in window i}                       (all-reduce MAX, negate: the order statistic) */
-#define SIMSTEP_QOP_MINMAX 0
+/* Device-side steps of the distributed q-quantile (amp_extensions_b200.parallel.global_quantile): exact radix
+ * selection of the two order statistics that bracket the quantile on the order-preserving key of the fp32 bit
+ * pattern, key = u ^ (sign ? 0xFFFFFFFF : 0x80000000); three HIST/SELECT rounds fix 12, 12 and 8 key bits, and a
+ * round costs no host round trip.  bins must be SIMSTEP_QUANTILE_BINS.
+ * qstate_dev: 12 doubles, [0] q (set by the caller, the rest zeroed before the first round), [1] the quantile
+ * (written by the SELECT that fixes the last bits; NaN when there are no samples or any NaN), [2] n, [3] NaN
+ * count; for order statistic i in {0, 1}: [4+4i] key prefix, [5+4i] key bits fixed, [6+4i] samples whose key is
+ * below the prefix, [7+4i] rank k.  Every op only enqueues work on `stream`; out_dev is unused.
+ *   HIST:   counts_dev[i*bins + d] (int64, 2*bins+1 entries, overwritten) = samples of x whose key extends prefix i
+ *           by digit d; counts_dev[2*bins] = NaN samples (first round)
+ *   SELECT: given the (all-reduced) counts: n, NaN count and ranks in the first round; appends each order
+ *           statistic's digit to its prefix
+ * Op numbers 0 and 3 (min/max and window minimum of an earlier, approximate scheme) are rejected. */
 #define SIMSTEP_QOP_HIST 1
 #define SIMSTEP_QOP_SELECT 2
-#define SIMSTEP_QOP_WINMIN 3
+#define SIMSTEP_QUANTILE_BINS 4096
 int simstep_quantile_op(simstep_handle* h, int32_t op, const float* x_dev, int64_t n, int32_t bins, double* qstate_dev,
                         int64_t* counts_dev, double* out_dev, void* stream);
 

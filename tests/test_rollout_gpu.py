@@ -368,8 +368,8 @@ def test_moments_and_whitening_match_numpy():
 
 
 def test_histogram_kernel_and_device_quantile_match_torch():
-    """simstep_histogram against torch.histc-style counting in fp64, and parallel.global_quantile through it against
-    torch.quantile (single process: the all-reduces are identities)."""
+    """simstep_histogram against torch.histc-style counting in fp64, and parallel.global_quantile's device path against
+    torch.quantile (single process: the all-reduces are identities; tests/test_quantile.py covers adversarial data)."""
     from amp_extensions_b200 import parallel
     _, eng = _tiny_engine()
     g = torch.Generator(device="cuda").manual_seed(2)

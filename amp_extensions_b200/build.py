@@ -1,8 +1,7 @@
 """In-tree build of libsimstep.so (nvcc, sm_100a only).
 
 `python -m amp_extensions_b200.build` compiles every translation unit under amp_extensions_b200/csrc
-(api.cu: the C ABI and most kernels; final_fused.cu: the fused final-layer kernel's instantiations; chain.cu: the column-fused
-ensemble forward kernel's) in
+(api.cu: the C ABI and most kernels; chain.cu: the column-fused ensemble forward kernel's instantiations) in
 parallel and links them into amp_extensions_b200/csrc/libsimstep.so.  nvcc cross-compiles without a GPU.
 """
 import hashlib
@@ -23,9 +22,7 @@ NVCC_FLAGS = [
     "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC",
 ]
-# extra nvcc flags for A/B builds, e.g. SIMSTEP_NVCC_EXTRA="-DSIMSTEP_GEMM_STAGES_CG2=4" (part of the build stamp)
-NVCC_FLAGS += os.environ.get("SIMSTEP_NVCC_EXTRA", "").split()
-UNITS = ("api.cu", "final_fused.cu", "chain.cu")
+UNITS = ("api.cu", "chain.cu")
 
 
 def _sources():

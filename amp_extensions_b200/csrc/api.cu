@@ -16,7 +16,6 @@
 #include "../../include/simstep.h"
 #include "elementwise.cuh"
 #include "gemm_tcgen05.cuh"
-#include "final_launch.h"
 #include "chain_launch.h"
 #include "imitation.cuh"
 #include "imitation_h3d.cuh"
@@ -58,7 +57,6 @@ struct simstep_handle {
   int sm_count = 148;
   int esize = 4;  // bytes per GEMM operand element
   int bk = 32;    // elements per 128-byte swizzle row
-  int cg = 2;     // CTAs per GEMM tile: 2 = cta_group::2 pairs (256-row tiles), 1 = single-CTA tiles
   int row_align = 256;  // workspace rows are padded to whole tiles
   int S = 0, A = 0, N = 0, L = 0;
   int XP = 0, HT = 0, SP = 0;
@@ -74,13 +72,11 @@ struct simstep_handle {
   void* xbuf = nullptr;
   void* hbuf = nullptr;
   float* dws = nullptr;
-  unsigned int* tickets = nullptr;  // fused final layer: one arrival counter per 128-row block (gemm_final.cuh)
   // SIMSTEP_DEBUG_GUARDS=1 (read at simstep_create): every workspace buffer sits between two 64 KB guard zones filled with
   // 0xA5; simstep_debug_check_guards counts the guard bytes that no longer are (compute-sanitizer is not available on
   // the GPU boxes: this is the out-of-bounds check the test suite runs instead)
   bool guards_on = false;
   std::vector<std::pair<void*, size_t>> guard_allocs;  // (user pointer, user bytes)
-  long long tail_rows_done = 0;       // rows [0, tail_rows_done) of the chunk had their step tail run inside the chain kernel
   bool forward_was_chain = false;     // the workspace's deltas were written by the chain kernel (in row order)
   unsigned int* chain_cnt = nullptr;  // chain kernel: tile counters of the shared units of the last round (zero between launches)
   CUtensorMap tmap_x, tmap_h, tmap_dws;
@@ -95,7 +91,6 @@ struct simstep_handle {
   float* rff_b = nullptr;
   float* rff_wpad = nullptr;
   void* rffin = nullptr;
-  float* rff_part = nullptr;
   double* colsum_partial = nullptr;
   CUtensorMap tmap_rffw, tmap_rffin;
   // feature net (MLPCost): hidden layers of this handle feed the cos-feature head instead of a packed input row
@@ -226,12 +221,12 @@ int encode_operand(simstep_handle* h, CUtensorMap* map, int prec, void* base, lo
   return SIMSTEP_OK;
 }
 
-template <typename E, int MODE, int CG, int EG>
+template <typename E, int MODE, int EG>
 int launch_gemm_t(simstep_handle* h, const CUtensorMap& ax, const CUtensorMap& ah, const CUtensorMap& b,
                   const CUtensorMap& out, const GemmArgs& ga, int sm_count, cudaStream_t st) {
   static bool attr_set[kMaxDevices] = {};  // function attributes are per device
-  auto kern = gemm_tcgen05_kernel<E, MODE, CG, EG>;
-  using Plan = GemmPlan<CG, EG, !epi_is_rff(MODE)>;
+  auto kern = gemm_tcgen05_kernel<E, MODE, EG>;
+  using Plan = GemmPlan<EG, !epi_is_rff(MODE)>;
   constexpr size_t smem = Plan::smem_bytes();
   int dev = h ? h->device : 0;  // h is null for simstep_debug_gemm: use the calling thread's current device
   if (!h) CU_TRY(h, cudaGetDevice(&dev));
@@ -242,17 +237,17 @@ int launch_gemm_t(simstep_handle* h, const CUtensorMap& ax, const CUtensorMap& a
   }
   const int total = ga.m_tiles * ga.n_tiles * ga.groups;
   if (total <= 0) return SIMSTEP_OK;
-  // persistent: one CTA (CG = 1) or one CTA pair (CG = 2) per tile slot, at most one CTA per SM
+  // persistent: one CTA pair per tile slot, at most one CTA per SM
   const int n_inner = ga.n_inner > 1 ? ga.n_inner : 1;
-  const int slots = std::min(total / n_inner, sm_count / CG);
+  const int slots = std::min(total / n_inner, sm_count / 2);
   cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(unsigned(slots * CG));
+  cfg.gridDim = dim3(unsigned(slots * 2));
   cfg.blockDim = dim3(Plan::kThreads);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
   cudaLaunchAttribute attr[2];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CG;
+  attr[0].val.clusterDim.x = 2;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -264,26 +259,18 @@ int launch_gemm_t(simstep_handle* h, const CUtensorMap& ax, const CUtensorMap& a
   return SIMSTEP_OK;
 }
 
-// SIMSTEP_GEMM_WIDE_EPI=0: one epilogue group everywhere (the round-1 kernels), for A/B runs
-bool wide_epilogue_enabled() {
-  static const bool on = [] { const char* e = std::getenv("SIMSTEP_GEMM_WIDE_EPI"); return !(e && e[0] == '0'); }();
-  return on;
-}
-
 template <int MODE>
-int launch_gemm(simstep_handle* h, int prec, int cg, const CUtensorMap& ax, const CUtensorMap& ah, const CUtensorMap& b,
+int launch_gemm(simstep_handle* h, int prec, const CUtensorMap& ax, const CUtensorMap& ah, const CUtensorMap& b,
                 const CUtensorMap& out, const GemmArgs& ga, int sm_count, cudaStream_t st) {
   // Two epilogue groups where the epilogue, not the MMAs, bounds a tile: the cost-feature modes (a cosine per
   // element, no store staging), and store modes whose whole K fits the shortened ring (the first layer).
   constexpr bool kStore = !epi_is_rff(MODE);
-  const bool wide = wide_epilogue_enabled() && cg == 2 && MODE != kEpiFinal &&
-                    (!kStore || ga.kb_x + ga.kb_h <= GemmPlan<2, 2, true>::kStages);
+  const bool wide = MODE != kEpiFinal && (!kStore || ga.kb_x + ga.kb_h <= GemmPlan<2, true>::kStages);
 #define SIMSTEP_GEMM_CASE(ELEM)                                                                    \
   if constexpr (MODE != kEpiFinal) {                                                               \
-    if (wide) return launch_gemm_t<ELEM, MODE, 2, 2>(h, ax, ah, b, out, ga, sm_count, st);          \
+    if (wide) return launch_gemm_t<ELEM, MODE, 2>(h, ax, ah, b, out, ga, sm_count, st);             \
   }                                                                                                \
-  return cg == 2 ? launch_gemm_t<ELEM, MODE, 2, 1>(h, ax, ah, b, out, ga, sm_count, st)             \
-                 : launch_gemm_t<ELEM, MODE, 1, 1>(h, ax, ah, b, out, ga, sm_count, st)
+  return launch_gemm_t<ELEM, MODE, 1>(h, ax, ah, b, out, ga, sm_count, st)
   switch (prec) {
     case SIMSTEP_PREC_TF32: SIMSTEP_GEMM_CASE(ElemTF32);
     case SIMSTEP_PREC_FP16: SIMSTEP_GEMM_CASE(ElemF16);
@@ -291,12 +278,6 @@ int launch_gemm(simstep_handle* h, int prec, int cg, const CUtensorMap& ax, cons
   }
 #undef SIMSTEP_GEMM_CASE
   return fail(h, SIMSTEP_EINVAL, "unknown precision");
-}
-
-// CTAs per GEMM tile: pairs unless SIMSTEP_GEMM_CG=1 asks for single-CTA tiles (bring-up / A-B comparisons)
-int gemm_cta_group() {
-  const char* e = std::getenv("SIMSTEP_GEMM_CG");
-  return (e && e[0] == '1') ? 1 : 2;
 }
 
 int grid_for(long long work_items, int threads, int sm_count) {
@@ -360,10 +341,8 @@ void free_workspace(simstep_handle* h) {
   ws_free(h, h->xbuf); h->xbuf = nullptr;
   ws_free(h, h->hbuf); h->hbuf = nullptr;
   ws_free(h, h->dws); h->dws = nullptr;
-  cudaFree(h->tickets); h->tickets = nullptr;
   cudaFree(h->chain_cnt); h->chain_cnt = nullptr;
   ws_free(h, h->rffin); h->rffin = nullptr;
-  ws_free(h, h->rff_part); h->rff_part = nullptr;
   h->cap_rows = 0;
 }
 
@@ -376,7 +355,7 @@ long long chunk_limit(const simstep_handle* h) {
 int ensure_workspace(simstep_handle* h, long long rows) {
   rows = round_up(rows < 1 ? 1 : rows, h->row_align);
   if (rows > chunk_limit(h)) rows = chunk_limit(h);
-  if (rows <= h->cap_rows && (!h->have_rff || h->rffin || (h->feat_net && h->rff_part))) return SIMSTEP_OK;
+  if (rows <= h->cap_rows && (!h->have_rff || h->feat_net || h->rffin)) return SIMSTEP_OK;
   if (rows < h->cap_rows) rows = h->cap_rows;
   CU_TRY(h, cudaDeviceSynchronize());
   free_workspace(h);
@@ -385,8 +364,6 @@ int ensure_workspace(simstep_handle* h, long long rows) {
     CU_TRY(h, ws_alloc(h, &h->xbuf, size_t(rows) * h->XP * h->esize));
     if (h->HT > 0) CU_TRY(h, ws_alloc(h, &h->hbuf, size_t(h->N) * rows * h->HT * h->esize));
     CU_TRY(h, ws_alloc(h, &h->dws, size_t(h->N) * rows * h->DP * sizeof(float)));
-    CU_TRY(h, cudaMalloc(&h->tickets, size_t(rows / kBlockM + 2) * sizeof(unsigned int)));
-    CU_TRY(h, cudaMemset(h->tickets, 0, size_t(rows / kBlockM + 2) * sizeof(unsigned int)));
     CU_TRY(h, cudaMalloc(&h->chain_cnt, size_t(h->sm_count) * 2 * sizeof(unsigned int)));
     CU_TRY(h, cudaMemset(h->chain_cnt, 0, size_t(h->sm_count) * 2 * sizeof(unsigned int)));
     CU_TRY(h, cudaMemset(h->xbuf, 0, size_t(rows) * h->XP * h->esize));
@@ -405,13 +382,10 @@ int ensure_workspace(simstep_handle* h, long long rows) {
                         kBlockM);
     if (rc) return rc;
   }
-  if (h->have_rff && h->feat_net) {
-    CU_TRY(h, ws_alloc(h, &h->rff_part, size_t(h->D_pad / kBlockN) * rows * sizeof(float)));  // A operand = hbuf
-  } else if (h->have_rff) {
+  if (h->have_rff && !h->feat_net) {  // a feature net's head reads the activation buffer instead
     const int rka = h->rff_split_cap ? 2 * h->RK : h->RK;  // [hi | lo]; the hi block is read twice by the GEMM
     CU_TRY(h, ws_alloc(h, &h->rffin, size_t(rows) * rka * h->esize));
     CU_TRY(h, cudaMemset(h->rffin, 0, size_t(rows) * rka * h->esize));
-    CU_TRY(h, ws_alloc(h, &h->rff_part, size_t(h->D_pad / kBlockN) * rows * sizeof(float)));
     int rc = encode_operand(h, &h->tmap_rffin, prec, h->rffin, rka, rows, rka, kBlockM);
     if (rc) return rc;
   }
@@ -433,89 +407,12 @@ void launch_prep(simstep_handle* h, const float* s, const float* a, long long n,
   g_launches++;
 }
 
-// The env step's tail for a chunk (caller tensors, chunk-local row 0): given to run_ensemble_chunk it is fused into
-// the final layer's launch (gemm_final.cuh) when final_fused_ok() says so; otherwise launch_post() runs it.
-struct StepTail {
-  const float* state = nullptr;
-  float* next_state = nullptr;
-  const int32_t* member = nullptr;
-  int32_t* num_steps = nullptr;
-  float* disc = nullptr;
-  uint8_t* done = nullptr;
-  bool rff = false;  // also write the cost features' operand rows of [s; s'] (input_type 'ss')
-};
-
-// SIMSTEP_FINAL_FUSED=1 selects the single-launch final layer + env-step tail (gemm_final.cuh).  It is correct
-// (the parity suite passes with it) but NOT the default: measured on B200 it is slower than the final-layer GEMM
-// followed by the post-step kernel (DESIGN.md section 5) - the final layer is HBM-bound, and the tails' L2 round
-// trips queue behind the operand stream.
-bool final_fused_enabled() {
-  static const bool on = [] { const char* e = std::getenv("SIMSTEP_FINAL_FUSED"); return e && e[0] == '1'; }();
-  return on;
-}
-
-bool final_fused_ok(const simstep_handle* h, const StepTail& t) {
-  const Layer& fin = h->layers[h->L];
-  return final_fused_enabled() && h->cg == 2 && h->S % 2 == 0 && h->S <= kBlockN && fin.o_pad == kBlockN &&
-         reinterpret_cast<uintptr_t>(t.state) % 16 == 0 && reinterpret_cast<uintptr_t>(t.next_state) % 16 == 0 &&
-         (t.next_state == nullptr || t.state != nullptr) && final_smem_bytes(h->S, h->N) <= 227 * 1024;
-}
-
-int launch_final(simstep_handle* h, long long n, long long rows_pad, const StepTail& t, cudaStream_t st) {
-  const Layer& ly = h->layers[h->L];
-  FinalLaunch fl;
-  fl.ax = h->tmap_x;
-  fl.ah = h->tmap_h;
-  fl.b = ly.tmap_w;
-  FinalArgs& fa = fl.args;
-  fa = FinalArgs{};
-  fa.m_tiles = int(rows_pad / (kBlockM * 2));
-  fa.groups = h->N;
-  fa.kb_x = ly.kb_x;
-  fa.kb_h0 = ly.kb_h0;
-  fa.kb_h = ly.kb_h;
-  fa.a_rows_per_group = int(h->cap_rows);
-  fa.b_rows_per_group = ly.o_pad;
-  fa.bias = ly.bias;
-  fa.scale = h->cfg.transform ? h->out_scale_dev : nullptr;
-  fa.shift = h->cfg.transform ? h->out_shift_dev : nullptr;
-  fa.dws_t = reinterpret_cast<float4*>(h->dws);
-  fa.n_blocks = int(rows_pad / kBlockM);
-  fa.counters = h->tickets;
-  fa.state = t.state;
-  fa.next_state = t.next_state;
-  fa.member = t.member;
-  fa.num_steps = t.num_steps;
-  fa.disc = t.disc;
-  fa.done = t.done;
-  fa.n_rows = n;
-  fa.S = h->S;
-  fa.tc = h->term;
-  if (t.rff) {
-    fa.rff_out = h->rffin;
-    fa.rff_pitch = h->rff_split_cap ? 2 * h->RK : h->RK;
-    fa.rff_col2 = h->rff_col2;
-    fa.rff_lo_off = h->rff_split ? h->RK : 0;
-  }
-  static const int dbg = [] { const char* e = std::getenv("SIMSTEP_FINAL_DEBUG"); return e ? std::atoi(e) : 0; }();
-  fa.debug = dbg;
-  CU_TRY(h, launch_final_fused(h->cfg.precision, fl, h->sm_count, h->device, st));
-  g_launches++;
-  return SIMSTEP_OK;
-}
-
 // The column-fused forward pass (gemm_chain.cuh): every layer of a (member, 256-row env tile) on one CTA pair, the
-// activations handed from layer to layer through L2.  SIMSTEP_CHAIN=0 restores one launch per layer (A/B runs);
-// SIMSTEP_CHAIN_SLOT=0 keeps the activation rows at their env rows instead of in the pair's L2-resident slot.
-// SIMSTEP_CHAIN (A/B runs): 0 one launch per layer; 1 activation rows at their env rows instead of in the pair's
-// L2-resident slot; 2 the default; 3 the last, partial round as a plain round instead of shared between pairs.
-int chain_mode() {
-  static const int mode = [] {
-    const char* e = std::getenv("SIMSTEP_CHAIN");
-    if (e && e[0] >= '0' && e[0] <= '3') return e[0] - '0';
-    return 2;
-  }();
-  return mode;
+// activations handed from layer to layer through L2.  SIMSTEP_CHAIN=0 forces one launch per layer, the reference the
+// column-fused kernel is tested against bit for bit.
+bool chain_enabled() {
+  static const bool on = [] { const char* e = std::getenv("SIMSTEP_CHAIN"); return !(e && e[0] == '0'); }();
+  return on;
 }
 
 // The chain kernel lives on L2 hits: every pair re-reads its unit's activation rows layer after layer while all members'
@@ -523,20 +420,8 @@ int chain_mode() {
 // pair - fits 90 % of the L2 (108 of 126 MB at 4 x (512 x 4); measured 10 % faster than one launch per layer); an
 // 8 x (1024 x 4) ensemble (136 MB of weights, 2.2 MB of activations per unit) thrashes it and was measured 14 % SLOWER,
 // so such shapes keep one launch per layer.
-// SIMSTEP_CHAIN_TAIL=1: the env step's tail (next state, discrepancy, termination, cost operand rows) runs INSIDE the
-// chain kernel, on four extra warps per CTA, for the env tiles of its whole rounds but the last
-// (SIMSTEP_CHAIN_TAIL_KEEP=<rounds left to the post-step kernel>, default 1).  Correct - next states, counters and masks
-// bit-identical to the post-step kernel, the discrepancy within 2e-6 - and NOT the default: the chain kernel is bound by
-// the L2->SM path its operands already saturate, so the tail's bytes cost there what they cost the post-step kernel
-// outside (first round fused: launch +16 us, post-step kernel -18 us; all rounds: the last tiles' tails run after the
-// MMAs have finished, +62 us against -36 us).
-bool chain_tail_enabled() {
-  static const bool on = [] { const char* e = std::getenv("SIMSTEP_CHAIN_TAIL"); return e && e[0] == '1'; }();
-  return on;
-}
-
 bool chain_ok(const simstep_handle* h, long long rows_pad) {
-  if (chain_mode() == 0 || h->cg != 2 || h->L < 1 || h->L + 1 > kChainMaxLayers || !h->have_ensemble) return false;
+  if (!chain_enabled() || h->L < 1 || h->L + 1 > kChainMaxLayers || !h->have_ensemble) return false;
   static int l2_bytes[kMaxDevices] = {};
   int& l2 = l2_bytes[h->device % kMaxDevices];
   if (l2 == 0 && cudaDeviceGetAttribute(&l2, cudaDevAttrL2CacheSize, h->device) != cudaSuccess) l2 = 1;
@@ -548,7 +433,7 @@ bool chain_ok(const simstep_handle* h, long long rows_pad) {
   return weights + pairs * unit_bytes <= 0.9 * double(l2);
 }
 
-// The cost operand rows the step's tail also writes for input_type 'ss' (post kernels and the chain kernel's tail warps)
+// The cost operand rows the step's tail also writes for input_type 'ss' (post kernels)
 PostRff make_post_rff(const simstep_handle* h, bool fuse_rff) {
   PostRff rff{};
   if (fuse_rff) {
@@ -562,7 +447,7 @@ PostRff make_post_rff(const simstep_handle* h, bool fuse_rff) {
   return rff;
 }
 
-int launch_chain(simstep_handle* h, long long rows_pad, cudaStream_t st, const StepTail* step_tail, long long n) {
+int launch_chain(simstep_handle* h, long long rows_pad, cudaStream_t st) {
   ChainLaunch cl;
   cl.maps.x = h->tmap_x;
   cl.maps.h = h->tmap_h;
@@ -574,7 +459,6 @@ int launch_chain(simstep_handle* h, long long rows_pad, cudaStream_t st, const S
   ca.groups = h->N;
   ca.a_rows_per_group = int(h->cap_rows);
   ca.out_rows_per_group = int(h->cap_rows);
-  ca.h_slot = chain_mode() == 1 ? 0 : 1;
   ca.scale = h->cfg.transform ? h->out_scale_dev : nullptr;
   ca.shift = h->cfg.transform ? h->out_shift_dev : nullptr;
   for (int l = 0; l <= h->L; ++l) {
@@ -591,20 +475,12 @@ int launch_chain(simstep_handle* h, long long rows_pad, cudaStream_t st, const S
     if (l < h->L) ca.hidden_tiles += c.n_tiles;
   }
   cl.maps.w_final64 = h->layers[h->L].tmap_w64;
-  // L2 eviction priorities of the kernel's TMA traffic: weights and activations evict_last (every unit of a member
-  // re-reads the same 5 MB of weights, a unit re-reads its own rows layer after layer), measured -2.5 % on the launch
-  // (and +2.5 us on the post-step kernel, whose delta rows find less room in L2); marking x / the output evict_first
-  // on top was measured neutral and is off.  SIMSTEP_CHAIN_HINTS=<mask> overrides for A/B runs.
-  static const int hints = [] { const char* e = std::getenv("SIMSTEP_CHAIN_HINTS"); return e ? std::atoi(e) : 3; }();
-  ca.l2_hints = hints;
   // the last, partial round: when its units are at most half the pairs, two pairs share each of them
   // whole rounds run with the members of an env tile in sequence on one pair: all pairs then stream the SAME member's
-  // weights at any time (measured -1.5 % on the launch against members side by side; SIMSTEP_CHAIN_SEQ=0 for A/B)
-  static const bool seq = [] { const char* e = std::getenv("SIMSTEP_CHAIN_SEQ"); return !(e && e[0] == '0'); }();
+  // weights at any time (measured -1.5 % on the launch against members side by side)
   int pairs = 1;
-  chain_schedule(ca.m_tiles, ca.groups, h->sm_count / 2, seq,
-                 chain_mode() != 3 && ca.hidden_tiles <= kChainMaxDepTiles && h->chain_cnt != nullptr, &pairs,
-                 &ca.seq_rounds, &ca.tail_units);
+  chain_schedule(ca.m_tiles, ca.groups, h->sm_count / 2, ca.hidden_tiles <= kChainMaxDepTiles && h->chain_cnt != nullptr,
+                 &pairs, &ca.seq_rounds, &ca.tail_units);
   if (ca.tail_units > 0) {
     ca.tail_cnt = h->chain_cnt;
     int t = 0;
@@ -614,47 +490,19 @@ int launch_chain(simstep_handle* h, long long rows_pad, cudaStream_t st, const S
         ca.dep_ord[t] = static_cast<unsigned char>(ca.tiles_per_role[n & 1]++);
       }
   }
-  // The env step's tail inside this launch (gemm_chain.cuh, tail warps) for the env tiles of the whole rounds; the
-  // post-step kernel then only gets the rows of the remaining units.
-  static const int tail_keep = [] { const char* e = std::getenv("SIMSTEP_CHAIN_TAIL_KEEP"); return e ? std::atoi(e) : 1; }();
-  const int tail_rounds = ca.seq_rounds - tail_keep;   // the last round's rows stay with the post-step kernel
-  if (step_tail != nullptr && chain_tail_enabled() && tail_rounds > 0 && h->N == 4 && h->S % 2 == 0 &&
-      h->S <= kPostMaxElems && reinterpret_cast<uintptr_t>(step_tail->state) % 8 == 0 &&
-      reinterpret_cast<uintptr_t>(step_tail->next_state) % 8 == 0 && (step_tail->next_state == nullptr || step_tail->state != nullptr)) {
-    ChainTail& t = ca.tail;
-    t.enabled = 1;
-    t.rounds = tail_rounds;
-    t.delta = h->dws;
-    t.delta_rows = h->cap_rows;
-    t.DP = h->DP;
-    t.state = step_tail->state;
-    t.next_state = step_tail->next_state;
-    t.member = step_tail->member;
-    t.num_steps = step_tail->num_steps;
-    t.disc = step_tail->disc;
-    t.done = step_tail->done;
-    t.n_rows = n;
-    t.S = h->S;
-    t.tc = h->term;
-    t.rff = make_post_rff(h, step_tail->rff);
-    h->tail_rows_done = std::min<long long>(n, static_cast<long long>(tail_rounds) * pairs * kBlockM * 2);
-  }
   CU_TRY(h, launch_ensemble_chain(h->cfg.precision, h->cfg.activation != SIMSTEP_ACT_RELU, cl, h->sm_count, h->device, st));
   g_launches++;
   return SIMSTEP_OK;
 }
 
-// prep + all layer GEMMs for rows [0, n) of a chunk.  Without a tail (or when the tail cannot be fused) the
-// un-normalised member deltas are left in h->dws[N][cap_rows][DP]; with a fusable tail the final layer's launch
-// also runs the env step's tail and *tail_done is set.
+// prep + all layer GEMMs for rows [0, n) of a chunk: the un-normalised member deltas are left in
+// h->dws[N][cap_rows][DP].
 // w_stage != nullptr: the prep kernel also copies the cost weights into h->rff_wpad (no separate memcpy node
 // between the step's kernels).
 int run_ensemble_chunk(simstep_handle* h, const float* s, const float* a, long long n, cudaStream_t st,
-                       const float* w_stage = nullptr, int last_layer = -2, const StepTail* tail = nullptr,
-                       bool* tail_done = nullptr) {
+                       const float* w_stage = nullptr, int last_layer = -2) {
   if (last_layer == -2) last_layer = h->L;  // -1: input preparation only
   const long long rows_pad = round_up(n, h->row_align);
-  if (tail_done) *tail_done = false;
   {
   ProfScope ps(h, SIMSTEP_PROF_PREP, st);
   switch (h->cfg.precision) {
@@ -666,20 +514,14 @@ int run_ensemble_chunk(simstep_handle* h, const float* s, const float* a, long l
   CU_TRY(h, cudaGetLastError());
   ProfScope ps(h, SIMSTEP_PROF_ENSEMBLE_GEMM, st);
   h->forward_was_chain = false;
-  h->tail_rows_done = 0;
-  if (last_layer == h->L && chain_ok(h, rows_pad) && !(tail != nullptr && final_fused_ok(h, *tail))) {
+  if (last_layer == h->L && chain_ok(h, rows_pad)) {
     h->forward_was_chain = true;
-    return launch_chain(h, rows_pad, st, tail, n);
+    return launch_chain(h, rows_pad, st);
   }
   for (int l = 0; l <= last_layer; ++l) {
     const Layer& ly = h->layers[l];
-    if (l == h->L && tail != nullptr && final_fused_ok(h, *tail)) {
-      if (int rc = launch_final(h, n, rows_pad, *tail, st)) return rc;
-      if (tail_done) *tail_done = true;
-      break;
-    }
     GemmArgs ga{};
-    ga.m_tiles = int(rows_pad / (kBlockM * h->cg));
+    ga.m_tiles = int(rows_pad / (kBlockM * 2));
     ga.n_tiles = ly.o_pad / kBlockN;
     ga.groups = h->N;
     ga.kb_x = ly.kb_x;
@@ -691,17 +533,16 @@ int run_ensemble_chunk(simstep_handle* h, const float* s, const float* a, long l
     ga.bias = ly.bias;
     ga.out_rows_per_group = int(h->cap_rows);
     // weight tiles with the evict_last L2 priority: every env tile of a member re-reads them while the activations
-    // stream past (8 x (1024 x 4): -1 % on the five launches; neutral at 4 x (512 x 4); SIMSTEP_GEMM_B_HINT=0 for A/B)
-    static const int b_hint = [] { const char* e = std::getenv("SIMSTEP_GEMM_B_HINT"); return e ? std::atoi(e) : 1; }();
-    ga.b_evict_last = b_hint;
+    // stream past (8 x (1024 x 4): -1 % on the five launches; neutral at 4 x (512 x 4))
+    ga.b_evict_last = 1;
     int rc;
     if (l < h->L) {
       // bias + activation straight into this layer's K-slice of the concat buffer
       ga.out_col0 = ly.out_col0;
       rc = h->cfg.activation == SIMSTEP_ACT_RELU
-               ? launch_gemm<kEpiHidden>(h, h->cfg.precision, h->cg, h->tmap_x, h->tmap_h, ly.tmap_w, h->tmap_h, ga,
+               ? launch_gemm<kEpiHidden>(h, h->cfg.precision, h->tmap_x, h->tmap_h, ly.tmap_w, h->tmap_h, ga,
                                          h->sm_count, st)
-               : launch_gemm<kEpiHiddenTanh>(h, h->cfg.precision, h->cg, h->tmap_x, h->tmap_h, ly.tmap_w, h->tmap_h, ga,
+               : launch_gemm<kEpiHiddenTanh>(h, h->cfg.precision, h->tmap_x, h->tmap_h, ly.tmap_w, h->tmap_h, ga,
                                              h->sm_count, st);
     } else {
       ga.out_col0 = 0;
@@ -709,11 +550,10 @@ int run_ensemble_chunk(simstep_handle* h, const float* s, const float* a, long l
       ga.shift = h->cfg.transform ? h->out_shift_dev : nullptr;
       // the final layer is HBM-bound (every member re-reads its whole concat row for 226 outputs): run the members
       // of an env tile side by side (x comes from HBM once) and start with the rows whose last hidden slice the
-      // previous launch wrote last (still in L2).  SIMSTEP_FINAL_ORDER=0 restores the plain order for A/B runs.
-      static const bool order = [] { const char* e = std::getenv("SIMSTEP_FINAL_ORDER"); return !(e && e[0] == '0'); }();
-      ga.group_fastest = order ? 1 : 0;
-      ga.reverse = order ? 1 : 0;
-      rc = launch_gemm<kEpiFinal>(h, h->cfg.precision, h->cg, h->tmap_x, h->tmap_h, ly.tmap_w, h->tmap_dws, ga,
+      // previous launch wrote last (still in L2)
+      ga.group_fastest = 1;
+      ga.reverse = 1;
+      rc = launch_gemm<kEpiFinal>(h, h->cfg.precision, h->tmap_x, h->tmap_h, ly.tmap_w, h->tmap_dws, ga,
                                   h->sm_count, st);
     }
     if (rc) return rc;
@@ -725,20 +565,6 @@ int run_ensemble_chunk(simstep_handle* h, const float* s, const float* a, long l
 int launch_post(simstep_handle* h, const float* state, const int32_t* member, int32_t* num_steps, long long n,
                 float* next_state, float* disc, uint8_t* done, cudaStream_t st, bool fuse_rff = false) {
   if (h->S > kPostMaxElems) return fail(h, SIMSTEP_EINVAL, "state_dim > 256 is not supported by the post kernel");
-  // rows whose tail already ran inside the chain kernel (launch_chain) are skipped: everything below is offset by row0
-  const long long row0 = h->tail_rows_done;
-  h->tail_rows_done = 0;
-  if (row0 >= n) return SIMSTEP_OK;
-  if (row0 > 0) {
-    n -= row0;
-    if (state) state += row0 * h->S;
-    if (member) member += row0;
-    if (num_steps) num_steps += row0;
-    if (next_state) next_state += row0 * h->S;
-    if (disc) disc += row0;
-    if (done) done += row0;
-  }
-  const float* dws_base = h->dws + row0 * h->DP;
   ProfScope ps(h, SIMSTEP_PROF_POST, st);
   // one warp per row and one row per warp: the block scheduler balances the tail, no grid-stride quantisation
   const int blocks = int(std::min<long long>((n + kPostWarps - 1) / kPostWarps, 1LL << 30));
@@ -747,17 +573,14 @@ int launch_post(simstep_handle* h, const float* state, const int32_t* member, in
   const bool vec2 = (h->S % 2 == 0) && (reinterpret_cast<uintptr_t>(state) % 8 == 0) &&
                     (reinterpret_cast<uintptr_t>(next_state) % 8 == 0);
   if (fuse_rff && !vec2) return fail(h, SIMSTEP_EINVAL, "internal: fused RFF operand needs the float2 path");
-  PostRff rff = make_post_rff(h, fuse_rff);
-  if (rff.out != nullptr) rff.out = static_cast<char*>(rff.out) + size_t(row0) * rff.pitch * h->esize;
+  const PostRff rff = make_post_rff(h, fuse_rff);
   // TMA-staged persistent kernel (post_tma.cuh) whenever rows pair up into 16-byte granular spans
   const PostTmaPlan plan = post_tma_plan(h->S, h->DP, h->N);
-  static const bool tma_off = [] { const char* e = std::getenv("SIMSTEP_POST_TMA"); return e && e[0] == '0'; }();
-  const bool tma = !tma_off && plan.ok && vec2 && state != nullptr && next_state != nullptr &&
+  const bool tma = plan.ok && vec2 && state != nullptr && next_state != nullptr &&
                    reinterpret_cast<uintptr_t>(state) % 16 == 0;
   // the chain kernel writes the deltas in row order: the last rows are the ones still in L2, so the rows are walked
-  // backwards (SIMSTEP_POST_REVERSE=0: A/B); the per-layer final GEMM itself runs backwards, its LAST rows are row 0's
-  static const int post_reverse_on = [] { const char* e = std::getenv("SIMSTEP_POST_REVERSE"); return (e && e[0] == '0') ? 0 : 1; }();
-  const int post_reverse = (post_reverse_on && h->forward_was_chain) ? 1 : 0;
+  // backwards; the per-layer final GEMM itself runs backwards, its LAST rows are row 0's
+  const int post_reverse = h->forward_was_chain ? 1 : 0;
 #define POST_TMA_LAUNCH(NM, ET)                                                                                \
   do {                                                                                                         \
     auto kern = h->S == 226 ? post_step_tma_kernel<NM, ET, 226> : post_step_tma_kernel<NM, ET, 0>;             \
@@ -769,7 +592,7 @@ int launch_post(simstep_handle* h, const float* state, const int32_t* member, in
     }                                                                                                          \
     const long long pairs = (n + 1) / 2;                                                                       \
     const int grid = int(std::min<long long>((pairs + plan.rings - 1) / plan.rings, h->sm_count));             \
-    launch_pdl(kern, dim3(grid), dim3(plan.rings * 64), plan.smem, st, dws_base, h->cap_rows, h->DP, state, member, \
+    launch_pdl(kern, dim3(grid), dim3(plan.rings * 64), plan.smem, st, h->dws, h->cap_rows, h->DP, state, member, \
                num_steps, h->S, n, next_state, disc, done, h->term, rff, plan.stages, post_reverse);           \
   } while (0)
 #define POST_CASE(NM)                                                                                          \
@@ -779,10 +602,10 @@ int launch_post(simstep_handle* h, const float* state, const int32_t* member, in
       else if (h->cfg.precision == SIMSTEP_PREC_TF32) POST_TMA_LAUNCH(NM, ElemTF32);                           \
       else POST_TMA_LAUNCH(NM, ElemBF16);                                                                      \
     } else if (vec2)                                                                                           \
-      launch_pdl(post_step_kernel<NM, 2>, dim3(blocks), dim3(kPostWarps * 32), smem, st, dws_base, h->cap_rows, h->DP, \
+      launch_pdl(post_step_kernel<NM, 2>, dim3(blocks), dim3(kPostWarps * 32), smem, st, h->dws, h->cap_rows, h->DP, \
                  state, member, num_steps, h->S, n, next_state, disc, done, h->term, rff);                      \
     else                                                                                                       \
-      launch_pdl(post_step_kernel<NM, 1>, dim3(blocks), dim3(kPostWarps * 32), smem, st, dws_base, h->cap_rows, h->DP, \
+      launch_pdl(post_step_kernel<NM, 1>, dim3(blocks), dim3(kPostWarps * 32), smem, st, h->dws, h->cap_rows, h->DP, \
                  state, member, num_steps, h->S, n, next_state, disc, done, h->term, rff);                      \
     break;
   switch (h->N) {
@@ -839,20 +662,14 @@ CombineArgs make_combine(const simstep_handle* h, const float* disc, float lambd
   return c;
 }
 
-// SIMSTEP_RFF_FUSED_COMBINE=0: partial dots per n-tile + cost_combine_kernel (the round-1 sequence), for A/B runs
-bool rff_fused_combine() {
-  static const bool on = [] { const char* e = std::getenv("SIMSTEP_RFF_FUSED_COMBINE"); return !(e && e[0] == '0'); }();
-  return on;
-}
-
 // RFF GEMM over the packed rows of the chunk.  w_pad == nullptr: features only.  comb != nullptr: the epilogue
 // finishes cost / ipm / bonus itself (a CTA pair then runs all n-tiles of its rows back to back and carries the dot
-// product in registers); otherwise the per-n-tile partial dots go to h->rff_part for cost_combine_kernel.
+// product in registers).
 int launch_rff_gemm(simstep_handle* h, long long n, const float* w_pad, float* phi, cudaStream_t st,
                     const CombineArgs* comb = nullptr) {
   ProfScope ps(h, SIMSTEP_PROF_RFF_GEMM, st);
   GemmArgs ga{};
-  ga.m_tiles = int(round_up(n, h->row_align) / (kBlockM * h->cg));
+  ga.m_tiles = int(round_up(n, h->row_align) / (kBlockM * 2));
   ga.n_tiles = h->D_pad / kBlockN;
   ga.groups = 1;
   // K loop: [hi | lo] through the first map, then the hi block again (x_hi * W_lo) through the second; without the
@@ -868,13 +685,10 @@ int launch_rff_gemm(simstep_handle* h, long long n, const float* w_pad, float* p
   ga.out_pitch = h->D;
   ga.rows_valid = int(n);
   ga.cols_valid = h->D;
-  ga.rff_part = w_pad ? h->rff_part : nullptr;
-  ga.rff_part_stride = h->cap_rows;
   ga.rff_phi_scale = float(std::sqrt(2.0 / h->D));
   if (comb != nullptr && w_pad != nullptr) {
     ga.comb = *comb;
     ga.n_inner = ga.n_tiles;
-    ga.rff_part = nullptr;
   }
   if (h->feat_net) {
     // the head reads the last hidden layer's slice of the activation buffer
@@ -885,23 +699,11 @@ int launch_rff_gemm(simstep_handle* h, long long n, const float* w_pad, float* p
     ga.rff_tanh = h->feat_mode == SIMSTEP_HEAD_TANH_COS;
     ga.rff_linear = h->feat_mode == SIMSTEP_HEAD_LINEAR;
     if (ga.rff_linear) ga.rff_phi_scale = 1.f;
-    return launch_gemm<kEpiFeat>(h, h->cfg.precision, h->cg, h->tmap_x, h->tmap_h, h->tmap_rffw, h->tmap_h, ga,
+    return launch_gemm<kEpiFeat>(h, h->cfg.precision, h->tmap_x, h->tmap_h, h->tmap_rffw, h->tmap_h, ga,
                                 h->sm_count, st);
   }
-  return launch_gemm<kEpiRff>(h, h->cfg.precision, h->cg, h->tmap_rffin, h->tmap_rffin, h->tmap_rffw, h->tmap_rffin, ga,
+  return launch_gemm<kEpiRff>(h, h->cfg.precision, h->tmap_rffin, h->tmap_rffin, h->tmap_rffw, h->tmap_rffin, ga,
                               h->sm_count, st);
-}
-
-// RFF GEMM + bonus combine for the packed rows of a chunk (one launch, or two with SIMSTEP_RFF_FUSED_COMBINE=0)
-int launch_rff_cost(simstep_handle* h, long long n, const CombineArgs& comb, cudaStream_t st) {
-  if (rff_fused_combine()) return launch_rff_gemm(h, n, h->rff_wpad, nullptr, st, &comb);
-  if (int rc = launch_rff_gemm(h, n, h->rff_wpad, nullptr, st)) return rc;
-  ProfScope ps(h, SIMSTEP_PROF_COMBINE, st);
-  launch_pdl(cost_combine_kernel, dim3(grid_for(n, 256, h->sm_count)), dim3(256), 0, st, h->rff_part, h->cap_rows,
-             h->D_pad / kBlockN, n, comb);
-  g_launches++;
-  CU_TRY(h, cudaGetLastError());
-  return SIMSTEP_OK;
 }
 
 int stage_w(simstep_handle* h, const float* w_dev, cudaStream_t st) {
@@ -971,7 +773,7 @@ int upload_layer(simstep_handle* h, int l, const float* const* weights_host, con
                               ly.k_pad, kBlockN / 4))
     return rc;
   return encode_operand(h, &ly.tmap_w, h->cfg.precision, ly.w, ly.k_pad, static_cast<long long>(h->N) * ly.o_pad,
-                        ly.k_pad, kBlockN / h->cg);
+                        ly.k_pad, kBlockN / 2);
 }
 
 void free_clip(simstep_handle* h);
@@ -1036,9 +838,8 @@ int simstep_create(const simstep_config* cfg, simstep_handle** out) {
   h->sm_count = prop.multiProcessorCount;
   h->esize = cfg->precision == SIMSTEP_PREC_TF32 ? 4 : 2;
   h->bk = 128 / h->esize;
-  h->cg = gemm_cta_group();
   { const char* e = std::getenv("SIMSTEP_DEBUG_GUARDS"); h->guards_on = e && e[0] == '1'; }
-  h->row_align = kBlockM * h->cg;
+  h->row_align = kBlockM * 2;
   h->S = cfg->state_dim;
   h->A = cfg->action_dim;
   h->N = cfg->n_models;
@@ -1205,9 +1006,9 @@ int simstep_load_rff(simstep_handle* h, int32_t feature_dim, int32_t in_dim, con
   DeviceScope dev_scope(h->device);  // parameters live on the handle's device; the caller's current device is restored
   CU_TRY(h, cudaDeviceSynchronize());
   cudaFree(h->rff_w); cudaFree(h->rff_b); cudaFree(h->rff_wpad); cudaFree(h->colsum_partial);
-  ws_free(h, h->rffin); ws_free(h, h->rff_part);
+  ws_free(h, h->rffin);
   h->rff_w = nullptr; h->rff_b = nullptr; h->rff_wpad = nullptr; h->colsum_partial = nullptr;
-  h->rffin = nullptr; h->rff_part = nullptr;
+  h->rffin = nullptr;
   h->have_rff = false;
   h->D = feature_dim;
   h->D_pad = int(round_up(feature_dim, kBlockN));
@@ -1248,7 +1049,7 @@ int simstep_load_rff(simstep_handle* h, int32_t feature_dim, int32_t in_dim, con
   }
   CU_TRY(h, cudaDeviceSynchronize());
   cudaFree(tmp);
-  int rc = encode_operand(h, &h->tmap_rffw, h->cfg.precision, h->rff_w, h->RKT, h->D_pad, h->RKT, kBlockN / h->cg);
+  int rc = encode_operand(h, &h->tmap_rffw, h->cfg.precision, h->rff_w, h->RKT, h->D_pad, h->RKT, kBlockN / 2);
   if (rc) return rc;
   h->have_rff = true;
   return SIMSTEP_OK;
@@ -1273,9 +1074,9 @@ int simstep_load_feature_net(simstep_handle* h, const float* const* weights_host
   if (!h->tf_dev) CU_TRY(h, cudaMalloc(&h->tf_dev, size_t(2 * h->S + 4) * sizeof(float)));
   // head = cos-feature layer over the last hidden activations (reuses the random-feature GEMM epilogue)
   cudaFree(h->rff_w); cudaFree(h->rff_b); cudaFree(h->rff_wpad); cudaFree(h->colsum_partial);
-  ws_free(h, h->rffin); ws_free(h, h->rff_part);
+  ws_free(h, h->rffin);
   h->rff_w = nullptr; h->rff_b = nullptr; h->rff_wpad = nullptr; h->colsum_partial = nullptr;
-  h->rffin = nullptr; h->rff_part = nullptr;
+  h->rffin = nullptr;
   h->have_rff = false;
   const Layer& fin = h->layers[h->L];
   const int in_dim = h->L > 0 ? h->cfg.hidden[h->L - 1] : h->S;
@@ -1305,7 +1106,7 @@ int simstep_load_feature_net(simstep_handle* h, const float* const* weights_host
   CU_TRY(h, cudaDeviceSynchronize());
   cudaFree(tmp);
   if (rc) return rc;
-  rc = encode_operand(h, &h->tmap_rffw, h->cfg.precision, h->rff_w, h->RKT, h->D_pad, h->RKT, kBlockN / h->cg);
+  rc = encode_operand(h, &h->tmap_rffw, h->cfg.precision, h->rff_w, h->RKT, h->D_pad, h->RKT, kBlockN / 2);
   if (rc) return rc;
   free_workspace(h);
   h->feat_mode = head_mode;
@@ -1359,7 +1160,7 @@ int simstep_debug_chain_schedule(int32_t m_tiles, int32_t groups, int32_t sm_cou
   a.m_tiles = m_tiles;
   a.groups = groups;
   int pairs = 1;
-  chain_schedule(m_tiles, groups, sm_count / 2, true, true, &pairs, &a.seq_rounds, &a.tail_units);
+  chain_schedule(m_tiles, groups, sm_count / 2, true, &pairs, &a.seq_rounds, &a.tail_units);
   *pairs_out = pairs;
   *seq_rounds_out = a.seq_rounds;
   *tail_units_out = a.tail_units;
@@ -1381,7 +1182,7 @@ int simstep_debug_chain_schedule(int32_t m_tiles, int32_t groups, int32_t sm_cou
 int simstep_forward_launches(const simstep_handle* h, int64_t n_envs, int32_t* launches_out) {
   if (!h || !launches_out || n_envs < 1) return SIMSTEP_EINVAL;
   const long long rows = std::min<long long>(round_up(n_envs, h->row_align), chunk_limit(h));
-  *launches_out = chain_ok(h, rows) && !final_fused_enabled() ? 1 : h->L + 1;
+  *launches_out = chain_ok(h, rows) ? 1 : h->L + 1;
   return SIMSTEP_OK;
 }
 
@@ -1424,12 +1225,8 @@ int simstep_discrepancy(simstep_handle* h, const float* state_dev, const float* 
   if ((rc = ensure_workspace(h, n_envs))) return rc;
   for (long long r0 = 0; r0 < n_envs; r0 += h->cap_rows) {
     const long long n = std::min<long long>(h->cap_rows, n_envs - r0);
-    StepTail tail;
-    tail.disc = disc_dev + r0;
-    bool tail_done = false;
-    if ((rc = run_ensemble_chunk(h, state_dev + r0 * h->S, action_dev + r0 * h->A, n, st, nullptr, -2, &tail, &tail_done)))
-      return rc;
-    if (!tail_done && (rc = launch_post(h, nullptr, nullptr, nullptr, n, nullptr, disc_dev + r0, nullptr, st))) return rc;
+    if ((rc = run_ensemble_chunk(h, state_dev + r0 * h->S, action_dev + r0 * h->A, n, st))) return rc;
+    if ((rc = launch_post(h, nullptr, nullptr, nullptr, n, nullptr, disc_dev + r0, nullptr, st))) return rc;
   }
   return SIMSTEP_OK;
 }
@@ -1445,17 +1242,11 @@ int simstep_step(simstep_handle* h, const float* state_dev, const float* action_
   if ((rc = ensure_workspace(h, n_envs))) return rc;
   for (long long r0 = 0; r0 < n_envs; r0 += h->cap_rows) {
     const long long n = std::min<long long>(h->cap_rows, n_envs - r0);
-    StepTail tail;
-    tail.state = state_dev + r0 * h->S;
-    tail.next_state = next_state_dev + r0 * h->S;
-    tail.member = member_dev ? member_dev + r0 : nullptr;
-    tail.num_steps = num_steps_dev ? num_steps_dev + r0 : nullptr;
-    tail.disc = disc_dev ? disc_dev + r0 : nullptr;
-    tail.done = done_dev ? done_dev + r0 : nullptr;
-    bool tail_done = false;
-    if ((rc = run_ensemble_chunk(h, tail.state, action_dev + r0 * h->A, n, st, nullptr, -2, &tail, &tail_done))) return rc;
-    if (!tail_done && (rc = launch_post(h, tail.state, tail.member, tail.num_steps, n, tail.next_state, tail.disc,
-                                        tail.done, st)))
+    const float* s = state_dev + r0 * h->S;
+    if ((rc = run_ensemble_chunk(h, s, action_dev + r0 * h->A, n, st))) return rc;
+    if ((rc = launch_post(h, s, member_dev ? member_dev + r0 : nullptr, num_steps_dev ? num_steps_dev + r0 : nullptr, n,
+                          next_state_dev + r0 * h->S, disc_dev ? disc_dev + r0 : nullptr, done_dev ? done_dev + r0 : nullptr,
+                          st)))
       return rc;
   }
   return SIMSTEP_OK;
@@ -1482,18 +1273,9 @@ int simstep_step_cost(simstep_handle* h, const float* state_dev, const float* ac
     // input_type 'ss' with float2-able rows: the step's tail writes the cost features' operand rows itself
     const bool fuse = h->rff_col2 > 0 && h->S % 2 == 0 && reinterpret_cast<uintptr_t>(s) % 8 == 0 &&
                       reinterpret_cast<uintptr_t>(s2) % 8 == 0;
-    StepTail tail;
-    tail.state = s;
-    tail.next_state = s2;
-    tail.member = member_dev ? member_dev + r0 : nullptr;
-    tail.num_steps = num_steps_dev ? num_steps_dev + r0 : nullptr;
-    tail.disc = disc_dev + r0;
-    tail.done = done_dev ? done_dev + r0 : nullptr;
-    tail.rff = fuse;
-    bool tail_done = false;
-    if ((rc = run_ensemble_chunk(h, s, a, n, st, r0 == 0 ? w_dev : nullptr, -2, &tail, &tail_done))) return rc;
-    if (!tail_done &&
-        (rc = launch_post(h, s, tail.member, tail.num_steps, n, s2, tail.disc, tail.done, st, fuse)))
+    if ((rc = run_ensemble_chunk(h, s, a, n, st, r0 == 0 ? w_dev : nullptr))) return rc;
+    if ((rc = launch_post(h, s, member_dev ? member_dev + r0 : nullptr, num_steps_dev ? num_steps_dev + r0 : nullptr, n,
+                          s2, disc_dev + r0, done_dev ? done_dev + r0 : nullptr, st, fuse)))
       return rc;
     if (!fuse) {
       RffSrc src;
@@ -1503,7 +1285,7 @@ int simstep_step_cost(simstep_handle* h, const float* state_dev, const float* ac
     const CombineArgs comb = make_combine(h, disc_dev + r0, lambda_b, threshold, c_min, c_max, clamp_cost, nullptr,
                                           cost_dev ? cost_dev + r0 : nullptr, ipm_dev ? ipm_dev + r0 : nullptr,
                                           bonus_dev ? bonus_dev + r0 : nullptr);
-    if ((rc = launch_rff_cost(h, n, comb, st))) return rc;
+    if ((rc = launch_rff_gemm(h, n, h->rff_wpad, nullptr, st, &comb))) return rc;
   }
   return SIMSTEP_OK;
 }
@@ -1572,7 +1354,7 @@ int simstep_bonus_cost(simstep_handle* h, const float* x_dev, const float* disc_
             : make_combine(h, disc_dev + r0, lambda_b, threshold, c_min, c_max, clamp_cost, nullptr,
                            cost_dev ? cost_dev + r0 : nullptr, ipm_dev ? ipm_dev + r0 : nullptr,
                            bonus_dev ? bonus_dev + r0 : nullptr);
-    if ((rc = launch_rff_cost(h, n, comb, st))) return rc;
+    if ((rc = launch_rff_gemm(h, n, h->rff_wpad, nullptr, st, &comb))) return rc;
   }
   return SIMSTEP_OK;
 }
@@ -1619,10 +1401,9 @@ int simstep_debug_gemm(int32_t precision, int32_t groups, int64_t m, int32_t n, 
     return fail(nullptr, SIMSTEP_EINVAL, "bad argument");
   simstep_handle* h = nullptr;  // errors go to the create-error slot
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int cg = gemm_cta_group();
   const int es = precision == SIMSTEP_PREC_TF32 ? 4 : 2;
   const int bk = 128 / es;
-  const long long m_pad = round_up(m, kBlockM * cg), n_pad = round_up(n, kBlockN), k_pad = round_up(k, 64);
+  const long long m_pad = round_up(m, kBlockM * 2), n_pad = round_up(n, kBlockN), k_pad = round_up(k, 64);
   cudaDeviceProp prop;
   int dev = 0;
   CU_TRY(h, cudaGetDevice(&dev));
@@ -1657,11 +1438,11 @@ int simstep_debug_gemm(int32_t precision, int32_t groups, int64_t m, int32_t n, 
   }
   CUtensorMap ta, tb, td;
   if (!rc) rc = encode_operand(h, &ta, precision, ap, k_pad, groups * m_pad, k_pad, kBlockM);
-  if (!rc) rc = encode_operand(h, &tb, precision, bp, k_pad, groups * n_pad, k_pad, kBlockN / cg);
+  if (!rc) rc = encode_operand(h, &tb, precision, bp, k_pad, groups * n_pad, k_pad, kBlockN / 2);
   if (!rc) rc = encode_operand(h, &td, SIMSTEP_PREC_TF32, dp, n_pad, groups * m_pad, n_pad, kBlockM);
   if (!rc) {
     GemmArgs ga{};
-    ga.m_tiles = int(m_pad / (kBlockM * cg));
+    ga.m_tiles = int(m_pad / (kBlockM * 2));
     ga.n_tiles = int(n_pad / kBlockN);
     ga.groups = groups;
     ga.kb_x = 0;
@@ -1672,7 +1453,7 @@ int simstep_debug_gemm(int32_t precision, int32_t groups, int64_t m, int32_t n, 
     ga.bias = biasp;
     ga.out_rows_per_group = int(m_pad);
     ga.out_col0 = 0;
-    rc = launch_gemm<kEpiFinal>(h, precision, cg, ta, ta, tb, td, ga, prop.multiProcessorCount, st);
+    rc = launch_gemm<kEpiFinal>(h, precision, ta, ta, tb, td, ga, prop.multiProcessorCount, st);
   }
   if (!rc) {
     const long long total = static_cast<long long>(groups) * m * n;

@@ -10,11 +10,11 @@ namespace simstep {
 
 namespace {
 
-template <typename E, bool TANH, int TAIL_NM>
+template <typename E, bool TANH>
 cudaError_t launch_t(const ChainLaunch& cl, int sm_count, int device, cudaStream_t st) {
   static bool attr_set[64] = {};  // function attributes are per device
-  auto kern = ensemble_chain_kernel<E, TANH, TAIL_NM>;
-  constexpr size_t smem = GemmPlan<2, 1, true>::smem_bytes() + (TAIL_NM > 0 ? kChainTailSmem : 0);
+  auto kern = ensemble_chain_kernel<E, TANH>;
+  constexpr size_t smem = GemmPlan<1, true>::smem_bytes();
   bool& done = attr_set[device % 64];
   if (!done) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
@@ -26,7 +26,7 @@ cudaError_t launch_t(const ChainLaunch& cl, int sm_count, int device, cudaStream
   const int pairs = units < sm_count / 2 ? units : sm_count / 2;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(unsigned(pairs * 2));
-  cfg.blockDim = dim3(kGemmThreads + (TAIL_NM > 0 ? kChainTailWarps * 32 : 0));
+  cfg.blockDim = dim3(kGemmThreads);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
   cudaLaunchAttribute attr[2];
@@ -43,10 +43,7 @@ cudaError_t launch_t(const ChainLaunch& cl, int sm_count, int device, cudaStream
 
 template <typename E>
 cudaError_t launch_a(bool tanh_act, const ChainLaunch& cl, int sm_count, int device, cudaStream_t st) {
-  // the fused tail exists for the four-member ensemble (the north-star shape); other sizes keep the post-step kernel
-  if (cl.args.tail.enabled && cl.args.groups == 4)
-    return tanh_act ? launch_t<E, true, 4>(cl, sm_count, device, st) : launch_t<E, false, 4>(cl, sm_count, device, st);
-  return tanh_act ? launch_t<E, true, 0>(cl, sm_count, device, st) : launch_t<E, false, 0>(cl, sm_count, device, st);
+  return tanh_act ? launch_t<E, true>(cl, sm_count, device, st) : launch_t<E, false>(cl, sm_count, device, st);
 }
 
 }  // namespace

@@ -1,7 +1,6 @@
 // HBM-bound kernels around the ensemble GEMMs: input normalisation, the fused
-// next-state / discrepancy / termination kernel, RFF operand packing, the
-// cost combine and small reductions.  All row-parallel, coalesced, no atomics
-// on the data path.
+// next-state / discrepancy / termination kernel, RFF operand packing and small
+// reductions.  All row-parallel, coalesced, no atomics on the data path.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -269,10 +268,8 @@ __device__ __forceinline__ void post_rff_store(const PostRff& r, long long row, 
 //   delta  [NM][delta_rows][SP] fp32 workspace of the final GEMM, row = chunk-local
 //   state  [E][S], next_state [E][S] (may alias state)
 // VEC = 2 when S is even: every row then starts 8-byte aligned and lanes move float2.
-// One env row, one warp: the body of post_step_kernel, also run by the tail warps of the column-fused forward kernel
-// (gemm_chain.cuh) on rows whose member deltas that same kernel has just stored - CG_LOADS reads them with ld.global.cg
-// (L2, never a stale L1 line).  srow: this warp's shared-memory row of (S + 3) & ~3 floats.
-template <int NM, int VEC, bool CG_LOADS>
+// One env row, one warp: the body of post_step_kernel.  srow: this warp's shared-memory row of (S + 3) & ~3 floats.
+template <int NM, int VEC>
 __device__ __forceinline__ void post_row_warp(const float* __restrict__ delta, long long delta_rows, int SP,
                                               const float* state, const int32_t* __restrict__ member,
                                               int32_t* num_steps, int S, long long row, float* next_state,
@@ -289,7 +286,7 @@ __device__ __forceinline__ void post_row_warp(const float* __restrict__ delta, l
 #pragma unroll
     for (int i = 0; i < kPerLane; ++i) {
       const int j = lane + 32 * i;
-      d[m][i] = (j < nvec) ? (CG_LOADS ? __ldcg(drow + j) : __ldg(drow + j)) : PostVec<VEC>::zero();
+      d[m][i] = (j < nvec) ? __ldg(drow + j) : PostVec<VEC>::zero();
     }
   }
   V sv[kPerLane];
@@ -415,7 +412,7 @@ post_step_kernel(const float* __restrict__ delta, long long delta_rows, int SP, 
   ptx::grid_dep_wait();
   ptx::grid_dep_launch();
   for (long long row = warp_global; row < n_rows; row += n_warps)
-    post_row_warp<NM, VEC, false>(delta, delta_rows, SP, state, member, num_steps, S, row, next_state, disc, done, tc,
+    post_row_warp<NM, VEC>(delta, delta_rows, SP, state, member, num_steps, S, row, next_state, disc, done, tc,
                                   rff, srow, lane);
 }
 
@@ -432,20 +429,6 @@ static __global__ void extract_delta_kernel(const float* __restrict__ ws, long l
     const int m = static_cast<int>(t / n_rows);
     out[(static_cast<long long>(m) * out_rows + out_row0 + row) * S + j] =
         ws[(static_cast<long long>(m) * ws_rows + row) * SP + j];
-  }
-}
-
-// ---- cost combine (reference milo/milo/linear_cost.py:96-103, 130-147) ------
-
-static __global__ void cost_combine_kernel(const float* __restrict__ part, long long part_stride, int n_parts,
-                                           long long n_rows, const CombineArgs comb) {
-  ptx::grid_dep_wait();
-  ptx::grid_dep_launch();
-  for (long long row = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; row < n_rows;
-       row += static_cast<long long>(gridDim.x) * blockDim.x) {
-    float dot = 0.f;
-    for (int t = 0; t < n_parts; ++t) dot += part[t * part_stride + row];
-    combine_row(comb, row, dot);
   }
 }
 

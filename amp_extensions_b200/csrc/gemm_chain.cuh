@@ -16,10 +16,11 @@
 //   * the activation rows of a unit are written and read back by the same SM pair within tens of microseconds, i.e.
 //     they are L2 hits: the final layer (HBM-bound when launched alone: it re-reads a member's whole 4.6 KB concat
 //     row for 226 outputs) and the short first layer (epilogue-bound alone) disappear into the tensor-bound average.
-//   * slot mode (h_slot != 0): a pair keeps its unit's activation rows in ITS OWN 256-row slot of the activation
-//     buffer instead of at the unit's rows - the live part of the buffer is then 74 pairs x 256 rows x 4 KB = 78 MB
-//     whatever the batch.  Safe without extra synchronisation: the first store into the slot for unit u+1 follows an
-//     MMA that was issued after every MMA of unit u, and those had consumed every load from the slot.
+//   * ACTIVATION SLOTS: a pair keeps a whole unit's activation rows in ITS OWN 256-row slot of the activation buffer
+//     instead of at the unit's rows - the live part of the buffer is then 74 pairs x 256 rows x 4 KB = 78 MB whatever
+//     the batch.  Safe without extra synchronisation: the first store into the slot for unit u+1 follows an MMA that
+//     was issued after every MMA of unit u, and those had consumed every load from the slot.  (The shared units of the
+//     last round, below, keep their rows at the unit's env rows, where both pairs find them.)
 //   * THE LAST, PARTIAL ROUND.  628 units of the bench batch are 8 rounds of 74 pairs plus 36 units; run as a ninth
 //     round they leave 38 pairs idle for a whole unit (6 % of the launch).  When the T left-over units are at most half
 //     the pairs, TWO pairs share each of them: pair 2u + p computes the n-tiles n % 2 == p of every hidden layer and the
@@ -32,22 +33,26 @@
 //
 //   * ORDER OF THE UNITS.  Whole rounds take the members of an env tile in sequence on one pair (all pairs then stream
 //     the same member's weights at any time: 1.5 % faster than members side by side); the units that do not fill a
-//     whole number of such rounds go round-robin, and the last partial round is shared as described above.  Because an
-//     env tile's members meet inside one CTA this way, the env step's tail can run here too (ChainTail: four extra
-//     warps, opt-in - measured break-even, see DESIGN.md section 5).
+//     whole number of such rounds go round-robin, and the last partial round is shared as described above.
+//   * L2 PRIORITIES.  Weights and activations are loaded and stored evict_last: every unit of a member re-reads the
+//     same weights, a unit re-reads its own rows layer after layer (measured 2.5 % faster on the launch, and 2.5 us
+//     slower on the post-step kernel, whose delta rows find less room in L2; marking x and the output evict_first on
+//     top was measured neutral).
 //
 // Tried and dropped: a cluster of FOUR CTAs per unit (both pairs on one unit throughout, the A operand multicast between
 // them: 25 % fewer bytes out of L2, bit-identical results).  Only 33 such clusters are co-schedulable on the 148 SMs
 // (GPC sizes), 132 SMs instead of 148, and the launch was 12 % slower; the multicast itself changed nothing.  Also
 // tried: running the first layer of the NEXT unit in front of the final layer of the current one (two slots per pair),
-// so that the short first layer's epilogues drain behind 36 k-blocks of MMAs - bit-identical, 1 % slower.
+// so that the short first layer's epilogues drain behind 36 k-blocks of MMAs - bit-identical, 1 % slower.  And the env
+// step's tail (next state, discrepancy, termination) on four extra warps of this kernel, for the env tiles whose
+// members had all run on one pair: correct, and break-even, because this kernel is bound by the L2 -> SM path that the
+// tail's bytes need as well (DESIGN.md section 5).
 //
 // Pipeline, barriers, TMEM double-buffering, the operand ring and the TMA-store epilogue are those of
-// gemm_tcgen05.cuh (CG = 2, one epilogue group); the accumulation order of every output element is the same as in
+// gemm_tcgen05.cuh (one epilogue group); the accumulation order of every output element is the same as in
 // the per-layer launches, so the results are bit-identical to them.
 #pragma once
 #include <type_traits>
-#include "elementwise.cuh"
 #include "gemm_tcgen05.cuh"
 
 #ifndef SIMSTEP_MAX_HIDDEN
@@ -67,44 +72,18 @@ struct ChainLayer {
 };
 
 constexpr int kChainMaxDepTiles = 64;
-constexpr int kChainTailWarps = 4;
-constexpr int kChainTailSmem = kChainTailWarps * (kPostMaxElems + 4) * 4;  // one state row per tail warp
-
-// The env step's tail (next state, discrepancy, termination, cost operand rows: what post_step_*_kernel does) for the
-// env tiles whose members all ran on this CTA pair: four extra warps pick a tile's 128 rows up when the last member's
-// deltas have been stored and run post_row_warp on them while the pair is already multiplying the next env tile.
-struct ChainTail {
-  int enabled;
-  int rounds;              // the first `rounds` whole rounds (the last round's tail would run after the kernel's MMAs are done)
-  const float* delta;      // the delta workspace [N][delta_rows][DP] this launch writes
-  long long delta_rows;
-  int DP;
-  const float* state;
-  float* next_state;
-  const int32_t* member;
-  int32_t* num_steps;
-  float* disc;
-  uint8_t* done;
-  long long n_rows;
-  int S;
-  TermConst tc;
-  PostRff rff;
-};
 
 struct ChainArgs {
   int n_layers;            // hidden layers + the final one (the last entry of layer[])
   int m_tiles, groups;
-  int a_rows_per_group;    // row stride between members in the activation buffer (ignored in slot mode)
+  int a_rows_per_group;    // row stride between members in the activation buffer (shared units; whole units use slots)
   int out_rows_per_group;  // row stride between members in the final output (delta workspace)
-  int h_slot;              // slot mode: activation rows live at pair * 256 (+ 128 for the second CTA)
   int hidden_tiles;        // hidden tiles per unit (sum of n_tiles over the hidden layers)
-  int l2_hints;            // bit 0: weights evict_last, 1: activations evict_last, 2: x evict_first, 3: output evict_first
   const float* scale;      // final layer: [n_tiles * kBlockN] or nullptr (dynamics.py:231-232)
   const float* shift;
   // the last, partial round: units [units - tail_units, units) are shared by two pairs each (0: plain extra round)
   int tail_units;
   int seq_rounds;          // whole rounds run with the members of an env tile in sequence on one pair (0: none)
-  ChainTail tail;          // the env step's tail for the rows of those rounds (TAIL_NM > 0 instantiations)
   int tiles_per_role[2];                      // hidden tiles role p stores per shared unit
   unsigned char dep_role[kChainMaxDepTiles];  // column tile T of the activation buffer: the role that stores it ...
   unsigned char dep_ord[kChainMaxDepTiles];   // ... and its ordinal among that role's tiles of the unit
@@ -151,12 +130,12 @@ struct ChainItem {
 // Host side of the schedule: how many CTA pairs run, how many whole rounds take an env tile's members in sequence, and how
 // many units of the last partial round are shared between two pairs (0: it runs as a plain round).  Used by the launcher
 // and by simstep_debug_chain_schedule (the CPU test of this arithmetic).
-inline void chain_schedule(int m_tiles, int groups, int max_pairs, bool seq, bool share, int* pairs, int* seq_rounds,
+inline void chain_schedule(int m_tiles, int groups, int max_pairs, bool share, int* pairs, int* seq_rounds,
                            int* tail_units) {
   const int units = m_tiles * groups;
   *pairs = units < max_pairs ? units : max_pairs;
   if (*pairs < 1) *pairs = 1;
-  *seq_rounds = (seq && units > *pairs) ? m_tiles / *pairs : 0;
+  *seq_rounds = units > *pairs ? m_tiles / *pairs : 0;
   const int tail = (units - *seq_rounds * *pairs * groups) % *pairs;
   *tail_units = (share && tail > 0 && 2 * tail <= *pairs) ? tail : 0;
 }
@@ -182,12 +161,12 @@ __host__ __device__ __forceinline__ bool chain_item(const ChainArgs& a, int pair
   return false;
 }
 
-template <typename E, bool TANH, int TAIL_NM>
-__global__ void __launch_bounds__(kGemmThreads + (TAIL_NM > 0 ? kChainTailWarps * 32 : 0), 1)
+template <typename E, bool TANH>
+__global__ void __launch_bounds__(kGemmThreads, 1)
 ensemble_chain_kernel(const __grid_constant__ ChainMaps maps, const __grid_constant__ ChainArgs args) {
   constexpr int CG = 2;
-  using S = GemmShape<CG>;
-  using Plan = GemmPlan<CG, 1, true>;
+  using S = GemmShape;
+  using Plan = GemmPlan<1, true>;
   constexpr int BK = ElemDims<E>::kBlockK;
   constexpr int UK = ElemDims<E>::kUmmaK;
   constexpr int kMmasPerBlock = BK / UK;
@@ -210,8 +189,6 @@ ensemble_chain_kernel(const __grid_constant__ ChainMaps maps, const __grid_const
   uint64_t* tmem_empty_bar = bars + 2 * kStages + 2;
   uint32_t* tmem_base_smem = reinterpret_cast<uint32_t*>(bars + 2 * kStages + 4);
   uint32_t* stored_cnt = tmem_base_smem + 1;  // hidden tiles of THIS CTA whose stores have completed
-  uint32_t* tail_ready = tmem_base_smem + 2;  // env tiles of THIS CTA whose members' deltas are all stored
-  float* tail_rows = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(bars) + 256);  // [kChainTailWarps][kPostMaxElems + 4]
 
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
   const int lane = threadIdx.x & 31;
@@ -228,7 +205,6 @@ ensemble_chain_kernel(const __grid_constant__ ChainMaps maps, const __grid_const
       ptx::mbar_init(&tmem_empty_bar[a], kNumEpiWarps * CG);
     }
     *stored_cnt = 0;
-    *tail_ready = 0;
     ptx::fence_barrier_init();
     ptx::prefetch_tensormap(&maps.x);
     ptx::prefetch_tensormap(&maps.h);
@@ -236,8 +212,8 @@ ensemble_chain_kernel(const __grid_constant__ ChainMaps maps, const __grid_const
     for (int l = 0; l < args.n_layers; ++l) ptx::prefetch_tensormap(&maps.w[l]);
   }
   if (warp == 1) {
-    ptx::tmem_alloc<CG>(tmem_base_smem, kTmemCols);
-    ptx::tmem_relinquish<CG>();
+    ptx::tmem_alloc(tmem_base_smem, kTmemCols);
+    ptx::tmem_relinquish();
   }
   ptx::tcgen05_fence_before();
   ptx::cluster_sync();
@@ -263,7 +239,7 @@ ensemble_chain_kernel(const __grid_constant__ ChainMaps maps, const __grid_const
     if (ptx::elect_one()) {
       int stage = 0;
       uint32_t phase = 0;
-      const uint64_t pol_last = l2_policy_evict_last(), pol_first = l2_policy_evict_first();
+      const uint64_t pol_last = l2_policy_evict_last();
       uint32_t have = 0;       // last value seen in stored_cnt
       uint32_t done_tiles = 0; // hidden tiles this CTA stored in the items before the current one
       ChainItem item;
@@ -271,7 +247,7 @@ ensemble_chain_kernel(const __grid_constant__ ChainMaps maps, const __grid_const
         const bool shared = item.role >= 0;
         const int g = item.unit % args.groups;
         const int m_row = ((item.unit / args.groups) * CG + int(cta_rank)) * kBlockM;
-        const int row_ah = (args.h_slot && !shared) ? slot_row : g * args.a_rows_per_group + m_row;
+        const int row_ah = shared ? g * args.a_rows_per_group + m_row : slot_row;
         // shared unit: the partner's tile counter for this row half (polled), zeroed again when this item is through
         unsigned int* partner_cnt = nullptr;
         uint32_t have_partner = 0;
@@ -319,15 +295,9 @@ ensemble_chain_kernel(const __grid_constant__ ChainMaps maps, const __grid_const
               uint8_t* sa = smem_tiles + size_t(stage) * S::kStageBytes;
               uint8_t* sb = sa + kABytes;
               if (leader) ptx::mbar_arrive_expect_tx(&full_bar[stage], stage_bytes);
-              if (kb < ly.kb_x) {
-                if (args.l2_hints & 4) tma_load_2d_pair_hint(sa, &maps.x, &full_bar[stage], kb * BK, m_row, pol_first);
-                else ptx::tma_load_2d<CG>(sa, &maps.x, &full_bar[stage], kb * BK, m_row);
-              } else {
-                if (args.l2_hints & 2) tma_load_2d_pair_hint(sa, &maps.h, &full_bar[stage], hk * BK, row_ah, pol_last);
-                else ptx::tma_load_2d<CG>(sa, &maps.h, &full_bar[stage], hk * BK, row_ah);
-              }
-              if (args.l2_hints & 1) tma_load_2d_pair_hint(sb, wmap, &full_bar[stage], kb * BK, row_b, pol_last);
-              else ptx::tma_load_2d<CG>(sb, wmap, &full_bar[stage], kb * BK, row_b);
+              if (kb < ly.kb_x) ptx::tma_load_2d(sa, &maps.x, &full_bar[stage], kb * BK, m_row);
+              else tma_load_2d_pair_hint(sa, &maps.h, &full_bar[stage], hk * BK, row_ah, pol_last);
+              tma_load_2d_pair_hint(sb, wmap, &full_bar[stage], kb * BK, row_b, pol_last);
               if (++stage == kStages) { stage = 0; phase ^= 1; }
             }
           }
@@ -369,9 +339,9 @@ ensemble_chain_kernel(const __grid_constant__ ChainMaps maps, const __grid_const
               const uint64_t db = ptx::umma_desc_k_sw128(sa + kABytes);
 #pragma unroll
               for (int k = 0; k < kMmasPerBlock; ++k)
-                ptx::umma_ss<E::kKind, CG>(d_tmem, da + 2 * k, db + 2 * k, idesc, (kb | k) != 0);
-              ptx::umma_commit<CG>(&empty_bar[stage]);
-              if (kb == kb_total - 1) ptx::umma_commit<CG>(&tmem_full_bar[acc]);
+                ptx::umma_ss<E::kKind>(d_tmem, da + 2 * k, db + 2 * k, idesc, (kb | k) != 0);
+              ptx::umma_commit(&empty_bar[stage]);
+              if (kb == kb_total - 1) ptx::umma_commit(&tmem_full_bar[acc]);
               if (++stage == kStages) { stage = 0; phase ^= 1; }
             }
           }
@@ -379,7 +349,7 @@ ensemble_chain_kernel(const __grid_constant__ ChainMaps maps, const __grid_const
       }
     }
     __syncwarp();
-  } else if (warp < 2 + kNumEpiWarps) {
+  } else {
     // ===== epilogue warps =====
     const int q = warp & 3;
     const int row_in_tile = q * 32 + lane;
@@ -394,7 +364,7 @@ ensemble_chain_kernel(const __grid_constant__ ChainMaps maps, const __grid_const
       const bool shared = item.role >= 0;
       const int g = item.unit % args.groups;
       const int m_row = ((item.unit / args.groups) * CG + int(cta_rank)) * kBlockM;
-      const int row_h = (args.h_slot && !shared) ? slot_row : g * args.a_rows_per_group + m_row;
+      const int row_h = shared ? g * args.a_rows_per_group + m_row : slot_row;
       unsigned int* my_cnt = nullptr;   // shared unit: this CTA's tile counter, read by the partner pair
       uint32_t my_tiles = 0;
       if (shared)
@@ -489,19 +459,11 @@ ensemble_chain_kernel(const __grid_constant__ ChainMaps maps, const __grid_const
               ptx::named_bar_sync(2, kNumEpiThreads);
               if (epi_tid == 0) {
                 const int col = (kFinal ? 0 : ly.out_col0) + n0 + (c / kChunksPerStore) * kTileCols;
-                if constexpr (kFinal) {
-                  if (args.l2_hints & 8)
-                    tma_store_2d_hint(&maps.out_final, smem_out + size_t(buf) * kOutStageBytes, col,
-                                      g * args.out_rows_per_group + m_row, l2_policy_evict_first());
-                  else
-                    ptx::tma_store_2d(&maps.out_final, smem_out + size_t(buf) * kOutStageBytes, col,
-                                      g * args.out_rows_per_group + m_row);
-                } else {
-                  if (args.l2_hints & 2)
-                    tma_store_2d_hint(&maps.h, smem_out + size_t(buf) * kOutStageBytes, col, row_h, l2_policy_evict_last());
-                  else
-                    ptx::tma_store_2d(&maps.h, smem_out + size_t(buf) * kOutStageBytes, col, row_h);
-                }
+                if constexpr (kFinal)
+                  ptx::tma_store_2d(&maps.out_final, smem_out + size_t(buf) * kOutStageBytes, col,
+                                    g * args.out_rows_per_group + m_row);
+                else
+                  tma_store_2d_hint(&maps.h, smem_out + size_t(buf) * kOutStageBytes, col, row_h, l2_policy_evict_last());
                 ptx::tma_store_commit();
                 if (pending) {
                   // the previous hidden tile (same layer: nothing this CTA runs next reads it yet) - every group but
@@ -527,23 +489,13 @@ ensemble_chain_kernel(const __grid_constant__ ChainMaps maps, const __grid_const
               } else {
                 ptx::tcgen05_fence_before();
                 __syncwarp();
-                if (lane == 0) ptx::mbar_arrive_cluster<CG>(&tmem_empty_bar[acc], 0);
+                if (lane == 0) ptx::mbar_arrive_cluster(&tmem_empty_bar[acc], 0);
               }
               process(final_tag, rb, c + 1);
             }
           };
           if (is_final) {
             run_tile(std::true_type{}, (half ? kHalfN : kBlockN) / 32);
-            if constexpr (TAIL_NM > 0) {
-              // the last member of an env tile that ran here in sequence: its rows go to the tail warps once the deltas
-              // of all its members have landed (earlier members' stores are older groups of the same thread)
-              if (args.tail.enabled && epi_tid == 0 && i < args.tail.rounds * args.groups && n_tile + 1 == ly.n_tiles &&
-                  i % args.groups == args.groups - 1) {
-                ptx::tma_store_wait<0>();
-                chain_fence_proxy_async_global();
-                st_release_cta_smem(tail_ready, uint32_t(i / args.groups) + 1u);
-              }
-            }
           } else {
             run_tile(std::false_type{}, kBlockN / 32);
             if (epi_tid == 0) {
@@ -564,36 +516,13 @@ ensemble_chain_kernel(const __grid_constant__ ChainMaps maps, const __grid_const
       }
     }
     if (epi_tid == 0) ptx::tma_store_wait<0>();
-  } else {
-    // ===== tail warps (launched only with TAIL_NM > 0) =====
-    if constexpr (TAIL_NM > 0) {
-      const ChainTail& t = args.tail;
-      if (t.enabled) {
-        const int tw = warp - (2 + kNumEpiWarps);
-        float* srow = tail_rows + tw * (kPostMaxElems + 4);
-        for (int su = 0; su < t.rounds; ++su) {
-          unsigned int spins = 0;
-          while (ld_acquire_cta_smem(tail_ready) < uint32_t(su) + 1u) {
-            __nanosleep(256);
-            if (++spins > (1u << 27)) __trap();
-          }
-          const long long row0 = (static_cast<long long>(pair + su * pairs) * CG + int(cta_rank)) * kBlockM;
-          for (int r = tw; r < kBlockM; r += kChainTailWarps) {
-            const long long row = row0 + r;
-            if (row < t.n_rows)
-              post_row_warp<TAIL_NM, 2, true>(t.delta, t.delta_rows, t.DP, t.state, t.member, t.num_steps, t.S, row,
-                                              t.next_state, t.disc, t.done, t.tc, t.rff, srow, lane);
-          }
-        }
-      }
-    }
   }
 
   ptx::tcgen05_fence_before();
   ptx::cluster_sync();
   if (warp == 1) {
     ptx::tcgen05_fence_after();
-    ptx::tmem_dealloc<CG>(tmem_base, kTmemCols);
+    ptx::tmem_dealloc(tmem_base, kTmemCols);
   }
 }
 

@@ -1,12 +1,12 @@
 // Grouped, persistent, warp-specialised tcgen05 GEMM for the ensemble MLP layers
 // and the random-feature projection:   D[g] = A[g] * B[g]^T  (both K-major).
 //
-//   * CTA pairs (cta_group::2, CG = 2): two SMs of one TPC own a 256 x 256 output tile.  Each CTA stages its
+//   * CTA pairs (cta_group::2): two SMs of one TPC own a 256 x 256 output tile.  Each CTA stages its
 //     own 128 rows of A and HALF of B (128 of the 256 output features) per k-block, so a pair moves 2 x 32 KB
 //     per k-block from L2 where two independent 128 x 256 tiles would move 2 x 48 KB; the leader CTA's single
 //     elected thread issues tcgen05.mma.cta_group::2 (M 256, N 256, K 16) reading both CTAs' shared memory,
-//     each CTA's TMEM receives its 128 accumulator rows.  CG = 1 is the single-CTA variant (M 128).
-//   * A / B tiles arrive by TMA with the 128-byte swizzle through an mbarrier ring; with CG = 2 both CTAs'
+//     each CTA's TMEM receives its 128 accumulator rows.
+//   * A / B tiles arrive by TMA with the 128-byte swizzle through an mbarrier ring; both CTAs'
 //     loads complete on the LEADER's full barrier, and the leader's tcgen05.commit multicasts the "stage free"
 //     and "accumulator ready" arrivals to both CTAs.
 //   * Two 256-column TMEM accumulators are double-buffered so the epilogue of tile i overlaps the MMAs of tile
@@ -25,22 +25,11 @@
 
 namespace simstep {
 
-// depth of the operand ring of the cta_group::2 kernel: 5 x 32 KB + 2 x 16 KB of store staging = 193 KB; 6 fits
-// (225 KB of the 227 KB a CTA may use) and was measured, see DESIGN.md section 7
-#ifndef SIMSTEP_GEMM_STAGES_CG2
-#define SIMSTEP_GEMM_STAGES_CG2 5
-#endif
-// B-resident small-K mode: when a tile's whole K fits the ring (kb_total <= kStages) the ring is shortened to kb_total
-// stages, so stage s always holds k-block s and the weight half of a stage stays valid for as long as consecutive tiles
-// of this CTA pair share their (group, n-tile) - which the tile order gives (tile_step and n_tiles are both even, the
-// group changes every m_tiles * n_tiles tiles); only the activation half is then reloaded per tile
-#ifndef SIMSTEP_GEMM_B_RESIDENT
-#define SIMSTEP_GEMM_B_RESIDENT 0
-#endif
+// depth of the operand ring: 5 x 32 KB + 2 x 16 KB of store staging = 193 KB; 6 fits (225 KB of the 227 KB a CTA
+// may use) and was measured, see DESIGN.md section 7
+constexpr int kGemmStages = 5;
 // staging tiles of the TMA-store epilogue (16 KB each); kOutStages - 1 stores may still be reading shared memory
-#ifndef SIMSTEP_GEMM_OUT_STAGES
-#define SIMSTEP_GEMM_OUT_STAGES 2
-#endif
+constexpr int kGemmOutStages = 2;
 constexpr int kBlockM = 128;   // accumulator rows per CTA
 constexpr int kBlockN = 256;   // accumulator columns (output features per tile)
 constexpr int kNumEpiWarps = 4;      // per epilogue group
@@ -55,12 +44,11 @@ constexpr int kOutStageBytes = kBlockM * 128;      // staging tile of the TMA-st
 constexpr int kEpiConstFloats = 3 * kBlockN;
 constexpr int kEpiConstBytes = 2 * kEpiConstFloats * 4;
 
-template <int CG>
+// One ring stage of a CTA: its 128 rows of A and half of the pair's 256 rows of B.
 struct GemmShape {
-  static constexpr int kBRows = kBlockN / CG;          // B rows staged per CTA
+  static constexpr int kBRows = kBlockN / 2;           // B rows staged per CTA
   static constexpr int kBBytes = kBRows * 128;
   static constexpr int kStageBytes = kABytes + kBBytes;
-  static constexpr int kStages = CG == 2 ? SIMSTEP_GEMM_STAGES_CG2 : 4;
 };
 
 // Shared-memory plan of one kernel variant.  EG = epilogue warp GROUPS (4 warps each: one per TMEM lane quarter).
@@ -68,13 +56,13 @@ struct GemmShape {
 // short-K tiles - the first layer, the cost features - are bound by the epilogue, not by the MMAs: with EG = 2 a
 // second group takes the upper half of the tile's columns.  Store-tile variants with EG = 2 give every group its own
 // pair of staging tiles and pay for them with one ring stage (they are only used where the whole K fits the ring).
-template <int CG, int EG, bool STORE>
+template <int EG, bool STORE>
 struct GemmPlan {
-  static constexpr int kStages = (CG == 2 && EG == 2 && STORE) ? 4 : GemmShape<CG>::kStages;
-  static constexpr int kOutStages = STORE ? SIMSTEP_GEMM_OUT_STAGES * EG : 0;
+  static constexpr int kStages = (EG == 2 && STORE) ? 4 : kGemmStages;
+  static constexpr int kOutStages = STORE ? kGemmOutStages * EG : 0;
   static constexpr int kThreads = 64 + 128 * EG;  // warp 0 TMA, warp 1 MMA, then the epilogue groups
   static constexpr size_t smem_bytes() {
-    return 1024 /*align slack*/ + size_t(kStages) * GemmShape<CG>::kStageBytes + size_t(kOutStages) * kOutStageBytes +
+    return 1024 /*align slack*/ + size_t(kStages) * GemmShape::kStageBytes + size_t(kOutStages) * kOutStageBytes +
            kEpiConstBytes + kBlockM * sizeof(float) /*dot hand-over*/ + 256;
   }
 };
@@ -150,8 +138,8 @@ enum EpiMode : int { kEpiHidden = 0, kEpiFinal = 1, kEpiRff = 2, kEpiHiddenTanh 
 __host__ __device__ constexpr bool epi_is_rff(int mode) { return mode == kEpiRff || mode == kEpiFeat; }
 
 // Bonus combine of MILO's cost (reference milo/milo/linear_cost.py:96-103, 130-147; GAILCost variants
-// gail_cost.py:232-246), applied to one row's feature dot product.  Used by the random-feature GEMM's epilogue
-// (fused: the dot never leaves registers) and by cost_combine_kernel (explicit partial dots).
+// gail_cost.py:232-246), applied to one row's feature dot product by the random-feature GEMM's epilogue (the dot
+// never leaves registers).
 struct CombineArgs {
   int enabled;            // epilogue: finish the row here (needs n_inner == n_tiles)
   const float* disc;      // nullptr: only dot_out is written
@@ -227,12 +215,12 @@ __device__ __forceinline__ void tma_store_2d_hint(const CUtensorMap* map, const 
 }
 
 struct GemmArgs {
-  // tile space: tile -> (group, m_tile, n_tile), n fastest; an m_tile is CG * 128 rows
+  // tile space: tile -> (group, m_tile, n_tile), n fastest; an m_tile is the 256 rows of a CTA pair
   int n_inner;            // consecutive n-tiles of one (group, m_tile) a CTA pair runs back to back (0 / 1: none)
   int group_fastest;      // tile -> (m_tile, group, n_tile): the members of an env tile run side by side on
                           // neighbouring CTA pairs, so the shared x tile is read from HBM once instead of per member
   int reverse;            // walk the tile space backwards: the rows the previous layer wrote LAST (still in L2) first
-  int b_evict_last;       // load the weight tiles with the evict_last L2 priority (cta_group::2 kernels)
+  int b_evict_last;       // load the weight tiles with the evict_last L2 priority
   int m_tiles;
   int n_tiles;
   int groups;
@@ -251,22 +239,20 @@ struct GemmArgs {
   int out_col0;           // first column (elements) of this layer's output in tmap_out
   void* out;              // kEpiRff: phi float or nullptr
   long long out_pitch;    // kEpiRff: elements
-  int rows_valid;         // kEpiRff: rows that exist in `out` / rff_part
+  int rows_valid;         // kEpiRff: rows that exist in `out` and in the combine's outputs
   int cols_valid;
-  float* rff_part;        // kEpiRff: [n_tiles][rff_part_stride] partial dots
-  long long rff_part_stride;
   float rff_phi_scale;    // sqrt(2/D)
   int rff_tanh;           // kEpiRff: phi = cos(tanh(pre-activation)) (MLPCost, linear_cost.py:208-221)
   int rff_linear;         // kEpiRff: phi = pre-activation (discriminator output, gail_cost.py:18-43)
   CombineArgs comb;       // kEpiRff: finish cost / ipm / bonus in the epilogue
 };
 
-template <typename E, int CG>
+template <typename E>
 __host__ __device__ constexpr uint32_t make_idesc() {
   return (1u << 4)                                        // D format: F32
          | (E::kFmt << 7) | (E::kFmt << 10)               // A / B format
          | (static_cast<uint32_t>(kBlockN >> 3) << 17)    // N
-         | (static_cast<uint32_t>((kBlockM * CG) >> 4) << 24);  // M (256 for a CTA pair)
+         | (static_cast<uint32_t>((kBlockM * 2) >> 4) << 24);  // M: 256 for a CTA pair
 }
 
 // cos(x) for the random-feature epilogue: two-constant Cody-Waite reduction to [-pi, pi] then the SFU
@@ -287,17 +273,18 @@ __device__ __forceinline__ float fast_tanh(float x) {
   return 1.f - __fdividef(2.f, t + 1.f);
 }
 
-template <typename E, int MODE, int CG, int EG = 1>
+template <typename E, int MODE, int EG = 1>
 __global__ void __launch_bounds__(64 + 128 * EG, 1)
 gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_ax, const __grid_constant__ CUtensorMap tmap_ah,
                     const __grid_constant__ CUtensorMap tmap_b, const __grid_constant__ CUtensorMap tmap_out,
                     const GemmArgs args) {
-  using S = GemmShape<CG>;
+  constexpr int CG = 2;  // CTAs per tile
+  using S = GemmShape;
   constexpr int BK = ElemDims<E>::kBlockK;
   constexpr int UK = ElemDims<E>::kUmmaK;
   constexpr int kMmasPerBlock = BK / UK;  // 4
   constexpr bool kStoreTile = !epi_is_rff(MODE);
-  using Plan = GemmPlan<CG, EG, kStoreTile>;
+  using Plan = GemmPlan<EG, kStoreTile>;
   constexpr int kStages = Plan::kStages;
   constexpr int kOutStages = Plan::kOutStages;
   constexpr int kEpiWarps = 4 * EG;
@@ -319,7 +306,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_ax, const __grid_co
 
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
   const int lane = threadIdx.x & 31;
-  const uint32_t cta_rank = CG == 2 ? ptx::cluster_ctarank() : 0u;
+  const uint32_t cta_rank = ptx::cluster_ctarank();
   const bool leader = cta_rank == 0;
 
   if (threadIdx.x == 0) {
@@ -338,11 +325,11 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_ax, const __grid_co
     if (kStoreTile) ptx::prefetch_tensormap(&tmap_out);
   }
   if (warp == 1) {
-    ptx::tmem_alloc<CG>(tmem_base_smem, kTmemCols);
-    ptx::tmem_relinquish<CG>();
+    ptx::tmem_alloc(tmem_base_smem, kTmemCols);
+    ptx::tmem_relinquish();
   }
   ptx::tcgen05_fence_before();
-  if (CG == 2) ptx::cluster_sync(); else __syncthreads();
+  ptx::cluster_sync();
   ptx::tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_base_smem;
   // everything above overlapped the previous kernel's tail; its outputs are read (and ours written) from here on
@@ -368,8 +355,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_ax, const __grid_co
     if (args.group_fastest) { g = t2 % args.groups; m_tile = t2 / args.groups; }
     else { m_tile = t2 % args.m_tiles; g = t2 / args.m_tiles; }
   };
-  const bool b_resident = SIMSTEP_GEMM_B_RESIDENT != 0 && kb_total <= kStages;
-  const int ring = b_resident ? kb_total : kStages;
 
   if (warp == 0) {
     // ===== TMA producer (both CTAs of a pair; the leader arms the barrier for both) =====
@@ -380,7 +365,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_ax, const __grid_co
     const uint64_t pol_last = l2_policy_evict_last();
     int stage = 0;
     uint32_t phase = 0;
-    int held_b = -1;  // (group, n-tile) whose weight k-blocks sit in the stages' B halves (B-resident mode)
     for (int it = 0, tile; (tile = tile_of(it)) >= 0; ++it) {
       int g, m_tile, n_tile;
       decode(tile, g, m_tile, n_tile);
@@ -388,24 +372,19 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_ax, const __grid_co
       const int row_ax = g * args.ax_rows_per_group + m_row;
       const int row_ah = g * args.a_rows_per_group + m_row;
       const int row_b = g * args.b_rows_per_group + n_tile * kBlockN + int(cta_rank) * S::kBRows;
-      const int this_b = g * args.n_tiles + n_tile;
-      const bool load_b = !b_resident || this_b != held_b;
-      held_b = this_b;
       for (int kb = 0; kb < kb_total; ++kb) {
         ptx::mbar_wait(&empty_bar[stage], phase ^ 1);
         uint8_t* sa = smem_tiles + size_t(stage) * S::kStageBytes;
         uint8_t* sb = sa + kABytes;
-        if (leader) ptx::mbar_arrive_expect_tx(&full_bar[stage], (load_b ? S::kStageBytes : kABytes) * CG);
+        if (leader) ptx::mbar_arrive_expect_tx(&full_bar[stage], S::kStageBytes * CG);
         if (kb < args.kb_x) {
-          ptx::tma_load_2d<CG>(sa, &tmap_ax, &full_bar[stage], kb * BK, row_ax);
+          ptx::tma_load_2d(sa, &tmap_ax, &full_bar[stage], kb * BK, row_ax);
         } else {
-          ptx::tma_load_2d<CG>(sa, &tmap_ah, &full_bar[stage], (args.kb_h0 + kb - args.kb_x) * BK, row_ah);
+          ptx::tma_load_2d(sa, &tmap_ah, &full_bar[stage], (args.kb_h0 + kb - args.kb_x) * BK, row_ah);
         }
-        if (load_b) {
-          if (CG == 2 && args.b_evict_last) tma_load_2d_pair_hint(sb, &tmap_b, &full_bar[stage], kb * BK, row_b, pol_last);
-          else ptx::tma_load_2d<CG>(sb, &tmap_b, &full_bar[stage], kb * BK, row_b);
-        }
-        if (++stage == ring) { stage = 0; phase ^= 1; }
+        if (args.b_evict_last) tma_load_2d_pair_hint(sb, &tmap_b, &full_bar[stage], kb * BK, row_b, pol_last);
+        else ptx::tma_load_2d(sb, &tmap_b, &full_bar[stage], kb * BK, row_b);
+        if (++stage == kStages) { stage = 0; phase ^= 1; }
       }
     }
     }
@@ -413,7 +392,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_ax, const __grid_co
   } else if (warp == 1) {
     // ===== MMA issuer (leader CTA only) =====
     if (leader && ptx::elect_one()) {
-      constexpr uint32_t idesc = make_idesc<E, CG>();
+      constexpr uint32_t idesc = make_idesc<E>();
       int stage = 0;
       uint32_t phase = 0;
       for (int it = 0; tile_of(it) >= 0; ++it) {
@@ -431,11 +410,11 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_ax, const __grid_co
 #pragma unroll
           for (int k = 0; k < kMmasPerBlock; ++k) {
             // advance 32 bytes (= UMMA_K elements) along K inside the swizzle atom
-            ptx::umma_ss<E::kKind, CG>(d_tmem, da + 2 * k, db + 2 * k, idesc, (kb | k) != 0);
+            ptx::umma_ss<E::kKind>(d_tmem, da + 2 * k, db + 2 * k, idesc, (kb | k) != 0);
           }
-          ptx::umma_commit<CG>(&empty_bar[stage]);
-          if (kb == kb_total - 1) ptx::umma_commit<CG>(&tmem_full_bar[acc]);
-          if (++stage == ring) { stage = 0; phase ^= 1; }
+          ptx::umma_commit(&empty_bar[stage]);
+          if (kb == kb_total - 1) ptx::umma_commit(&tmem_full_bar[acc]);
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
         }
       }
     }
@@ -534,7 +513,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_ax, const __grid_co
           }
           // staging tile: row r holds 128 bytes, 16-byte unit j sits at unit j ^ (r & 7) (TMA SWIZZLE_128B)
           const int sub = c % kChunksPerStore;            // position of this chunk inside the staging row
-          constexpr int kGroupStages = SIMSTEP_GEMM_OUT_STAGES;  // staging tiles owned by one group
+          constexpr int kGroupStages = kGemmOutStages;  // staging tiles owned by one group
           const int buf = grp * kGroupStages + store_it % kGroupStages;
           if (sub == 0) {
             // the TMA store that last read this staging buffer must have finished reading shared memory
@@ -608,7 +587,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_ax, const __grid_co
           // accumulator drained: the MMA warp (leader CTA) may overwrite it
           ptx::tcgen05_fence_before();
           __syncwarp();
-          if (lane == 0) ptx::mbar_arrive_cluster<CG>(&tmem_empty_bar[acc], 0);
+          if (lane == 0) ptx::mbar_arrive_cluster(&tmem_empty_bar[acc], 0);
         }
         process(rb, c + 1);
       }
@@ -625,23 +604,17 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_ax, const __grid_co
             // only after this read
           }
         }
-        if (grp == 0 && finish) {
-          if (args.comb.enabled) {
-            if (row < args.rows_valid) combine_row(args.comb, row, total);
-          } else if (args.rff_part != nullptr && row < args.rows_valid) {
-            args.rff_part[size_t(n_tile) * args.rff_part_stride + row] = total;
-          }
-        }
+        if (grp == 0 && finish && args.comb.enabled && row < args.rows_valid) combine_row(args.comb, row, total);
       }
     }
     if (kStoreTile && gtid == 0) ptx::tma_store_wait<0>();  // shared memory must outlive the last store's read
   }
 
   ptx::tcgen05_fence_before();
-  if (CG == 2) ptx::cluster_sync(); else __syncthreads();  // nobody leaves while its peer can still signal it
+  ptx::cluster_sync();  // nobody leaves while its peer can still signal it
   if (warp == 1) {
     ptx::tcgen05_fence_after();
-    ptx::tmem_dealloc<CG>(tmem_base, kTmemCols);
+    ptx::tmem_dealloc(tmem_base, kTmemCols);
   }
 }
 

@@ -14,8 +14,6 @@
 // which is what a bulk copy needs.  The delta workspace has a 912-byte row pitch (S rounded up to 4 floats) for
 // the same reason.  An odd trailing row is staged with plain loads.
 #pragma once
-#include <algorithm>
-#include <cstdlib>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include "elementwise.cuh"
@@ -24,7 +22,7 @@
 namespace simstep {
 
 // 10 rings of two warps, 2 stages each: measured (B200, 40 000 rows, 4 members) 48.0 us against 49.3 us for 8 x 2,
-// 55.0 us for 8 x 3 and 60.1 us for 6 x 4 - more warps beat deeper rings (SIMSTEP_POST_RINGS / _STAGES override)
+// 55.0 us for 8 x 3 and 60.1 us for 6 x 4 - more warps beat deeper rings
 constexpr int kPostTmaMaxWarps = 20;
 constexpr int kPostTmaLaunchWarps = 20;  // launch bound
 constexpr int kPostTmaMaxStages = 2;
@@ -44,8 +42,6 @@ inline PostTmaPlan post_tma_plan(int S, int DP, int NM) {
   p.stage_bytes = 2 * S * 4 + NM * 2 * DP * 4;
   p.rings = kPostTmaMaxWarps / 2;
   p.stages = kPostTmaMaxStages;
-  if (const char* e = std::getenv("SIMSTEP_POST_RINGS")) p.rings = std::max(1, std::min(std::atoi(e), kPostTmaLaunchWarps / 2));
-  if (const char* e = std::getenv("SIMSTEP_POST_STAGES")) p.stages = std::max(2, std::min(std::atoi(e), 4));
   while (p.rings * p.stages * p.stage_bytes > kPostTmaSmemBudget) {
     if (p.stages > 2) --p.stages;
     else if (p.rings > 1) --p.rings;

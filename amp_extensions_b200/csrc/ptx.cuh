@@ -90,37 +90,17 @@ __device__ __forceinline__ void prefetch_tensormap(const CUtensorMap* m) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(m)) : "memory");
 }
 
-// 2-D tiled load global -> shared, completion signalled on an mbarrier.  CG = 2: the load belongs to a CTA
-// pair and its bytes complete on the LEADER CTA's barrier (bit 24 of a shared::cluster address selects the
-// CTA of the pair; clearing it addresses the even CTA's copy of the barrier).
-template <int CG = 1>
+// 2-D tiled load global -> shared of a CTA pair, completion signalled on an mbarrier: the bytes complete on the
+// LEADER CTA's barrier (bit 24 of a shared::cluster address selects the CTA of the pair; clearing it addresses the
+// even CTA's copy of the barrier).
 __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int32_t c0,
                                             int32_t c1) {
-  if constexpr (CG == 1) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-        :
-        : "r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-        : "memory");
-  } else {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes"
-        " [%0], [%1, {%3, %4}], [%2];"
-        :
-        : "r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar) & 0xFEFFFFFFu), "r"(c0),
-          "r"(c1)
-        : "memory");
-  }
-}
-
-__device__ __forceinline__ void tma_load_2d_hint(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int32_t c0,
-                                                 int32_t c1, uint64_t policy) {
   asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint"
-      " [%0], [%1, {%3, %4}], [%2], %5;"
+      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes"
+      " [%0], [%1, {%3, %4}], [%2];"
       :
-      : "r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1),
-        "l"(policy)
+      : "r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar) & 0xFEFFFFFFu), "r"(c0),
+        "r"(c1)
       : "memory");
 }
 
@@ -157,32 +137,17 @@ __device__ __forceinline__ void tma_store_wait() {
 
 // ---- TMEM -----------------------------------------------------------------
 
-// Executed by one full warp (of EACH CTA of the pair when CG = 2).  Writes the TMEM base address to
-// *smem_result.
-template <int CG = 1>
+// Executed by one full warp of EACH CTA of the pair.  Writes the TMEM base address to *smem_result.
 __device__ __forceinline__ void tmem_alloc(uint32_t* smem_result, uint32_t cols) {
-  if constexpr (CG == 1)
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_result)),
-                 "r"(cols)
-                 : "memory");
-  else
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_result)),
-                 "r"(cols)
-                 : "memory");
+  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_result)),
+               "r"(cols)
+               : "memory");
 }
-template <int CG = 1>
 __device__ __forceinline__ void tmem_relinquish() {
-  if constexpr (CG == 1)
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  else
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
 }
-template <int CG = 1>
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
-  if constexpr (CG == 1)
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-  else
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
+  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
 }
 
 __device__ __forceinline__ void tcgen05_fence_before() {
@@ -222,43 +187,35 @@ __device__ __forceinline__ uint64_t umma_desc_k_sw128(uint32_t smem_addr) {
   return d;
 }
 
-// kind: 0 tf32, 1 f16 (fp16 / bf16 operands).  d_tmem (+)= A * B^T.  CG = 2: issued by the leader CTA of a
-// pair; A rows and B rows (output features) of both CTAs' shared memory form one M 256 x N 256 product.
-#define SIMSTEP_UMMA(GROUP, KINDSTR)                                                               \
+// kind: 0 tf32, 1 f16 (fp16 / bf16 operands).  d_tmem (+)= A * B^T, issued by the leader CTA of a pair; A rows
+// and B rows (output features) of both CTAs' shared memory form one M 256 x N 256 product.
+#define SIMSTEP_UMMA(KINDSTR)                                                                      \
   asm volatile(                                                                                    \
       "{\n\t"                                                                                      \
       ".reg .pred p;\n\t"                                                                          \
       "setp.ne.b32 p, %4, 0;\n\t"                                                                  \
-      "tcgen05.mma.cta_group::" GROUP ".kind::" KINDSTR " [%0], %1, %2, %3, p;\n\t"                \
+      "tcgen05.mma.cta_group::2.kind::" KINDSTR " [%0], %1, %2, %3, p;\n\t"                       \
       "}\n"                                                                                        \
       :                                                                                            \
       : "r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)                         \
       : "memory")
-template <int KIND, int CG = 1>
+template <int KIND>
 __device__ __forceinline__ void umma_ss(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
                                         uint32_t accumulate) {
-  if constexpr (KIND == 0 && CG == 1) SIMSTEP_UMMA("1", "tf32");
-  else if constexpr (KIND == 0) SIMSTEP_UMMA("2", "tf32");
-  else if constexpr (CG == 1) SIMSTEP_UMMA("1", "f16");
-  else SIMSTEP_UMMA("2", "f16");
+  if constexpr (KIND == 0) SIMSTEP_UMMA("tf32");
+  else SIMSTEP_UMMA("f16");
 }
 #undef SIMSTEP_UMMA
 
-// Arrives on the mbarrier once every previously issued UMMA has completed.  CG = 2: the arrival is
-// multicast to the barrier at the same offset in both CTAs of the pair.
-template <int CG = 1>
+// Arrives on the mbarrier once every previously issued UMMA has completed.  The arrival is multicast to the
+// barrier at the same offset in both CTAs of the pair.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  if constexpr (CG == 1) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-                 : "memory");
-  } else {
-    const uint16_t mask = 3;
-    asm volatile(
-        "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-            smem_u32(bar)),
-        "h"(mask)
-        : "memory");
-  }
+  const uint16_t mask = 3;
+  asm volatile(
+      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
+          smem_u32(bar)),
+      "h"(mask)
+      : "memory");
 }
 
 // ---- clusters ---------------------------------------------------------------
@@ -273,19 +230,14 @@ __device__ __forceinline__ void cluster_sync() {
   asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
   asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
-// mbarrier arrive on the barrier at the same offset in CTA `cta_rank` of the cluster (CG = 1: local arrive).
-template <int CG = 1>
+// mbarrier arrive on the barrier at the same offset in CTA `cta_rank` of the cluster.
 __device__ __forceinline__ void mbar_arrive_cluster(uint64_t* bar, uint32_t cta_rank) {
-  if constexpr (CG == 1) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-  } else {
-    // default semantics (release at cta scope), as CUTLASS's ClusterBarrier::arrive(cta_id): what this arrival hands
-    // over is TMEM that the tcgen05 fences already ordered; `.release.cluster` made ptxas emit a gpu-wide MEMBAR +
-    // ERRBAR in front of every arrival, the top stall of the short-K epilogues (ncu r02: 27 % of layer 1's samples)
-    uint32_t remote;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(smem_u32(bar)), "r"(cta_rank));
-    asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(remote) : "memory");
-  }
+  // default semantics (release at cta scope), as CUTLASS's ClusterBarrier::arrive(cta_id): what this arrival hands
+  // over is TMEM that the tcgen05 fences already ordered; `.release.cluster` made ptxas emit a gpu-wide MEMBAR +
+  // ERRBAR in front of every arrival, the top stall of the short-K epilogues (ncu r02: 27 % of layer 1's samples)
+  uint32_t remote;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(smem_u32(bar)), "r"(cta_rank));
+  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(remote) : "memory");
 }
 
 __device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t n_threads) {

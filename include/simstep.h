@@ -132,7 +132,7 @@ int simstep_forward_launches(const simstep_handle* h, int64_t n_envs, int32_t* l
 
 /* Out-of-bounds check of the handle's workspaces (compute-sanitizer is not available where the GPU tests run): with
  * SIMSTEP_DEBUG_GUARDS=1 in the environment at simstep_create every workspace buffer (normalised inputs, activations,
- * member deltas, cost operand rows, partial dots) is allocated between two 64 KB guard zones filled with 0xA5.
+ * member deltas, cost operand rows) is allocated between two 64 KB guard zones filled with 0xA5.
  * buffers_out = guarded buffers currently allocated (0 when the switch is off), bad_bytes_out = guard bytes that
  * have been overwritten.  Synchronises with the device.  No reference counterpart. */
 int simstep_debug_check_guards(simstep_handle* h, int64_t* buffers_out, int64_t* bad_bytes_out);

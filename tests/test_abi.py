@@ -108,6 +108,22 @@ def test_product_package_never_imports_the_oracle():
                 assert not re.search(r"^\s*(from|import)\s+oracle\b", src, re.M), f"{f} imports the oracle"
 
 
+def test_native_code_reads_only_the_documented_environment_switches():
+    """The library reads three environment variables (README.md, "Diagnostic switches"): SIMSTEP_CHAIN=0 forces one
+    launch per layer, SIMSTEP_IMIT_GENERIC=1 the generic imitation kernel, SIMSTEP_DEBUG_GUARDS=1 the workspace guard
+    zones.  A selection between kernels is made from the inputs, not left to a variable set by the user."""
+    csrc = os.path.join(ROOT, "amp_extensions_b200", "csrc")
+    calls, names = 0, []
+    for f in sorted(os.listdir(csrc)):
+        if f.endswith((".cu", ".cuh", ".inc", ".h")):
+            with open(os.path.join(csrc, f)) as fh:
+                src = fh.read()
+            calls += src.count("getenv(")
+            names += re.findall(r'getenv\(\s*"([A-Za-z0-9_]+)"\s*\)', src)
+    assert calls == len(names), "every getenv call names its variable literally"
+    assert set(names) == {"SIMSTEP_CHAIN", "SIMSTEP_IMIT_GENERIC", "SIMSTEP_DEBUG_GUARDS"}, sorted(names)
+
+
 def test_forward_kernel_schedule_covers_every_unit_exactly_once():
     """The column-fused forward kernel's unit schedule (csrc/gemm_chain.cuh: chain_schedule + chain_item, evaluated on
     the HOST through simstep_debug_chain_schedule - no GPU involved): for every batch / ensemble shape each

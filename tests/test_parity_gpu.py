@@ -569,61 +569,32 @@ def test_unaligned_state_rows_take_the_fallback_kernel_with_the_same_results(pre
     assert_close(out_odd[3], out_al[3], out_al[3].abs().max().item(), rel=1e-5, what="cost")
 
 
-def test_fused_final_kernel_matches_the_default_two_launch_path(tmp_path):
-    """SIMSTEP_FINAL_FUSED=1 runs the final ensemble layer and the env step's tail as ONE launch (csrc/gemm_final.cuh:
-    transposed L2 scratch, tickets, tail warps).  Same fp32 arithmetic per element as the final-layer GEMM followed by
-    post_step_tma_kernel, so next states, step counters and termination masks are bit-identical (including the NaN row
-    of an out-of-range member index); the discrepancy sums its squares in a different order (1e-6)."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    files = {}
-    for flag in ("0", "1"):
-        out = str(tmp_path / f"fused{flag}.npz")
-        env = dict(os.environ, SIMSTEP_FINAL_FUSED=flag)
-        res = subprocess.run([sys.executable, os.path.join(root, "tools", "final_fused_check.py"), out], env=env,
-                             capture_output=True, text=True, timeout=600)
-        assert res.returncode == 0, res.stdout[-2000:] + res.stderr[-2000:]
-        files[flag] = np.load(out)
-    a, b = files["0"], files["1"]
-    assert sorted(a.files) == sorted(b.files)
-    for k in a.files:
-        x, y = a[k], b[k]
-        if k.endswith(("_next", "_done", "_steps")):
-            assert np.array_equal(x, y, equal_nan=True), k
-        else:
-            scale = max(float(np.nanmax(np.abs(x))), 1e-12)
-            assert float(np.nanmax(np.abs(x - y))) <= 2e-6 * scale, (k, float(np.nanmax(np.abs(x - y))), scale)
-    assert np.isnan(a["E2000_s1_next"][3]).all() and not np.isnan(a["E2000_s1_next"][4]).any()
-
-
-def test_column_fused_forward_is_bit_identical_to_one_launch_per_layer(tmp_path):
+def test_column_fused_forward_matches_one_launch_per_layer_bit_for_bit(tmp_path):
     """The default forward pass is ONE launch (csrc/gemm_chain.cuh): a CTA pair runs every layer of a (member, 256-row
     env tile), the activations handed on through L2, the last partial round shared between pairs with the final layer
     as M 256 x N 128 halves.  Every output element accumulates its K blocks in the same order as in the per-layer
     launches (SIMSTEP_CHAIN=0), so ALL outputs of the step are bit-identical - for batches of 1 .. 40 001 rows, i.e.
-    with fewer units than CTA pairs, whole rounds only, and shared units in the last round (4 800 and 40 001 rows) - and for
-    an irregular second ensemble (three members, no dense connections, tanh, hidden 512 / 256 / 512: the pairs sharing a
-    unit get unequal work) at 6 812 and 19 193 rows."""
+    with fewer units than CTA pairs, whole rounds only, shared units in the last round (4 800 and 40 001 rows) and a
+    plain, unshared last round (7 000 rows: no whole round in sequence, 38 units left over for 74 pairs; 21 500 rows: one
+    round in sequence, 40 left over) - and for an irregular second ensemble (three members, no dense connections, tanh,
+    hidden 512 / 256 / 512: the pairs sharing a unit get unequal work) at 6 812 and 19 193 rows."""
     import os
     import subprocess
     import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    script = os.path.join(os.path.dirname(os.path.abspath(__file__)), "write_step_outputs.py")
     files = {}
-    for mode in ("0", "1", "2", "3"):
-        out = str(tmp_path / f"chain{mode}.npz")
-        env = dict(os.environ, SIMSTEP_CHAIN=mode)
-        env.pop("SIMSTEP_FINAL_FUSED", None)
-        res = subprocess.run([sys.executable, os.path.join(root, "tools", "final_fused_check.py"), out], env=env,
-                             capture_output=True, text=True, timeout=600)
+    for name in ("per_layer", "default"):
+        out = str(tmp_path / f"{name}.npz")
+        env = {k: v for k, v in os.environ.items() if k != "SIMSTEP_CHAIN"}
+        if name == "per_layer":
+            env["SIMSTEP_CHAIN"] = "0"
+        res = subprocess.run([sys.executable, script, out], env=env, capture_output=True, text=True, timeout=600)
         assert res.returncode == 0, res.stdout[-2000:] + res.stderr[-2000:]
-        files[mode] = np.load(out)
-    ref = files["0"]
-    for mode in ("1", "2", "3"):
-        assert sorted(ref.files) == sorted(files[mode].files)
-        for k in ref.files:
-            assert np.array_equal(ref[k], files[mode][k], equal_nan=True), (mode, k)
+        files[name] = np.load(out)
+    ref, chain = files["per_layer"], files["default"]
+    assert sorted(ref.files) == sorted(chain.files)
+    for k in ref.files:
+        assert np.array_equal(ref[k], chain[k], equal_nan=True), k
 
 
 def test_column_fused_forward_replays_from_a_cuda_graph_with_shared_units():
@@ -705,35 +676,3 @@ for prec, chunk in (("fp16", 0), ("tf32", 0), ("fp16", 4096)):
         res = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=900)
         assert res.returncode == 0, res.stdout[-2000:] + res.stderr[-3000:]
         assert res.stdout.count("GUARDS") == 3
-
-
-def test_step_tail_inside_the_forward_kernel_matches_the_post_step_kernel(tmp_path):
-    """SIMSTEP_CHAIN_TAIL=1 (opt-in, DESIGN.md section 5): the tail of the env step - next state, counters, termination,
-    discrepancy, cost operand rows - runs on four extra warps INSIDE the column-fused forward kernel for the env tiles
-    whose members all ran on one CTA pair (post_row_warp, the one-warp-per-row kernel's body, on deltas read back with
-    ld.global.cg), the post-step kernel only gets the remaining rows.  Same fp32 arithmetic per element: next states,
-    step counters and masks are bit-identical (including the NaN row of an out-of-range member index), the discrepancy
-    sums its squares in another order (2e-6), the cost follows."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    files = {}
-    for flag, keep in (("0", "1"), ("1", "1"), ("1", "0")):
-        out = str(tmp_path / f"tail{flag}{keep}.npz")
-        env = dict(os.environ, SIMSTEP_CHAIN_TAIL=flag, SIMSTEP_CHAIN_TAIL_KEEP=keep)
-        res = subprocess.run([sys.executable, os.path.join(root, "tools", "final_fused_check.py"), out], env=env,
-                             capture_output=True, text=True, timeout=600)
-        assert res.returncode == 0, res.stdout[-2000:] + res.stderr[-2000:]
-        files[flag + keep] = np.load(out)
-    a = files["01"]
-    for key in ("11", "10"):
-        b = files[key]
-        assert sorted(a.files) == sorted(b.files)
-        for k in a.files:
-            x, y = a[k], b[k]
-            if k.endswith(("_next", "_done", "_steps")):
-                assert np.array_equal(x, y, equal_nan=True), (key, k)
-            else:
-                scale = max(float(np.nanmax(np.abs(x))), 1e-12)
-                assert float(np.nanmax(np.abs(x - y))) <= 2e-6 * scale, (key, k)

@@ -1,31 +1,20 @@
 #!/bin/bash
 # column-fused forward (gemm_chain.cuh) against one launch per layer: bitwise comparison of the step's outputs, then a
-# short bench per mode.  Usage: bash tools/gpu_chain.sh [tag] [modes...]
-TAG=${1:-chain}; shift
-MODES=${@:-0 1 2 3}
+# short bench of each (SIMSTEP_CHAIN=0: one launch per layer; 2: the default).  Usage: bash tools/gpu_chain.sh [tag]
+TAG=${1:-chain}
 OUT=gpurun_out; mkdir -p $OUT
-SIMSTEP_CHAIN=0 timeout 300 python tools/final_fused_check.py /tmp/c0.npz || echo "per-layer run failed"
-for m in $MODES; do
-  [ $m = 0 ] && continue
-  SIMSTEP_CHAIN=$m timeout 300 python tools/final_fused_check.py /tmp/c$m.npz 2>&1 | tail -5 || echo "chain mode $m run failed"
+for m in 0 2; do
+  SIMSTEP_CHAIN=$m timeout 300 python tests/write_step_outputs.py /tmp/c$m.npz 2>&1 | tail -5 || echo "mode $m run failed"
 done
-python - $MODES <<'PY'
-import sys
+python - <<'PY'
 import numpy as np
-a = np.load("/tmp/c0.npz")
-for m in sys.argv[1:]:
-    if m == "0":
-        continue
-    try:
-        b = np.load("/tmp/c%s.npz" % m)
-    except Exception as e:
-        print("mode", m, "missing", e); continue
-    bad = [k for k in a.files if not np.array_equal(a[k], b[k], equal_nan=True)]
-    print("mode", m, "bitwise identical" if not bad else "DIFFERS in %s" % bad[:8])
-    for k in bad[:4]:
-        print("  ", k, float(np.nanmax(np.abs(a[k].astype(np.float64) - b[k].astype(np.float64)))))
+a, b = np.load("/tmp/c0.npz"), np.load("/tmp/c2.npz")
+bad = [k for k in a.files if not np.array_equal(a[k], b[k], equal_nan=True)]
+print("bitwise identical" if not bad else "DIFFERS in %s" % bad[:8])
+for k in bad[:4]:
+    print("  ", k, float(np.nanmax(np.abs(a[k].astype(np.float64) - b[k].astype(np.float64)))))
 PY
-for m in $MODES; do
+for m in 0 2; do
 for i in 1 2; do
 SIMSTEP_CHAIN=$m timeout 300 python bench.py --steps 50 --warmup 5 --skip-cpu-baseline --skip-e2e --skip-sustained --skip-extras > $OUT/${TAG}_m${m}_$i.json 2> $OUT/${TAG}_m${m}_$i.err
 python - <<PY

@@ -19,6 +19,7 @@ ABI_VERSION = 1
 PREC = {"tf32": 0, "fp16": 1, "bf16": 2}
 ACT = {"relu": 0, "tanh": 1}
 SHAPE = {"sphere": 0, "capsule": 1, "box": 2}
+RFF_INPUT = {None: 0, "s": 1, "sa": 2, "ss": 3, "sas": 4}  # SIMSTEP_RFF_INPUT_*; None: inferred from in_dim
 
 
 class SimstepConfig(C.Structure):
@@ -82,6 +83,7 @@ _SIGNATURES = {
     "simstep_load_ensemble": (C.c_int, [_c_void_p, C.POINTER(_c_void_p), C.POINTER(_c_void_p), C.POINTER(_c_void_p)]),
     "simstep_set_termination": (C.c_int, [_c_void_p, C.POINTER(SimstepTermination)]),
     "simstep_load_rff": (C.c_int, [_c_void_p, C.c_int32, C.c_int32, _c_void_p, _c_void_p, C.c_int32]),
+    "simstep_load_rff_typed": (C.c_int, [_c_void_p, C.c_int32, C.c_int32, C.c_int32, _c_void_p, _c_void_p, C.c_int32]),
     "simstep_set_rff_split": (C.c_int, [_c_void_p, C.c_int32]),
     "simstep_saturation_count": (C.c_int, [_c_void_p, C.POINTER(C.c_int64), C.c_int32]),
     "simstep_forward_launches": (C.c_int, [_c_void_p, C.c_int64, C.POINTER(C.c_int32)]),

@@ -86,6 +86,7 @@ struct simstep_handle {
   int D = 0, D_pad = 0, rff_in = 0, RK = 0, RKT = 0;
   int rff_split_cap = 0;  // operands were packed as hi/lo pairs: rows hold [hi | lo], weights [hi | hi | lo]
   int rff_split = 0;      // the three-product evaluation is in use (simstep_set_rff_split; needs rff_split_cap)
+  int rff_type = 0;  // SIMSTEP_RFF_INPUT_S / SA / SS / SAS, resolved at load time
   int rff_col2 = 0;  // input_type 'ss': operand column of s' (s sits at 0); the weight columns are packed to match
   void* rff_w = nullptr;
   float* rff_b = nullptr;
@@ -715,15 +716,17 @@ int stage_w(simstep_handle* h, const float* w_dev, cudaStream_t st) {
 // order (linear_cost.py:115-126) except for input_type 'ss', where s' starts at column rff_col2 (see load_rff).
 int rff_sources(simstep_handle* h, const float* s, const float* a, const float* s2, RffSrc* out) {
   RffSrc r{};
-  const int S = h->S, A = h->A, in = h->rff_in;
+  const int S = h->S, A = h->A;
   auto seg = [&](const float* p, int width, int pitch, int dst0) {
     r.ptr[r.n] = p; r.width[r.n] = width; r.pitch[r.n] = pitch; r.dst0[r.n] = dst0; r.n++;
   };
-  if (in == 2 * S && s2) { seg(s, S, S, 0); seg(s2, S, S, h->rff_col2); }
-  else if (in == S) { seg(s, S, S, 0); }
-  else if (in == S + A) { seg(s, S, S, 0); seg(a, A, A, S); }
-  else if (in == 2 * S + A && s2) { seg(s, S, S, 0); seg(a, A, A, S); seg(s2, S, S, S + A); }
-  else return fail(h, SIMSTEP_EINVAL, "rff in_dim does not match an input_type of s/ss/sa/sas");
+  switch (h->rff_type) {
+    case SIMSTEP_RFF_INPUT_S: seg(s, S, S, 0); break;
+    case SIMSTEP_RFF_INPUT_SA: seg(s, S, S, 0); seg(a, A, A, S); break;
+    case SIMSTEP_RFF_INPUT_SS: seg(s, S, S, 0); seg(s2, S, S, h->rff_col2); break;
+    case SIMSTEP_RFF_INPUT_SAS: seg(s, S, S, 0); seg(a, A, A, S); seg(s2, S, S, S + A); break;
+    default: return fail(h, SIMSTEP_EINVAL, "the random-feature layer has no input_type");
+  }
   *out = r;
   return SIMSTEP_OK;
 }
@@ -958,13 +961,16 @@ int simstep_load_ensemble(simstep_handle* h, const float* const* weights_host, c
   if (!h->out_scale_dev) CU_TRY(h, cudaMalloc(&h->out_scale_dev, size_t(h->SP) * sizeof(float)));
   if (!h->out_shift_dev) CU_TRY(h, cudaMalloc(&h->out_shift_dev, size_t(h->SP) * sizeof(float)));
   if (h->cfg.transform) {
-    for (int i = 0; i < 6; ++i)
-      if (!transforms_host[i]) return fail(h, SIMSTEP_EINVAL, "null transform vector");
+    for (int i = 0; i < 6; ++i)  // the action vectors are empty (and may be NULL) when action_dim == 0
+      if (!transforms_host[i] && !(A == 0 && (i == 2 || i == 3)))
+        return fail(h, SIMSTEP_EINVAL, "null transform vector");
     std::vector<float> tf(2 * S + 2 * A), osc(h->SP, 1.f), osh(h->SP, 0.f);
     std::memcpy(tf.data(), transforms_host[0], S * sizeof(float));
     std::memcpy(tf.data() + S, transforms_host[1], S * sizeof(float));
-    std::memcpy(tf.data() + 2 * S, transforms_host[2], A * sizeof(float));
-    std::memcpy(tf.data() + 2 * S + A, transforms_host[3], A * sizeof(float));
+    if (A > 0) {
+      std::memcpy(tf.data() + 2 * S, transforms_host[2], A * sizeof(float));
+      std::memcpy(tf.data() + 2 * S + A, transforms_host[3], A * sizeof(float));
+    }
     std::memcpy(osh.data(), transforms_host[4], S * sizeof(float));
     std::memcpy(osc.data(), transforms_host[5], S * sizeof(float));
     CU_TRY(h, cudaMemcpy(h->tf_dev, tf.data(), tf.size() * sizeof(float), cudaMemcpyHostToDevice));
@@ -1002,7 +1008,30 @@ int simstep_set_termination(simstep_handle* h, const simstep_termination* t) {
 
 int simstep_load_rff(simstep_handle* h, int32_t feature_dim, int32_t in_dim, const float* weight_host,
                      const float* bias_host, int32_t split) {
+  return simstep_load_rff_typed(h, feature_dim, in_dim, SIMSTEP_RFF_INPUT_AUTO, weight_host, bias_host, split);
+}
+
+int simstep_load_rff_typed(simstep_handle* h, int32_t feature_dim, int32_t in_dim, int32_t input_type,
+                           const float* weight_host, const float* bias_host, int32_t split) {
   if (!h || !weight_host || !bias_host || feature_dim < 1 || in_dim < 1) return fail(h, SIMSTEP_EINVAL, "bad argument");
+  // operand width of each input_type, indexed by SIMSTEP_RFF_INPUT_*; the type fixes the operand layout the weights are
+  // packed to, so it has to be known here: an 'sa' layer of an S == A handle has the width of 'ss'
+  const int width[5] = {0, h->S, h->S + h->A, 2 * h->S, 2 * h->S + h->A};
+  if (input_type == SIMSTEP_RFF_INPUT_AUTO) {
+    int matches = 0;
+    for (int t = SIMSTEP_RFF_INPUT_S; t <= SIMSTEP_RFF_INPUT_SAS; ++t)
+      if (width[t] == in_dim) { input_type = t; ++matches; }
+    if (matches == 0) return fail(h, SIMSTEP_EINVAL, "rff in_dim does not match an input_type of s/sa/ss/sas");
+    if (matches > 1)
+      return fail(h, SIMSTEP_EINVAL, "rff in_dim " + std::to_string(in_dim) + " is the width of more than one input_type at " +
+                                         "state_dim " + std::to_string(h->S) + ", action_dim " + std::to_string(h->A) +
+                                         ": load it with simstep_load_rff_typed");
+  } else if (input_type < SIMSTEP_RFF_INPUT_S || input_type > SIMSTEP_RFF_INPUT_SAS) {
+    return fail(h, SIMSTEP_EINVAL, "bad rff input_type");
+  } else if (width[input_type] != in_dim) {
+    return fail(h, SIMSTEP_EINVAL, "rff in_dim " + std::to_string(in_dim) + " is not the width " +
+                                       std::to_string(width[input_type]) + " of its input_type");
+  }
   DeviceScope dev_scope(h->device);  // parameters live on the handle's device; the caller's current device is restored
   CU_TRY(h, cudaDeviceSynchronize());
   cudaFree(h->rff_w); cudaFree(h->rff_b); cudaFree(h->rff_wpad); cudaFree(h->colsum_partial);
@@ -1013,9 +1042,10 @@ int simstep_load_rff(simstep_handle* h, int32_t feature_dim, int32_t in_dim, con
   h->D = feature_dim;
   h->D_pad = int(round_up(feature_dim, kBlockN));
   h->rff_in = in_dim;
-  // input_type 'ss' on an ensemble handle (in_dim == 2 S): s' starts at column S rounded up to 8 instead of S, so the
-  // step's fused tail writes both halves of an operand row with aligned 16-byte stores; weight columns follow
-  h->rff_col2 = (h->S > 0 && in_dim == 2 * h->S && !h->feat_net) ? int(round_up(h->S, 8)) : 0;
+  h->rff_type = input_type;
+  // input_type 'ss': s' starts at column S rounded up to 8 instead of S, so the step's fused tail writes both halves of
+  // an operand row with aligned 16-byte stores; weight columns follow
+  h->rff_col2 = (input_type == SIMSTEP_RFF_INPUT_SS && !h->feat_net) ? int(round_up(h->S, 8)) : 0;
   h->RK = int(round_up(h->rff_col2 > 0 ? h->rff_col2 + h->S : in_dim, 64));
   h->rff_split_cap = split ? 1 : 0;
   h->rff_split = h->rff_split_cap;
@@ -1200,7 +1230,7 @@ int simstep_forward(simstep_handle* h, const float* state_dev, const float* acti
   int rc = check_step_ready(h, n_envs);
   if (rc) return rc;
   if (n_envs == 0) return SIMSTEP_OK;
-  if (!state_dev || !action_dev || !delta_dev) return fail(h, SIMSTEP_EINVAL, "null device pointer");
+  if (!state_dev || (!action_dev && h->A > 0) || !delta_dev) return fail(h, SIMSTEP_EINVAL, "null device pointer");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if ((rc = ensure_workspace(h, n_envs))) return rc;
   for (long long r0 = 0; r0 < n_envs; r0 += h->cap_rows) {
@@ -1220,7 +1250,7 @@ int simstep_discrepancy(simstep_handle* h, const float* state_dev, const float* 
   int rc = check_step_ready(h, n_envs);
   if (rc) return rc;
   if (n_envs == 0) return SIMSTEP_OK;
-  if (!state_dev || !action_dev || !disc_dev) return fail(h, SIMSTEP_EINVAL, "null device pointer");
+  if (!state_dev || (!action_dev && h->A > 0) || !disc_dev) return fail(h, SIMSTEP_EINVAL, "null device pointer");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if ((rc = ensure_workspace(h, n_envs))) return rc;
   for (long long r0 = 0; r0 < n_envs; r0 += h->cap_rows) {
@@ -1237,7 +1267,7 @@ int simstep_step(simstep_handle* h, const float* state_dev, const float* action_
   int rc = check_step_ready(h, n_envs);
   if (rc) return rc;
   if (n_envs == 0) return SIMSTEP_OK;
-  if (!state_dev || !action_dev || !next_state_dev) return fail(h, SIMSTEP_EINVAL, "null device pointer");
+  if (!state_dev || (!action_dev && h->A > 0) || !next_state_dev) return fail(h, SIMSTEP_EINVAL, "null device pointer");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if ((rc = ensure_workspace(h, n_envs))) return rc;
   for (long long r0 = 0; r0 < n_envs; r0 += h->cap_rows) {
@@ -1260,7 +1290,7 @@ int simstep_step_cost(simstep_handle* h, const float* state_dev, const float* ac
   if (rc) return rc;
   if (!h->have_rff) return fail(h, SIMSTEP_EINVAL, "simstep_load_rff has not been called");
   if (n_envs == 0) return SIMSTEP_OK;
-  if (!state_dev || !action_dev || !next_state_dev || !disc_dev || !w_dev)
+  if (!state_dev || (!action_dev && h->A > 0) || !next_state_dev || !disc_dev || !w_dev)
     return fail(h, SIMSTEP_EINVAL, "null device pointer (state, action, next_state, disc and w are required)");
   if (next_state_dev == state_dev) return fail(h, SIMSTEP_EINVAL, "next_state must not alias state in step_cost");
   cudaStream_t st = static_cast<cudaStream_t>(stream);

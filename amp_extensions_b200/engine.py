@@ -182,11 +182,17 @@ class Engine:
         self._check(self.lib.simstep_set_termination(self._h, C.byref(t)))
         self.generation += 1
 
-    def load_rff(self, weight, bias, split=True):
+    def load_rff(self, weight, bias, split=True, input_type=None):
+        """RBFLinearCost's rff layer (weight [D, in_dim], bias [D]).  input_type ('s', 'sa', 'ss' or 'sas') says which of
+        (s, a, s') step_cost builds the cost rows from; None infers it from in_dim, which fails where two types have
+        that width (state_dim == action_dim, or action_dim == 0)."""
+        if input_type not in _lib.RFF_INPUT:
+            raise ValueError(f"input_type must be one of 's', 'sa', 'ss', 'sas' or None, got {input_type!r}")
         w = weight.detach().to("cpu", torch.float32).contiguous()
         b = bias.detach().to("cpu", torch.float32).contiguous()
         with torch.cuda.device(self.device):
-            self._check(self.lib.simstep_load_rff(self._h, w.shape[0], w.shape[1], _ptr(w), _ptr(b), int(bool(split))))
+            self._check(self.lib.simstep_load_rff_typed(self._h, w.shape[0], w.shape[1], _lib.RFF_INPUT[input_type],
+                                                        _ptr(w), _ptr(b), int(bool(split))))
             self.generation += 1
         self.rff_dim, self.rff_in = int(w.shape[0]), int(w.shape[1])
         self.rff_split_loaded = bool(split)

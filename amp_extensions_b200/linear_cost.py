@@ -66,7 +66,8 @@ class RBFLinearCost:
         # its id() is not a stamp; an assignment to `.data` changes data_ptr()
         stamp = tuple((p.data_ptr(), p._version) for p in (self.rff.weight, self.rff.bias))
         if stamp != self._rff_stamp:
-            self._eng.load_rff(self.rff.weight.data, self.rff.bias.data, split=bool(self._split))
+            # this engine's "state" is the whole cost input row, whatever input_type built it
+            self._eng.load_rff(self.rff.weight.data, self.rff.bias.data, split=bool(self._split), input_type="s")
             self._rff_stamp = stamp
         if self._eng.rff_split_loaded and self._eng.rff_split != self.split_active:
             self._eng.set_rff_split(self.split_active)

@@ -58,7 +58,7 @@ class VecSimEnv:
         """Fuse an RBFLinearCost into the step: loads its rff layer into the ensemble's handle."""
         self.cost = cost
         eng = self.dynamic_ensemble.engine()
-        eng.load_rff(cost.rff.weight.data, cost.rff.bias.data, split=bool(cost._split))
+        eng.load_rff(cost.rff.weight.data, cost.rff.bias.data, split=bool(cost._split), input_type=cost.input_type)
         self.set_cost_weights(cost.w)
 
     def set_cost_weights(self, w):

@@ -147,9 +147,23 @@ int simstep_debug_chain_schedule(int32_t m_tiles, int32_t groups, int32_t sm_cou
                                  int32_t* items_out);
 
 /* Replaces the rff layer of RBFLinearCost (LC:53-55): weight_host [D,in_dim],
- * bias_host [D].  in_dim must be S (input_type 's'), 2S ('ss'), S+A ('sa') or
- * 2S+A ('sas').  split != 0 keeps ~21 mantissa bits of the pre-activation by
+ * bias_host [D].  input_type (SIMSTEP_RFF_INPUT_*, LC:115-126) says which of
+ * (s, a, s') the step's cost rows are built from; in_dim must be its width:
+ * S ('s'), S+A ('sa'), 2S ('ss') or 2S+A ('sas').  SIMSTEP_RFF_INPUT_AUTO infers
+ * the type from in_dim and fails with SIMSTEP_EINVAL where two types have that
+ * width (S == A: 'sa' and 'ss'; A == 0: 's' and 'sa', 'ss' and 'sas').  The
+ * type also fixes the column layout of explicit rows (simstep_rff_features,
+ * simstep_rff_dot, simstep_bonus_cost): [s | s'] for 'ss', the row as given
+ * otherwise.  split != 0 keeps ~21 mantissa bits of the pre-activation by
  * running the GEMM on hi/lo operand pairs. */
+#define SIMSTEP_RFF_INPUT_AUTO 0
+#define SIMSTEP_RFF_INPUT_S 1
+#define SIMSTEP_RFF_INPUT_SA 2
+#define SIMSTEP_RFF_INPUT_SS 3
+#define SIMSTEP_RFF_INPUT_SAS 4
+int simstep_load_rff_typed(simstep_handle* h, int32_t feature_dim, int32_t in_dim, int32_t input_type,
+                           const float* weight_host, const float* bias_host, int32_t split);
+/* simstep_load_rff_typed with SIMSTEP_RFF_INPUT_AUTO. */
 int simstep_load_rff(simstep_handle* h, int32_t feature_dim, int32_t in_dim,
                      const float* weight_host, const float* bias_host, int32_t split);
 
@@ -165,7 +179,9 @@ int simstep_set_rff_split(simstep_handle* h, int32_t split);
 
 /* DynamicsModel.forward(state, action, unnormalize_out=True) for ALL members
  * at once (DYN:216-233, DYN:422-433): delta_dev[m][e][:] is member m's
- * predicted state difference, layout [N][E][S]. */
+ * predicted state difference, layout [N][E][S].  Here and in simstep_discrepancy,
+ * simstep_step and simstep_step_cost, action_dev may be NULL when action_dim == 0
+ * (an empty action tensor has no storage). */
 int simstep_forward(simstep_handle* h, const float* state_dev, const float* action_dev, int64_t n_envs,
                     float* delta_dev, void* stream);
 
@@ -189,7 +205,7 @@ int simstep_step(simstep_handle* h, const float* state_dev, const float* action_
                  void* stream);
 
 /* simstep_step followed by RBFLinearCost.get_bonus_costs (LC:111-152) on the
- * same rows, input_type taken from simstep_load_rff:
+ * same rows, input_type taken from simstep_load_rff_typed:
  *   w_dev [D]       cost weights (LC:91)
  *   cost = (1-lambda_b)*clamp(phi.w, c_min, c_max) - lambda_b*min(disc/threshold,1)*c_min
  *   cost_dev, ipm_dev, bonus_dev: [E] each, any may be NULL (bonus is the

@@ -46,6 +46,8 @@ def test_abi_version_and_constants_match_header():
         assert int(re.search(rf"#define {macro} (\d+)", h).group(1)) == val
     for name, code in _lib.PREC.items():
         assert int(re.search(rf"#define SIMSTEP_PREC_{name.upper()} (\d+)", h).group(1)) == code
+    for name, code in _lib.RFF_INPUT.items():
+        assert int(re.search(rf"#define SIMSTEP_RFF_INPUT_{(name or 'auto').upper()} (\d+)", h).group(1)) == code
     n_cat = int(re.search(r"#define SIMSTEP_PROF_CATEGORIES (\d+)", h).group(1))
     assert len(_lib.PROF_CATEGORIES) == n_cat
 

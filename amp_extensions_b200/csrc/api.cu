@@ -9,6 +9,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <string>
 #include <utility>
 #include <vector>
@@ -33,7 +34,27 @@ thread_local std::string g_create_error;
 
 inline long long round_up(long long x, long long m) { return (x + m - 1) / m * m; }
 
-constexpr int kMaxDevices = 64;  // per-device bookkeeping of kernel attributes / scratch buffers
+constexpr int kMaxDevices = 64;  // per-device bookkeeping of kernel attributes
+
+constexpr size_t kGuardBytes = 64 * 1024;
+using GuardList = std::vector<std::pair<void*, size_t>>;  // (user pointer, user bytes) of a handle's guarded buffers
+
+// Frees a device buffer.  A guarded buffer (see dev_alloc) also leaves its handle's guard list.
+struct DevFree {
+  GuardList* guards = nullptr;
+  void operator()(void* p) const {
+    if (!guards) {
+      cudaFree(p);
+      return;
+    }
+    guards->erase(std::remove_if(guards->begin(), guards->end(), [p](const auto& g) { return g.first == p; }),
+                  guards->end());
+    cudaFree(static_cast<char*>(p) - kGuardBytes);
+  }
+};
+// The one owner of device memory: every buffer of a handle, its stores and the temporaries of a call.
+template <typename T>
+using DevPtr = std::unique_ptr<T, DevFree>;
 
 struct Layer {
   int in_ref = 0;   // reference nn.Linear in_features
@@ -43,15 +64,23 @@ struct Layer {
   int kb_x = 0, kb_h0 = 0, kb_h = 0;
   int out_col0 = 0; // column of this layer's output inside the activation buffer
   PackSegs segs{};
-  void* w = nullptr;      // [N][o_pad][k_pad] operand storage
-  float* bias = nullptr;  // [N][o_pad]
+  DevPtr<void> w;      // [N][o_pad][k_pad] operand storage
+  DevPtr<float> bias;  // [N][o_pad]
   CUtensorMap tmap_w;
   CUtensorMap tmap_w64;  // the same operand with a 64-row box (column halves of the chain kernel's shared units)
 };
 
+// Per-feature stores (imitation_api.inc, policy_api.inc, train_api.inc, npg_api.inc).
+struct ClipStore;
+struct PolicyStore;
+struct TrainStore;
+struct NpgStore;
+
 }  // namespace
 
 struct simstep_handle {
+  ~simstep_handle();  // defined after the stores (end of this file)
+
   simstep_config cfg{};
   int device = 0;
   int sm_count = 148;
@@ -61,24 +90,26 @@ struct simstep_handle {
   int S = 0, A = 0, N = 0, L = 0;
   int XP = 0, HT = 0, SP = 0;
   int DP = 0;  // pitch (floats) of the fp32 delta workspace rows: S rounded up to 4, so a row is 16-byte granular
+  // SIMSTEP_DEBUG_GUARDS=1 (read at simstep_create): every workspace buffer sits between two 64 KB guard zones filled with
+  // 0xA5; simstep_debug_check_guards counts the guard bytes that no longer are (compute-sanitizer is not available on
+  // the GPU boxes: this is the out-of-bounds check the test suite runs instead).  Declared before every buffer, so that
+  // it outlives them: a guarded buffer's deleter removes it from this list.
+  bool guards_on = false;
+  GuardList guard_allocs;
   std::vector<Layer> layers;  // L hidden + 1 final
-  unsigned long long* sat_dev = nullptr;  // normalised inputs beyond the fp16 range seen so far (prep kernel)
-  float* tf_dev = nullptr;         // mean_s | scale_s | mean_a | scale_a
-  float* out_scale_dev = nullptr;  // [SP]
-  float* out_shift_dev = nullptr;  // [SP]
+  DevPtr<unsigned long long> sat_dev;  // normalised inputs beyond the fp16 range seen so far (prep kernel)
+  DevPtr<double> moments_partial;      // [kMomentsMaxBlocks][3] (simstep_moments)
+  DevPtr<float> tf_dev;         // mean_s | scale_s | mean_a | scale_a
+  DevPtr<float> out_scale_dev;  // [SP]
+  DevPtr<float> out_shift_dev;  // [SP]
   bool have_ensemble = false;
 
   long long cap_rows = 0;
-  void* xbuf = nullptr;
-  void* hbuf = nullptr;
-  float* dws = nullptr;
-  // SIMSTEP_DEBUG_GUARDS=1 (read at simstep_create): every workspace buffer sits between two 64 KB guard zones filled with
-  // 0xA5; simstep_debug_check_guards counts the guard bytes that no longer are (compute-sanitizer is not available on
-  // the GPU boxes: this is the out-of-bounds check the test suite runs instead)
-  bool guards_on = false;
-  std::vector<std::pair<void*, size_t>> guard_allocs;  // (user pointer, user bytes)
+  DevPtr<void> xbuf;
+  DevPtr<void> hbuf;
+  DevPtr<float> dws;
   bool forward_was_chain = false;     // the workspace's deltas were written by the chain kernel (in row order)
-  unsigned int* chain_cnt = nullptr;  // chain kernel: tile counters of the shared units of the last round (zero between launches)
+  DevPtr<unsigned int> chain_cnt;  // chain kernel: tile counters of the shared units of the last round (zero between launches)
   CUtensorMap tmap_x, tmap_h, tmap_dws;
 
   // RFF cost
@@ -88,11 +119,11 @@ struct simstep_handle {
   int rff_split = 0;      // the three-product evaluation is in use (simstep_set_rff_split; needs rff_split_cap)
   int rff_type = 0;  // SIMSTEP_RFF_INPUT_S / SA / SS / SAS, resolved at load time
   int rff_col2 = 0;  // input_type 'ss': operand column of s' (s sits at 0); the weight columns are packed to match
-  void* rff_w = nullptr;
-  float* rff_b = nullptr;
-  float* rff_wpad = nullptr;
-  void* rffin = nullptr;
-  double* colsum_partial = nullptr;
+  DevPtr<void> rff_w;
+  DevPtr<float> rff_b;
+  DevPtr<float> rff_wpad;
+  DevPtr<void> rffin;
+  DevPtr<double> colsum_partial;
   CUtensorMap tmap_rffw, tmap_rffin;
   // feature net (MLPCost): hidden layers of this handle feed the cos-feature head instead of a packed input row
   bool feat_net = false;
@@ -100,13 +131,11 @@ struct simstep_handle {
   int cost_transform = 0;  // SIMSTEP_COST_*
 
   TermConst term{};
-  ImitConst* imit_dev = nullptr;
-  void* policy = nullptr;  // PolicyStore (policy_api.inc)
-  void* train = nullptr;   // TrainStore (train_api.inc)
-  void* npg = nullptr;     // NpgStore (npg_api.inc)
+  std::unique_ptr<ClipStore> clip;
+  std::unique_ptr<PolicyStore> policy;
+  std::unique_ptr<TrainStore> train;
+  std::unique_ptr<NpgStore> npg;
   bool train_raw = false;  // tf32 handle in training: parameters keep all fp32 bits (they are the master copy)
-  bool have_clip = false;
-  int dof = 0;
 
   // optional per-category device timing (simstep_profile_*)
   bool prof_on = false;
@@ -160,12 +189,18 @@ int fail(simstep_handle* h, int code, const std::string& msg) {
   return code;
 }
 
+// Reports a failed CUDA call.  The error is also cleared from the runtime's last-error slot: it has been reported
+// here, and a later call's cudaGetLastError() must not report it again.
+int cuda_fail(simstep_handle* h, int code, const std::string& what, cudaError_t e, const std::string& where = "") {
+  cudaGetLastError();
+  return fail(h, code, what + ": " + cudaGetErrorString(e) + where);
+}
+
 #define CU_TRY(h, expr)                                                                                   \
   do {                                                                                                    \
     cudaError_t e__ = (expr);                                                                             \
     if (e__ != cudaSuccess)                                                                               \
-      return fail(h, SIMSTEP_ECUDA, std::string(#expr) + ": " + cudaGetErrorString(e__) + " (" __FILE__ ":" + \
-                                        std::to_string(__LINE__) + ")");                                 \
+      return cuda_fail(h, SIMSTEP_ECUDA, #expr, e__, " (" __FILE__ ":" + std::to_string(__LINE__) + ")"); \
   } while (0)
 
 // Launch with programmatic stream serialization (see ptx::grid_dep_wait): the kernel may be scheduled while the
@@ -310,40 +345,34 @@ int pack_matrix(simstep_handle* h, int prec, const float* src_dev, int src_pitch
   return SIMSTEP_OK;
 }
 
-constexpr size_t kGuardBytes = 64 * 1024;
-
-cudaError_t ws_alloc_bytes(simstep_handle* h, void** p, size_t bytes) {
-  if (!h->guards_on) return cudaMalloc(p, bytes);
+// Frees `out`, then allocates `bytes` of device memory into it.  guarded: a workspace buffer, which
+// SIMSTEP_DEBUG_GUARDS=1 places between two guard zones of the handle (h may be null for an unguarded buffer).
+template <typename T>
+cudaError_t dev_alloc(simstep_handle* h, DevPtr<T>& out, size_t bytes, bool guarded = false) {
+  out.reset();
+  if (!guarded || !h->guards_on) {
+    void* p = nullptr;
+    cudaError_t e = cudaMalloc(&p, bytes);
+    if (e == cudaSuccess) out.reset(static_cast<T*>(p));
+    return e;
+  }
   char* base = nullptr;
   cudaError_t e = cudaMalloc(&base, bytes + 2 * kGuardBytes);
   if (e != cudaSuccess) return e;
   cudaMemset(base, 0xA5, kGuardBytes);
   cudaMemset(base + kGuardBytes + bytes, 0xA5, kGuardBytes);
-  *p = base + kGuardBytes;
-  h->guard_allocs.emplace_back(*p, bytes);
+  h->guard_allocs.emplace_back(base + kGuardBytes, bytes);
+  out = DevPtr<T>(reinterpret_cast<T*>(base + kGuardBytes), DevFree{&h->guard_allocs});
   return cudaSuccess;
 }
-template <typename T>
-cudaError_t ws_alloc(simstep_handle* h, T** p, size_t bytes) {
-  return ws_alloc_bytes(h, reinterpret_cast<void**>(p), bytes);
-}
-void ws_free(simstep_handle* h, void* p) {
-  if (!p) return;
-  for (size_t i = 0; i < h->guard_allocs.size(); ++i)
-    if (h->guard_allocs[i].first == p) {
-      cudaFree(static_cast<char*>(p) - kGuardBytes);
-      h->guard_allocs.erase(h->guard_allocs.begin() + i);
-      return;
-    }
-  cudaFree(p);
-}
 
-void free_workspace(simstep_handle* h) {
-  ws_free(h, h->xbuf); h->xbuf = nullptr;
-  ws_free(h, h->hbuf); h->hbuf = nullptr;
-  ws_free(h, h->dws); h->dws = nullptr;
-  cudaFree(h->chain_cnt); h->chain_cnt = nullptr;
-  ws_free(h, h->rffin); h->rffin = nullptr;
+// Frees the workspace (simstep_load_feature_net; ensure_workspace before it allocates a larger one).
+void drop_workspace(simstep_handle* h) {
+  h->xbuf.reset();
+  h->hbuf.reset();
+  h->dws.reset();
+  h->chain_cnt.reset();
+  h->rffin.reset();
   h->cap_rows = 0;
 }
 
@@ -359,35 +388,35 @@ int ensure_workspace(simstep_handle* h, long long rows) {
   if (rows <= h->cap_rows && (!h->have_rff || h->feat_net || h->rffin)) return SIMSTEP_OK;
   if (rows < h->cap_rows) rows = h->cap_rows;
   CU_TRY(h, cudaDeviceSynchronize());
-  free_workspace(h);
+  drop_workspace(h);  // before allocating the new one: holding both would raise the peak
   const int prec = h->cfg.precision;
   if (h->have_ensemble || h->S > 0) {
-    CU_TRY(h, ws_alloc(h, &h->xbuf, size_t(rows) * h->XP * h->esize));
-    if (h->HT > 0) CU_TRY(h, ws_alloc(h, &h->hbuf, size_t(h->N) * rows * h->HT * h->esize));
-    CU_TRY(h, ws_alloc(h, &h->dws, size_t(h->N) * rows * h->DP * sizeof(float)));
-    CU_TRY(h, cudaMalloc(&h->chain_cnt, size_t(h->sm_count) * 2 * sizeof(unsigned int)));
-    CU_TRY(h, cudaMemset(h->chain_cnt, 0, size_t(h->sm_count) * 2 * sizeof(unsigned int)));
-    CU_TRY(h, cudaMemset(h->xbuf, 0, size_t(rows) * h->XP * h->esize));
-    if (h->HT > 0) CU_TRY(h, cudaMemset(h->hbuf, 0, size_t(h->N) * rows * h->HT * h->esize));
-    int rc = encode_operand(h, &h->tmap_x, prec, h->xbuf, h->XP, rows, h->XP, kBlockM);
+    CU_TRY(h, dev_alloc(h, h->xbuf, size_t(rows) * h->XP * h->esize, true));
+    if (h->HT > 0) CU_TRY(h, dev_alloc(h, h->hbuf, size_t(h->N) * rows * h->HT * h->esize, true));
+    CU_TRY(h, dev_alloc(h, h->dws, size_t(h->N) * rows * h->DP * sizeof(float), true));
+    CU_TRY(h, dev_alloc(h, h->chain_cnt, size_t(h->sm_count) * 2 * sizeof(unsigned int)));
+    CU_TRY(h, cudaMemset(h->chain_cnt.get(), 0, size_t(h->sm_count) * 2 * sizeof(unsigned int)));
+    CU_TRY(h, cudaMemset(h->xbuf.get(), 0, size_t(rows) * h->XP * h->esize));
+    if (h->HT > 0) CU_TRY(h, cudaMemset(h->hbuf.get(), 0, size_t(h->N) * rows * h->HT * h->esize));
+    int rc = encode_operand(h, &h->tmap_x, prec, h->xbuf.get(), h->XP, rows, h->XP, kBlockM);
     if (rc) return rc;
     if (h->HT > 0) {
-      rc = encode_operand(h, &h->tmap_h, prec, h->hbuf, h->HT, static_cast<long long>(h->N) * rows, h->HT, kBlockM);
+      rc = encode_operand(h, &h->tmap_h, prec, h->hbuf.get(), h->HT, static_cast<long long>(h->N) * rows, h->HT, kBlockM);
       if (rc) return rc;
     } else {
       h->tmap_h = h->tmap_x;
     }
     // fp32 delta workspace, written by the final layer's TMA-store epilogue (32-float x 128-row boxes); the
     // map is DP columns wide, so the store clips the padded output columns instead of writing them
-    rc = encode_operand(h, &h->tmap_dws, SIMSTEP_PREC_TF32, h->dws, h->DP, static_cast<long long>(h->N) * rows, h->DP,
+    rc = encode_operand(h, &h->tmap_dws, SIMSTEP_PREC_TF32, h->dws.get(), h->DP, static_cast<long long>(h->N) * rows, h->DP,
                         kBlockM);
     if (rc) return rc;
   }
   if (h->have_rff && !h->feat_net) {  // a feature net's head reads the activation buffer instead
     const int rka = h->rff_split_cap ? 2 * h->RK : h->RK;  // [hi | lo]; the hi block is read twice by the GEMM
-    CU_TRY(h, ws_alloc(h, &h->rffin, size_t(rows) * rka * h->esize));
-    CU_TRY(h, cudaMemset(h->rffin, 0, size_t(rows) * rka * h->esize));
-    int rc = encode_operand(h, &h->tmap_rffin, prec, h->rffin, rka, rows, rka, kBlockM);
+    CU_TRY(h, dev_alloc(h, h->rffin, size_t(rows) * rka * h->esize, true));
+    CU_TRY(h, cudaMemset(h->rffin.get(), 0, size_t(rows) * rka * h->esize));
+    int rc = encode_operand(h, &h->tmap_rffin, prec, h->rffin.get(), rka, rows, rka, kBlockM);
     if (rc) return rc;
   }
   h->cap_rows = rows;
@@ -403,8 +432,8 @@ void launch_prep(simstep_handle* h, const float* s, const float* a, long long n,
                    reinterpret_cast<uintptr_t>(a) % 8 == 0;
   auto kern = vec ? prep_input_kernel<E, true> : prep_input_kernel<E, false>;
   launch_pdl(kern, dim3(grid), dim3(kPrepThreads), 0, st, s, a, h->S, h->A, h->XP, n, rows_pad,
-             h->cfg.transform ? h->tf_dev : nullptr, static_cast<typename E::storage*>(h->xbuf), w_src,
-             w_src ? h->rff_wpad : nullptr, h->D, h->sat_dev);
+             h->cfg.transform ? h->tf_dev.get() : nullptr, static_cast<typename E::storage*>(h->xbuf.get()),
+             w_src, w_src ? h->rff_wpad.get() : nullptr, h->D, h->sat_dev.get());
   g_launches++;
 }
 
@@ -438,7 +467,7 @@ bool chain_ok(const simstep_handle* h, long long rows_pad) {
 PostRff make_post_rff(const simstep_handle* h, bool fuse_rff) {
   PostRff rff{};
   if (fuse_rff) {
-    rff.out = h->rffin;
+    rff.out = h->rffin.get();
     rff.prec = h->cfg.precision;
     rff.RK = h->RK;
     rff.split = h->rff_split;
@@ -460,8 +489,8 @@ int launch_chain(simstep_handle* h, long long rows_pad, cudaStream_t st) {
   ca.groups = h->N;
   ca.a_rows_per_group = int(h->cap_rows);
   ca.out_rows_per_group = int(h->cap_rows);
-  ca.scale = h->cfg.transform ? h->out_scale_dev : nullptr;
-  ca.shift = h->cfg.transform ? h->out_shift_dev : nullptr;
+  ca.scale = h->cfg.transform ? h->out_scale_dev.get() : nullptr;
+  ca.shift = h->cfg.transform ? h->out_shift_dev.get() : nullptr;
   for (int l = 0; l <= h->L; ++l) {
     const Layer& ly = h->layers[l];
     cl.maps.w[l] = ly.tmap_w;
@@ -472,7 +501,7 @@ int launch_chain(simstep_handle* h, long long rows_pad, cudaStream_t st) {
     c.kb_h = ly.kb_h;
     c.b_rows_per_group = ly.o_pad;
     c.out_col0 = ly.out_col0;
-    c.bias = ly.bias;
+    c.bias = ly.bias.get();
     if (l < h->L) ca.hidden_tiles += c.n_tiles;
   }
   cl.maps.w_final64 = h->layers[h->L].tmap_w64;
@@ -480,10 +509,10 @@ int launch_chain(simstep_handle* h, long long rows_pad, cudaStream_t st) {
   // whole rounds run with the members of an env tile in sequence on one pair: all pairs then stream the SAME member's
   // weights at any time (measured -1.5 % on the launch against members side by side)
   int pairs = 1;
-  chain_schedule(ca.m_tiles, ca.groups, h->sm_count / 2, ca.hidden_tiles <= kChainMaxDepTiles && h->chain_cnt != nullptr,
+  chain_schedule(ca.m_tiles, ca.groups, h->sm_count / 2, ca.hidden_tiles <= kChainMaxDepTiles && h->chain_cnt,
                  &pairs, &ca.seq_rounds, &ca.tail_units);
   if (ca.tail_units > 0) {
-    ca.tail_cnt = h->chain_cnt;
+    ca.tail_cnt = h->chain_cnt.get();
     int t = 0;
     for (int l = 0; l < h->L; ++l)
       for (int n = 0; n < ca.layer[l].n_tiles; ++n, ++t) {
@@ -531,7 +560,7 @@ int run_ensemble_chunk(simstep_handle* h, const float* s, const float* a, long l
     ga.a_rows_per_group = int(h->cap_rows);
     ga.ax_rows_per_group = 0;
     ga.b_rows_per_group = ly.o_pad;
-    ga.bias = ly.bias;
+    ga.bias = ly.bias.get();
     ga.out_rows_per_group = int(h->cap_rows);
     // weight tiles with the evict_last L2 priority: every env tile of a member re-reads them while the activations
     // stream past (8 x (1024 x 4): -1 % on the five launches; neutral at 4 x (512 x 4))
@@ -547,8 +576,8 @@ int run_ensemble_chunk(simstep_handle* h, const float* s, const float* a, long l
                                              h->sm_count, st);
     } else {
       ga.out_col0 = 0;
-      ga.scale = h->cfg.transform ? h->out_scale_dev : nullptr;
-      ga.shift = h->cfg.transform ? h->out_shift_dev : nullptr;
+      ga.scale = h->cfg.transform ? h->out_scale_dev.get() : nullptr;
+      ga.shift = h->cfg.transform ? h->out_shift_dev.get() : nullptr;
       // the final layer is HBM-bound (every member re-reads its whole concat row for 226 outputs): run the members
       // of an env tile side by side (x comes from HBM once) and start with the rows whose last hidden slice the
       // previous launch wrote last (still in L2)
@@ -593,7 +622,7 @@ int launch_post(simstep_handle* h, const float* state, const int32_t* member, in
     }                                                                                                          \
     const long long pairs = (n + 1) / 2;                                                                       \
     const int grid = int(std::min<long long>((pairs + plan.rings - 1) / plan.rings, h->sm_count));             \
-    launch_pdl(kern, dim3(grid), dim3(plan.rings * 64), plan.smem, st, h->dws, h->cap_rows, h->DP, state, member, \
+    launch_pdl(kern, dim3(grid), dim3(plan.rings * 64), plan.smem, st, h->dws.get(), h->cap_rows, h->DP, state, member, \
                num_steps, h->S, n, next_state, disc, done, h->term, rff, plan.stages, post_reverse);           \
   } while (0)
 #define POST_CASE(NM)                                                                                          \
@@ -603,10 +632,10 @@ int launch_post(simstep_handle* h, const float* state, const int32_t* member, in
       else if (h->cfg.precision == SIMSTEP_PREC_TF32) POST_TMA_LAUNCH(NM, ElemTF32);                           \
       else POST_TMA_LAUNCH(NM, ElemBF16);                                                                      \
     } else if (vec2)                                                                                           \
-      launch_pdl(post_step_kernel<NM, 2>, dim3(blocks), dim3(kPostWarps * 32), smem, st, h->dws, h->cap_rows, h->DP, \
+      launch_pdl(post_step_kernel<NM, 2>, dim3(blocks), dim3(kPostWarps * 32), smem, st, h->dws.get(), h->cap_rows, h->DP, \
                  state, member, num_steps, h->S, n, next_state, disc, done, h->term, rff);                      \
     else                                                                                                       \
-      launch_pdl(post_step_kernel<NM, 1>, dim3(blocks), dim3(kPostWarps * 32), smem, st, h->dws, h->cap_rows, h->DP, \
+      launch_pdl(post_step_kernel<NM, 1>, dim3(blocks), dim3(kPostWarps * 32), smem, st, h->dws.get(), h->cap_rows, h->DP, \
                  state, member, num_steps, h->S, n, next_state, disc, done, h->term, rff);                      \
     break;
   switch (h->N) {
@@ -628,15 +657,15 @@ int launch_rff_pack(simstep_handle* h, const RffSrc& src, long long n, cudaStrea
   switch (h->cfg.precision) {
     case SIMSTEP_PREC_TF32:
       launch_pdl(rff_pack_kernel<ElemTF32>, dim3(grid), dim3(kPrepThreads), 0, st, src, h->RK, h->rff_split, pitch, n,
-                 rows_pad, static_cast<float*>(h->rffin));
+                 rows_pad, static_cast<float*>(h->rffin.get()));
       break;
     case SIMSTEP_PREC_FP16:
       launch_pdl(rff_pack_kernel<ElemF16>, dim3(grid), dim3(kPrepThreads), 0, st, src, h->RK, h->rff_split, pitch, n,
-                 rows_pad, static_cast<__half*>(h->rffin));
+                 rows_pad, static_cast<__half*>(h->rffin.get()));
       break;
     default:
       launch_pdl(rff_pack_kernel<ElemBF16>, dim3(grid), dim3(kPrepThreads), 0, st, src, h->RK, h->rff_split, pitch, n,
-                 rows_pad, static_cast<__nv_bfloat16*>(h->rffin));
+                 rows_pad, static_cast<__nv_bfloat16*>(h->rffin.get()));
   }
   g_launches++;
   CU_TRY(h, cudaGetLastError());
@@ -680,7 +709,7 @@ int launch_rff_gemm(simstep_handle* h, long long n, const float* w_pad, float* p
   ga.kb_h = h->rff_split ? h->RK / h->bk : 0;
   ga.a_rows_per_group = 0;
   ga.b_rows_per_group = h->D_pad;
-  ga.bias = h->rff_b;
+  ga.bias = h->rff_b.get();
   ga.scale = w_pad;
   ga.out = phi;
   ga.out_pitch = h->D;
@@ -708,7 +737,7 @@ int launch_rff_gemm(simstep_handle* h, long long n, const float* w_pad, float* p
 }
 
 int stage_w(simstep_handle* h, const float* w_dev, cudaStream_t st) {
-  CU_TRY(h, cudaMemcpyAsync(h->rff_wpad, w_dev, size_t(h->D) * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  CU_TRY(h, cudaMemcpyAsync(h->rff_wpad.get(), w_dev, size_t(h->D) * sizeof(float), cudaMemcpyDeviceToDevice, st));
   return SIMSTEP_OK;
 }
 
@@ -753,36 +782,91 @@ int upload_layer(simstep_handle* h, int l, const float* const* weights_host, con
   cudaStream_t st = nullptr;
   Layer& ly = h->layers[l];
   const size_t wbytes = size_t(h->N) * ly.o_pad * ly.k_pad * h->esize;
-  if (!ly.w) CU_TRY(h, cudaMalloc(&ly.w, wbytes));
-  if (!ly.bias) CU_TRY(h, cudaMalloc(&ly.bias, size_t(h->N) * ly.o_pad * sizeof(float)));
-  CU_TRY(h, cudaMemsetAsync(ly.w, 0, wbytes, st));
-  CU_TRY(h, cudaMemsetAsync(ly.bias, 0, size_t(h->N) * ly.o_pad * sizeof(float), st));
-  float* tmp = nullptr;
-  CU_TRY(h, cudaMalloc(&tmp, size_t(ly.out) * ly.in_ref * sizeof(float)));
+  if (!ly.w) CU_TRY(h, dev_alloc(h, ly.w, wbytes));
+  if (!ly.bias) CU_TRY(h, dev_alloc(h, ly.bias, size_t(h->N) * ly.o_pad * sizeof(float)));
+  CU_TRY(h, cudaMemsetAsync(ly.w.get(), 0, wbytes, st));
+  CU_TRY(h, cudaMemsetAsync(ly.bias.get(), 0, size_t(h->N) * ly.o_pad * sizeof(float), st));
+  DevPtr<float> tmp;
+  CU_TRY(h, dev_alloc(h, tmp, size_t(ly.out) * ly.in_ref * sizeof(float)));
   for (int m = 0; m < h->N; ++m) {
     const float* wsrc = weights_host[m * stride + l];
     const float* bsrc = biases_host[m * stride + l];
-    if (!wsrc || !bsrc) { cudaFree(tmp); return fail(h, SIMSTEP_EINVAL, "null weight or bias pointer"); }
-    CU_TRY(h, cudaMemcpyAsync(tmp, wsrc, size_t(ly.out) * ly.in_ref * sizeof(float), cudaMemcpyHostToDevice, st));
-    void* dst = static_cast<char*>(ly.w) + size_t(m) * ly.o_pad * ly.k_pad * h->esize;
-    int rc = pack_matrix(h, h->cfg.precision, tmp, ly.in_ref, ly.out, dst, ly.k_pad, ly.segs, h->train_raw ? 3 : 0, st);
-    if (rc) { cudaFree(tmp); return rc; }
-    CU_TRY(h, cudaMemcpyAsync(ly.bias + size_t(m) * ly.o_pad, bsrc, size_t(ly.out) * sizeof(float),
+    if (!wsrc || !bsrc) return fail(h, SIMSTEP_EINVAL, "null weight or bias pointer");
+    CU_TRY(h, cudaMemcpyAsync(tmp.get(), wsrc, size_t(ly.out) * ly.in_ref * sizeof(float), cudaMemcpyHostToDevice, st));
+    void* dst = static_cast<char*>(ly.w.get()) + size_t(m) * ly.o_pad * ly.k_pad * h->esize;
+    int rc = pack_matrix(h, h->cfg.precision, tmp.get(), ly.in_ref, ly.out, dst, ly.k_pad, ly.segs, h->train_raw ? 3 : 0,
+                         st);
+    if (rc) return rc;
+    CU_TRY(h, cudaMemcpyAsync(ly.bias.get() + size_t(m) * ly.o_pad, bsrc, size_t(ly.out) * sizeof(float),
                               cudaMemcpyHostToDevice, st));
     CU_TRY(h, cudaStreamSynchronize(st));  // tmp and the pageable host source are reused
   }
-  cudaFree(tmp);
-  if (int rc = encode_operand(h, &ly.tmap_w64, h->cfg.precision, ly.w, ly.k_pad, static_cast<long long>(h->N) * ly.o_pad,
-                              ly.k_pad, kBlockN / 4))
+  if (int rc = encode_operand(h, &ly.tmap_w64, h->cfg.precision, ly.w.get(), ly.k_pad,
+                              static_cast<long long>(h->N) * ly.o_pad, ly.k_pad, kBlockN / 4))
     return rc;
-  return encode_operand(h, &ly.tmap_w, h->cfg.precision, ly.w, ly.k_pad, static_cast<long long>(h->N) * ly.o_pad,
+  return encode_operand(h, &ly.tmap_w, h->cfg.precision, ly.w.get(), ly.k_pad, static_cast<long long>(h->N) * ly.o_pad,
                         ly.k_pad, kBlockN / 2);
 }
 
-void free_clip(simstep_handle* h);
-void free_policy(simstep_handle* h);
-void free_train(simstep_handle* h);
-void free_npg(simstep_handle* h);
+// Replaces the cost head: feature_dim features of operand rows RK wide, from an nn.Linear weight [feature_dim][in_dim]
+// whose columns are packed from operand column 0 (input_type 'ss': the s' half from column col2).  split: the weights
+// are packed as [hi | hi | lo] for the three-product evaluation.  The old head is freed first; the caller sets have_rff.
+int load_cost_head(simstep_handle* h, int feature_dim, int in_dim, int RK, int col2, bool split, const float* weight_host,
+                   const float* bias_host) {
+  CU_TRY(h, cudaDeviceSynchronize());
+  h->rff_w.reset();
+  h->rff_b.reset();
+  h->rff_wpad.reset();
+  h->colsum_partial.reset();
+  h->rffin.reset();  // the workspace's cost operand rows are RK wide
+  const int D_pad = int(round_up(feature_dim, kBlockN));
+  const int RKT = split ? 3 * RK : RK;  // K of the packed weight; the row operand stores 2*RK
+  const size_t wbytes = size_t(D_pad) * RKT * h->esize;
+  DevPtr<void> w;
+  DevPtr<float> b, wpad, tmp;
+  DevPtr<double> colsum;
+  CU_TRY(h, dev_alloc(h, w, wbytes));
+  CU_TRY(h, cudaMemset(w.get(), 0, wbytes));
+  CU_TRY(h, dev_alloc(h, b, size_t(D_pad) * sizeof(float)));
+  CU_TRY(h, cudaMemset(b.get(), 0, size_t(D_pad) * sizeof(float)));
+  CU_TRY(h, dev_alloc(h, wpad, size_t(D_pad) * sizeof(float)));
+  CU_TRY(h, cudaMemset(wpad.get(), 0, size_t(D_pad) * sizeof(float)));
+  CU_TRY(h, dev_alloc(h, colsum, size_t(1024) * D_pad * sizeof(double)));
+  CU_TRY(h, dev_alloc(h, tmp, size_t(feature_dim) * in_dim * sizeof(float)));
+  CU_TRY(h, cudaMemcpy(tmp.get(), weight_host, size_t(feature_dim) * in_dim * sizeof(float), cudaMemcpyHostToDevice));
+  CU_TRY(h, cudaMemcpy(b.get(), bias_host, size_t(feature_dim) * sizeof(float), cudaMemcpyHostToDevice));
+  PackSegs sg{};
+  sg.n = 1; sg.src0[0] = 0; sg.width[0] = in_dim;
+  if (col2 > 0) {
+    sg.n = 2; sg.width[0] = h->S;
+    sg.src0[1] = h->S; sg.width[1] = h->S;
+  }
+  // operand triple on the A side is [hi | lo | hi]; B side is [hi | hi | lo]
+  const int modes[3] = {1, 1, 2};
+  for (int part = 0; part < (split ? 3 : 1); ++part) {
+    sg.dst0[0] = part * RK;
+    sg.dst0[1] = part * RK + col2;
+    if (int rc = pack_matrix(h, h->cfg.precision, tmp.get(), in_dim, feature_dim, w.get(), RKT, sg, split ? modes[part] : 0,
+                             nullptr))
+      return rc;
+  }
+  CU_TRY(h, cudaDeviceSynchronize());
+  CUtensorMap tmap;
+  if (int rc = encode_operand(h, &tmap, h->cfg.precision, w.get(), RKT, D_pad, RKT, kBlockN / 2)) return rc;
+  h->D = feature_dim;
+  h->D_pad = D_pad;
+  h->rff_in = in_dim;
+  h->RK = RK;
+  h->RKT = RKT;
+  h->rff_col2 = col2;
+  h->rff_split_cap = h->rff_split = split ? 1 : 0;
+  h->rff_w = std::move(w);
+  h->rff_b = std::move(b);
+  h->rff_wpad = std::move(wpad);
+  h->colsum_partial = std::move(colsum);
+  h->tmap_rffw = tmap;
+  return SIMSTEP_OK;
+}
 
 // A handle's buffers, tensor maps and kernel attributes belong to the device it was created on; work can only be
 // enqueued from a thread whose current device is that one (one process per GPU does this by construction).
@@ -827,10 +911,10 @@ int simstep_create(const simstep_config* cfg, simstep_handle** out) {
     if (cfg->hidden[i] < 1) return fail(nullptr, SIMSTEP_EINVAL, "bad hidden size");
   int dev = 0;
   cudaError_t e = cudaGetDevice(&dev);
-  if (e != cudaSuccess) return fail(nullptr, SIMSTEP_ENODEV, std::string("cudaGetDevice: ") + cudaGetErrorString(e));
+  if (e != cudaSuccess) return cuda_fail(nullptr, SIMSTEP_ENODEV, "cudaGetDevice", e);
   cudaDeviceProp prop;
   e = cudaGetDeviceProperties(&prop, dev);
-  if (e != cudaSuccess) return fail(nullptr, SIMSTEP_ENODEV, std::string("cudaGetDeviceProperties: ") + cudaGetErrorString(e));
+  if (e != cudaSuccess) return cuda_fail(nullptr, SIMSTEP_ENODEV, "cudaGetDeviceProperties", e);
   if (prop.major != 10)
     return fail(nullptr, SIMSTEP_ENODEV,
                 "libsimstep is built for sm_100a only; device is sm_" + std::to_string(prop.major * 10 + prop.minor));
@@ -890,8 +974,10 @@ int simstep_create(const simstep_config* cfg, simstep_handle** out) {
       sg.src0[0] = 0; sg.width[0] = cfg->hidden[l - 1]; sg.dst0[0] = 0; sg.n = 1;
     }
   }
-  if (cudaMalloc(&h->sat_dev, sizeof(unsigned long long)) != cudaSuccess ||
-      cudaMemset(h->sat_dev, 0, sizeof(unsigned long long)) != cudaSuccess) {
+  if (dev_alloc(h, h->sat_dev, sizeof(unsigned long long)) != cudaSuccess ||
+      cudaMemset(h->sat_dev.get(), 0, sizeof(unsigned long long)) != cudaSuccess ||
+      dev_alloc(h, h->moments_partial, size_t(kMomentsMaxBlocks) * 3 * sizeof(double)) != cudaSuccess) {
+    cudaGetLastError();  // reported here, not again by a later call
     delete h;
     return fail(nullptr, SIMSTEP_ENOMEM, "cudaMalloc failed");
   }
@@ -907,23 +993,6 @@ int simstep_create(const simstep_config* cfg, simstep_handle** out) {
 int simstep_destroy(simstep_handle* h) {
   if (!h) return SIMSTEP_OK;
   cudaDeviceSynchronize();
-  free_workspace(h);
-  for (auto& ly : h->layers) {
-    cudaFree(ly.w);
-    cudaFree(ly.bias);
-  }
-  cudaFree(h->sat_dev);
-  cudaFree(h->tf_dev);
-  cudaFree(h->out_scale_dev);
-  cudaFree(h->out_shift_dev);
-  cudaFree(h->rff_w);
-  cudaFree(h->rff_b);
-  cudaFree(h->rff_wpad);
-  cudaFree(h->colsum_partial);
-  free_clip(h);
-  free_npg(h);
-  free_policy(h);
-  free_train(h);
   delete h;
   return SIMSTEP_OK;
 }
@@ -949,6 +1018,7 @@ int simstep_load_ensemble(simstep_handle* h, const float* const* weights_host, c
                           const float* const* transforms_host) {
   if (!h || !weights_host || !biases_host) return fail(h, SIMSTEP_EINVAL, "null argument");
   if (h->cfg.transform && !transforms_host) return fail(h, SIMSTEP_EINVAL, "transform set but no transforms given");
+  h->have_ensemble = false;  // until every layer is packed again: the weight buffers are rewritten in place
   DeviceScope dev_scope(h->device);  // parameters live on the handle's device; the caller's current device is restored
   const int nl = h->L + 1;
   for (int l = 0; l < nl; ++l) {
@@ -957,9 +1027,9 @@ int simstep_load_ensemble(simstep_handle* h, const float* const* weights_host, c
   }
   // transforms
   const int S = h->S, A = h->A;
-  if (!h->tf_dev) CU_TRY(h, cudaMalloc(&h->tf_dev, size_t(2 * S + 2 * A + 4) * sizeof(float)));
-  if (!h->out_scale_dev) CU_TRY(h, cudaMalloc(&h->out_scale_dev, size_t(h->SP) * sizeof(float)));
-  if (!h->out_shift_dev) CU_TRY(h, cudaMalloc(&h->out_shift_dev, size_t(h->SP) * sizeof(float)));
+  if (!h->tf_dev) CU_TRY(h, dev_alloc(h, h->tf_dev, size_t(2 * S + 2 * A + 4) * sizeof(float)));
+  if (!h->out_scale_dev) CU_TRY(h, dev_alloc(h, h->out_scale_dev, size_t(h->SP) * sizeof(float)));
+  if (!h->out_shift_dev) CU_TRY(h, dev_alloc(h, h->out_shift_dev, size_t(h->SP) * sizeof(float)));
   if (h->cfg.transform) {
     for (int i = 0; i < 6; ++i)  // the action vectors are empty (and may be NULL) when action_dim == 0
       if (!transforms_host[i] && !(A == 0 && (i == 2 || i == 3)))
@@ -973,9 +1043,9 @@ int simstep_load_ensemble(simstep_handle* h, const float* const* weights_host, c
     }
     std::memcpy(osh.data(), transforms_host[4], S * sizeof(float));
     std::memcpy(osc.data(), transforms_host[5], S * sizeof(float));
-    CU_TRY(h, cudaMemcpy(h->tf_dev, tf.data(), tf.size() * sizeof(float), cudaMemcpyHostToDevice));
-    CU_TRY(h, cudaMemcpy(h->out_scale_dev, osc.data(), osc.size() * sizeof(float), cudaMemcpyHostToDevice));
-    CU_TRY(h, cudaMemcpy(h->out_shift_dev, osh.data(), osh.size() * sizeof(float), cudaMemcpyHostToDevice));
+    CU_TRY(h, cudaMemcpy(h->tf_dev.get(), tf.data(), tf.size() * sizeof(float), cudaMemcpyHostToDevice));
+    CU_TRY(h, cudaMemcpy(h->out_scale_dev.get(), osc.data(), osc.size() * sizeof(float), cudaMemcpyHostToDevice));
+    CU_TRY(h, cudaMemcpy(h->out_shift_dev.get(), osh.data(), osh.size() * sizeof(float), cudaMemcpyHostToDevice));
   }
   CU_TRY(h, cudaDeviceSynchronize());
   h->have_ensemble = true;
@@ -1032,55 +1102,14 @@ int simstep_load_rff_typed(simstep_handle* h, int32_t feature_dim, int32_t in_di
     return fail(h, SIMSTEP_EINVAL, "rff in_dim " + std::to_string(in_dim) + " is not the width " +
                                        std::to_string(width[input_type]) + " of its input_type");
   }
-  DeviceScope dev_scope(h->device);  // parameters live on the handle's device; the caller's current device is restored
-  CU_TRY(h, cudaDeviceSynchronize());
-  cudaFree(h->rff_w); cudaFree(h->rff_b); cudaFree(h->rff_wpad); cudaFree(h->colsum_partial);
-  ws_free(h, h->rffin);
-  h->rff_w = nullptr; h->rff_b = nullptr; h->rff_wpad = nullptr; h->colsum_partial = nullptr;
-  h->rffin = nullptr;
   h->have_rff = false;
-  h->D = feature_dim;
-  h->D_pad = int(round_up(feature_dim, kBlockN));
-  h->rff_in = in_dim;
-  h->rff_type = input_type;
+  DeviceScope dev_scope(h->device);  // parameters live on the handle's device; the caller's current device is restored
   // input_type 'ss': s' starts at column S rounded up to 8 instead of S, so the step's fused tail writes both halves of
   // an operand row with aligned 16-byte stores; weight columns follow
-  h->rff_col2 = (input_type == SIMSTEP_RFF_INPUT_SS && !h->feat_net) ? int(round_up(h->S, 8)) : 0;
-  h->RK = int(round_up(h->rff_col2 > 0 ? h->rff_col2 + h->S : in_dim, 64));
-  h->rff_split_cap = split ? 1 : 0;
-  h->rff_split = h->rff_split_cap;
-  h->RKT = h->rff_split_cap ? 3 * h->RK : h->RK;  // K of the packed weight; the row operand stores 2*RK
-  const size_t wbytes = size_t(h->D_pad) * h->RKT * h->esize;
-  CU_TRY(h, cudaMalloc(&h->rff_w, wbytes));
-  CU_TRY(h, cudaMemset(h->rff_w, 0, wbytes));
-  CU_TRY(h, cudaMalloc(&h->rff_b, size_t(h->D_pad) * sizeof(float)));
-  CU_TRY(h, cudaMemset(h->rff_b, 0, size_t(h->D_pad) * sizeof(float)));
-  CU_TRY(h, cudaMalloc(&h->rff_wpad, size_t(h->D_pad) * sizeof(float)));
-  CU_TRY(h, cudaMemset(h->rff_wpad, 0, size_t(h->D_pad) * sizeof(float)));
-  CU_TRY(h, cudaMalloc(&h->colsum_partial, size_t(1024) * h->D_pad * sizeof(double)));
-  float* tmp = nullptr;
-  CU_TRY(h, cudaMalloc(&tmp, size_t(feature_dim) * in_dim * sizeof(float)));
-  CU_TRY(h, cudaMemcpy(tmp, weight_host, size_t(feature_dim) * in_dim * sizeof(float), cudaMemcpyHostToDevice));
-  CU_TRY(h, cudaMemcpy(h->rff_b, bias_host, size_t(feature_dim) * sizeof(float), cudaMemcpyHostToDevice));
-  PackSegs sg{};
-  sg.n = 1; sg.src0[0] = 0; sg.width[0] = in_dim;
-  if (h->rff_col2 > 0) {
-    sg.n = 2; sg.width[0] = h->S;
-    sg.src0[1] = h->S; sg.width[1] = h->S;
-  }
-  // operand triple on the A side is [hi | lo | hi]; B side is [hi | hi | lo]
-  const int modes[3] = {1, 1, 2};
-  for (int part = 0; part < (h->rff_split_cap ? 3 : 1); ++part) {
-    sg.dst0[0] = part * h->RK;
-    sg.dst0[1] = part * h->RK + h->rff_col2;
-    int rc = pack_matrix(h, h->cfg.precision, tmp, in_dim, feature_dim, h->rff_w, h->RKT, sg,
-                         h->rff_split_cap ? modes[part] : 0, nullptr);
-    if (rc) { cudaFree(tmp); return rc; }
-  }
-  CU_TRY(h, cudaDeviceSynchronize());
-  cudaFree(tmp);
-  int rc = encode_operand(h, &h->tmap_rffw, h->cfg.precision, h->rff_w, h->RKT, h->D_pad, h->RKT, kBlockN / 2);
-  if (rc) return rc;
+  const int col2 = (input_type == SIMSTEP_RFF_INPUT_SS && !h->feat_net) ? int(round_up(h->S, 8)) : 0;
+  const int RK = int(round_up(col2 > 0 ? col2 + h->S : in_dim, 64));
+  if (int rc = load_cost_head(h, feature_dim, in_dim, RK, col2, split != 0, weight_host, bias_host)) return rc;
+  h->rff_type = input_type;
   h->have_rff = true;
   return SIMSTEP_OK;
 }
@@ -1095,50 +1124,21 @@ int simstep_load_feature_net(simstep_handle* h, const float* const* weights_host
   if (h->N != 1 || h->A != 0 || h->cfg.transform || h->cfg.dense_connect)
     return fail(h, SIMSTEP_EINVAL,
                 "a feature net needs a handle with n_models = 1, action_dim = 0, transform = 0 and dense_connect = 0");
+  h->have_ensemble = false;
+  h->have_rff = false;
   DeviceScope dev_scope(h->device);  // parameters live on the handle's device; the caller's current device is restored
   CU_TRY(h, cudaDeviceSynchronize());
   for (int l = 0; l < h->L; ++l) {
     int rc = upload_layer(h, l, weights_host, biases_host, h->L);
     if (rc) return rc;
   }
-  if (!h->tf_dev) CU_TRY(h, cudaMalloc(&h->tf_dev, size_t(2 * h->S + 4) * sizeof(float)));
+  if (!h->tf_dev) CU_TRY(h, dev_alloc(h, h->tf_dev, size_t(2 * h->S + 4) * sizeof(float)));
   // head = cos-feature layer over the last hidden activations (reuses the random-feature GEMM epilogue)
-  cudaFree(h->rff_w); cudaFree(h->rff_b); cudaFree(h->rff_wpad); cudaFree(h->colsum_partial);
-  ws_free(h, h->rffin);
-  h->rff_w = nullptr; h->rff_b = nullptr; h->rff_wpad = nullptr; h->colsum_partial = nullptr;
-  h->rffin = nullptr;
-  h->have_rff = false;
   const Layer& fin = h->layers[h->L];
   const int in_dim = h->L > 0 ? h->cfg.hidden[h->L - 1] : h->S;
-  h->D = feature_dim;
-  h->D_pad = int(round_up(feature_dim, kBlockN));
-  h->rff_in = in_dim;
-  h->RK = (fin.kb_x + fin.kb_h) * h->bk;  // the padded width of the last hidden layer's slice (or of the input)
-  h->rff_split = 0;
-  h->rff_split_cap = 0;
-  h->rff_col2 = 0;
-  h->RKT = h->RK;
-  const size_t wbytes = size_t(h->D_pad) * h->RKT * h->esize;
-  CU_TRY(h, cudaMalloc(&h->rff_w, wbytes));
-  CU_TRY(h, cudaMemset(h->rff_w, 0, wbytes));
-  CU_TRY(h, cudaMalloc(&h->rff_b, size_t(h->D_pad) * sizeof(float)));
-  CU_TRY(h, cudaMemset(h->rff_b, 0, size_t(h->D_pad) * sizeof(float)));
-  CU_TRY(h, cudaMalloc(&h->rff_wpad, size_t(h->D_pad) * sizeof(float)));
-  CU_TRY(h, cudaMemset(h->rff_wpad, 0, size_t(h->D_pad) * sizeof(float)));
-  CU_TRY(h, cudaMalloc(&h->colsum_partial, size_t(1024) * h->D_pad * sizeof(double)));
-  float* tmp = nullptr;
-  CU_TRY(h, cudaMalloc(&tmp, size_t(feature_dim) * in_dim * sizeof(float)));
-  CU_TRY(h, cudaMemcpy(tmp, head_weight_host, size_t(feature_dim) * in_dim * sizeof(float), cudaMemcpyHostToDevice));
-  CU_TRY(h, cudaMemcpy(h->rff_b, head_bias_host, size_t(feature_dim) * sizeof(float), cudaMemcpyHostToDevice));
-  PackSegs sg{};
-  sg.n = 1; sg.src0[0] = 0; sg.width[0] = in_dim; sg.dst0[0] = 0;
-  int rc = pack_matrix(h, h->cfg.precision, tmp, in_dim, feature_dim, h->rff_w, h->RKT, sg, 0, nullptr);
-  CU_TRY(h, cudaDeviceSynchronize());
-  cudaFree(tmp);
-  if (rc) return rc;
-  rc = encode_operand(h, &h->tmap_rffw, h->cfg.precision, h->rff_w, h->RKT, h->D_pad, h->RKT, kBlockN / 2);
-  if (rc) return rc;
-  free_workspace(h);
+  const int RK = (fin.kb_x + fin.kb_h) * h->bk;  // the padded width of the last hidden layer's slice (or of the input)
+  if (int rc = load_cost_head(h, feature_dim, in_dim, RK, 0, false, head_weight_host, head_bias_host)) return rc;
+  drop_workspace(h);
   h->feat_mode = head_mode;
   h->feat_net = true;
   h->have_rff = true;
@@ -1156,8 +1156,8 @@ int simstep_set_cost_transform(simstep_handle* h, int32_t transform) {
 int simstep_saturation_count(simstep_handle* h, int64_t* count_out, int32_t reset) {
   if (!h || !count_out) return fail(h, SIMSTEP_EINVAL, "null argument");
   unsigned long long v = 0;
-  CU_TRY(h, cudaMemcpy(&v, h->sat_dev, sizeof(v), cudaMemcpyDeviceToHost));  // synchronises with the device
-  if (reset) CU_TRY(h, cudaMemset(h->sat_dev, 0, sizeof(v)));
+  CU_TRY(h, cudaMemcpy(&v, h->sat_dev.get(), sizeof(v), cudaMemcpyDeviceToHost));  // synchronises with the device
+  if (reset) CU_TRY(h, cudaMemset(h->sat_dev.get(), 0, sizeof(v)));
   *count_out = static_cast<int64_t>(v);
   return SIMSTEP_OK;
 }
@@ -1237,7 +1237,7 @@ int simstep_forward(simstep_handle* h, const float* state_dev, const float* acti
     const long long n = std::min<long long>(h->cap_rows, n_envs - r0);
     if ((rc = run_ensemble_chunk(h, state_dev + r0 * h->S, action_dev + r0 * h->A, n, st))) return rc;
     const long long total = static_cast<long long>(h->N) * n * h->S;
-    extract_delta_kernel<<<grid_for(total, 256, h->sm_count), 256, 0, st>>>(h->dws, h->cap_rows, h->DP, h->N, h->S, n,
+    extract_delta_kernel<<<grid_for(total, 256, h->sm_count), 256, 0, st>>>(h->dws.get(), h->cap_rows, h->DP, h->N, h->S, n,
                                                                             delta_dev, n_envs, r0);
     g_launches++;
     CU_TRY(h, cudaGetLastError());
@@ -1315,7 +1315,7 @@ int simstep_step_cost(simstep_handle* h, const float* state_dev, const float* ac
     const CombineArgs comb = make_combine(h, disc_dev + r0, lambda_b, threshold, c_min, c_max, clamp_cost, nullptr,
                                           cost_dev ? cost_dev + r0 : nullptr, ipm_dev ? ipm_dev + r0 : nullptr,
                                           bonus_dev ? bonus_dev + r0 : nullptr);
-    if ((rc = launch_rff_gemm(h, n, h->rff_wpad, nullptr, st, &comb))) return rc;
+    if ((rc = launch_rff_gemm(h, n, h->rff_wpad.get(), nullptr, st, &comb))) return rc;
   }
   return SIMSTEP_OK;
 }
@@ -1343,8 +1343,8 @@ int simstep_rff_features(simstep_handle* h, const float* x_dev, int64_t n_rows, 
   if (phi_sum_dev) {
     const int nb = int(std::min<long long>(1024, std::max<long long>(1, (n_rows + 63) / 64)));
     const int rpb = int((n_rows + nb - 1) / nb);
-    colsum_partial_kernel<<<nb, 256, 0, st>>>(phi_dev, n_rows, h->D, rpb > 0 ? rpb : 1, h->colsum_partial);
-    colsum_final_kernel<<<(h->D + 255) / 256, 256, 0, st>>>(h->colsum_partial, nb, h->D, phi_sum_dev, 0);
+    colsum_partial_kernel<<<nb, 256, 0, st>>>(phi_dev, n_rows, h->D, rpb > 0 ? rpb : 1, h->colsum_partial.get());
+    colsum_final_kernel<<<(h->D + 255) / 256, 256, 0, st>>>(h->colsum_partial.get(), nb, h->D, phi_sum_dev, 0);
     g_launches += 2;
     CU_TRY(h, cudaGetLastError());
   }
@@ -1384,7 +1384,7 @@ int simstep_bonus_cost(simstep_handle* h, const float* x_dev, const float* disc_
             : make_combine(h, disc_dev + r0, lambda_b, threshold, c_min, c_max, clamp_cost, nullptr,
                            cost_dev ? cost_dev + r0 : nullptr, ipm_dev ? ipm_dev + r0 : nullptr,
                            bonus_dev ? bonus_dev + r0 : nullptr);
-    if ((rc = launch_rff_gemm(h, n, h->rff_wpad, nullptr, st, &comb))) return rc;
+    if ((rc = launch_rff_gemm(h, n, h->rff_wpad.get(), nullptr, st, &comb))) return rc;
   }
   return SIMSTEP_OK;
 }
@@ -1439,65 +1439,53 @@ int simstep_debug_gemm(int32_t precision, int32_t groups, int64_t m, int32_t n, 
   CU_TRY(h, cudaGetDevice(&dev));
   CU_TRY(h, cudaGetDeviceProperties(&prop, dev));
   if (prop.major != 10) return fail(nullptr, SIMSTEP_ENODEV, "libsimstep is built for sm_100a only");
-  void *ap = nullptr, *bp = nullptr;
-  float *biasp = nullptr, *dp = nullptr;  // dp: padded fp32 output [groups][m_pad][n_pad] of the TMA-store epilogue
-  CU_TRY(h, cudaMalloc(&ap, size_t(groups) * m_pad * k_pad * es));
-  CU_TRY(h, cudaMalloc(&bp, size_t(groups) * n_pad * k_pad * es));
-  CU_TRY(h, cudaMalloc(&biasp, size_t(groups) * n_pad * sizeof(float)));
-  CU_TRY(h, cudaMalloc(&dp, size_t(groups) * m_pad * n_pad * sizeof(float)));
-  CU_TRY(h, cudaMemsetAsync(ap, 0, size_t(groups) * m_pad * k_pad * es, st));
-  CU_TRY(h, cudaMemsetAsync(bp, 0, size_t(groups) * n_pad * k_pad * es, st));
-  CU_TRY(h, cudaMemsetAsync(biasp, 0, size_t(groups) * n_pad * sizeof(float), st));
+  DevPtr<void> ap, bp;
+  DevPtr<float> biasp, dp;  // dp: padded fp32 output [groups][m_pad][n_pad] of the TMA-store epilogue
+  CU_TRY(h, dev_alloc(h, ap, size_t(groups) * m_pad * k_pad * es));
+  CU_TRY(h, dev_alloc(h, bp, size_t(groups) * n_pad * k_pad * es));
+  CU_TRY(h, dev_alloc(h, biasp, size_t(groups) * n_pad * sizeof(float)));
+  CU_TRY(h, dev_alloc(h, dp, size_t(groups) * m_pad * n_pad * sizeof(float)));
+  CU_TRY(h, cudaMemsetAsync(ap.get(), 0, size_t(groups) * m_pad * k_pad * es, st));
+  CU_TRY(h, cudaMemsetAsync(bp.get(), 0, size_t(groups) * n_pad * k_pad * es, st));
+  CU_TRY(h, cudaMemsetAsync(biasp.get(), 0, size_t(groups) * n_pad * sizeof(float), st));
   PackSegs sg{};
   sg.n = 1; sg.src0[0] = 0; sg.width[0] = k; sg.dst0[0] = 0;
-  int rc = SIMSTEP_OK;
-  for (int g = 0; g < groups && !rc; ++g) {
-    rc = pack_matrix(h, precision, a_dev + size_t(g) * m * k, k, int(m), static_cast<char*>(ap) + size_t(g) * m_pad * k_pad * es,
-                     k_pad, sg, 0, st);
-    if (!rc)
-      rc = pack_matrix(h, precision, b_dev + size_t(g) * n * k, k, n, static_cast<char*>(bp) + size_t(g) * n_pad * k_pad * es,
-                       k_pad, sg, 0, st);
-    if (!rc && bias_dev)
-      if (cudaMemcpyAsync(biasp + size_t(g) * n_pad, bias_dev + size_t(g) * n, size_t(n) * sizeof(float),
-                          cudaMemcpyDeviceToDevice, st) != cudaSuccess)
-        rc = fail(nullptr, SIMSTEP_ECUDA, "bias copy failed");
+  for (int g = 0; g < groups; ++g) {
+    if (int rc = pack_matrix(h, precision, a_dev + size_t(g) * m * k, k, int(m),
+                             static_cast<char*>(ap.get()) + size_t(g) * m_pad * k_pad * es, k_pad, sg, 0, st))
+      return rc;
+    if (int rc = pack_matrix(h, precision, b_dev + size_t(g) * n * k, k, n,
+                             static_cast<char*>(bp.get()) + size_t(g) * n_pad * k_pad * es, k_pad, sg, 0, st))
+      return rc;
+    if (bias_dev)
+      CU_TRY(h, cudaMemcpyAsync(biasp.get() + size_t(g) * n_pad, bias_dev + size_t(g) * n, size_t(n) * sizeof(float),
+                                cudaMemcpyDeviceToDevice, st));
   }
-  if (!rc) {
-    cudaError_t pe = cudaStreamSynchronize(st);
-    if (pe != cudaSuccess) rc = fail(nullptr, SIMSTEP_ECUDA, std::string("debug gemm pack stage: ") + cudaGetErrorString(pe));
-  }
+  CU_TRY(h, cudaStreamSynchronize(st));
   CUtensorMap ta, tb, td;
-  if (!rc) rc = encode_operand(h, &ta, precision, ap, k_pad, groups * m_pad, k_pad, kBlockM);
-  if (!rc) rc = encode_operand(h, &tb, precision, bp, k_pad, groups * n_pad, k_pad, kBlockN / 2);
-  if (!rc) rc = encode_operand(h, &td, SIMSTEP_PREC_TF32, dp, n_pad, groups * m_pad, n_pad, kBlockM);
-  if (!rc) {
-    GemmArgs ga{};
-    ga.m_tiles = int(m_pad / (kBlockM * 2));
-    ga.n_tiles = int(n_pad / kBlockN);
-    ga.groups = groups;
-    ga.kb_x = 0;
-    ga.kb_h0 = 0;
-    ga.kb_h = int(k_pad / bk);
-    ga.a_rows_per_group = int(m_pad);
-    ga.b_rows_per_group = int(n_pad);
-    ga.bias = biasp;
-    ga.out_rows_per_group = int(m_pad);
-    ga.out_col0 = 0;
-    rc = launch_gemm<kEpiFinal>(h, precision, ta, ta, tb, td, ga, prop.multiProcessorCount, st);
-  }
-  if (!rc) {
-    const long long total = static_cast<long long>(groups) * m * n;
-    extract_delta_kernel<<<grid_for(total, 256, prop.multiProcessorCount), 256, 0, st>>>(dp, m_pad, int(n_pad), groups, n,
-                                                                                         m, d_dev, m, 0);
-    g_launches++;
-  }
-  cudaError_t e = cudaStreamSynchronize(st);
-  cudaFree(ap);
-  cudaFree(bp);
-  cudaFree(biasp);
-  cudaFree(dp);
-  if (!rc && e != cudaSuccess) return fail(nullptr, SIMSTEP_ECUDA, std::string("debug gemm: ") + cudaGetErrorString(e));
-  return rc;
+  if (int rc = encode_operand(h, &ta, precision, ap.get(), k_pad, groups * m_pad, k_pad, kBlockM)) return rc;
+  if (int rc = encode_operand(h, &tb, precision, bp.get(), k_pad, groups * n_pad, k_pad, kBlockN / 2)) return rc;
+  if (int rc = encode_operand(h, &td, SIMSTEP_PREC_TF32, dp.get(), n_pad, groups * m_pad, n_pad, kBlockM)) return rc;
+  GemmArgs ga{};
+  ga.m_tiles = int(m_pad / (kBlockM * 2));
+  ga.n_tiles = int(n_pad / kBlockN);
+  ga.groups = groups;
+  ga.kb_x = 0;
+  ga.kb_h0 = 0;
+  ga.kb_h = int(k_pad / bk);
+  ga.a_rows_per_group = int(m_pad);
+  ga.b_rows_per_group = int(n_pad);
+  ga.bias = biasp.get();
+  ga.out_rows_per_group = int(m_pad);
+  ga.out_col0 = 0;
+  if (int rc = launch_gemm<kEpiFinal>(h, precision, ta, ta, tb, td, ga, prop.multiProcessorCount, st)) return rc;
+  const long long total = static_cast<long long>(groups) * m * n;
+  extract_delta_kernel<<<grid_for(total, 256, prop.multiProcessorCount), 256, 0, st>>>(dp.get(), m_pad, int(n_pad), groups,
+                                                                                       n, m, d_dev, m, 0);
+  g_launches++;
+  CU_TRY(h, cudaGetLastError());
+  CU_TRY(h, cudaStreamSynchronize(st));  // the owners free the buffers on return
+  return SIMSTEP_OK;
 }
 
 }  // extern "C"
@@ -1506,3 +1494,7 @@ int simstep_debug_gemm(int32_t precision, int32_t groups, int64_t m, int32_t n, 
 #include "policy_api.inc"
 #include "train_api.inc"
 #include "npg_api.inc"
+
+simstep_handle::~simstep_handle() {
+  for (cudaEvent_t e : prof_ev) cudaEventDestroy(e);
+}

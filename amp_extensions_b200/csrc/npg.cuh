@@ -25,6 +25,7 @@ constexpr int kNpgThreads = 512;
 constexpr int kNpgWarps = kNpgThreads / 32;
 constexpr int kNpgMaxItems = 3;                       // 4x4 gradient blocks per thread (48 accumulator registers)
 constexpr int kNpgMaxBlocks = kNpgThreads * kNpgMaxItems;
+constexpr int kNpgMaxRows = 64;                       // rows per tile: 64, or 32 when that plan does not fit
 constexpr int kNpgExtra = 4;                          // per-row scalar sums after the log_std entries
 constexpr int kNpgCgThreads = 1024;
 
@@ -140,10 +141,22 @@ npg_rows_kernel(const NpgConst q, const float* __restrict__ pack, const float* _
 #pragma unroll
     for (int e = 0; e < 16; ++e) acc[j][e] = 0.f;
   float ext = 0.f;  // thread t < A + kNpgExtra owns per-row scalar column t
+  // source row of each tile row: idx[row] or row; -1 past n_rows or masked out by `valid`.  A masked row enters the
+  // tile as zeros, like a row past the end, so whatever it holds (NaN, Inf) never reaches a product that is summed.
+  __shared__ long long s_src[kNpgMaxRows];
 
   const long long n_tiles = (a.n_rows + R - 1) / R;
   for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
     const long long r0 = tile * R;
+    for (int r = threadIdx.x; r < R; r += blockDim.x) {  // last read by the previous tile's output stage, then a barrier
+      const long long row = r0 + r;
+      long long src = -1;
+      if (row < a.n_rows) {
+        src = a.idx ? a.idx[row] : row;
+        if (a.valid && !a.valid[src]) src = -1;
+      }
+      s_src[r] = src;
+    }
     __syncthreads();  // the previous tile's tiles are consumed
     // ---- input rows: normalised observations, the constant-1 column, and (FVP) the cached hidden activations
     {
@@ -151,13 +164,8 @@ npg_rows_kernel(const NpgConst q, const float* __restrict__ pack, const float* _
       const int sa0 = q.sa[0];
       for (int i = threadIdx.x; i < R * c.obs_dim; i += blockDim.x) {
         const int r = i / c.obs_dim, k = i - r * c.obs_dim;
-        const long long row = r0 + r;
-        float v = 0.f;
-        if (row < a.n_rows) {
-          const long long src = a.idx ? a.idx[row] : row;
-          v = (a.obs[src * c.obs_dim + k] - in_shift[k]) / in_div[k];
-        }
-        a0[r * sa0 + k] = v;
+        const long long src = s_src[r];
+        a0[r * sa0 + k] = src >= 0 ? (a.obs[src * c.obs_dim + k] - in_shift[k]) / in_div[k] : 0.f;
       }
       for (int l = 0; l < L; ++l)
         for (int r = threadIdx.x; r < R; r += blockDim.x) {
@@ -170,7 +178,7 @@ npg_rows_kernel(const NpgConst q, const float* __restrict__ pack, const float* _
           for (int i = threadIdx.x; i < R * w; i += blockDim.x) {
             const int r = i / w, k = i - r * w;
             const long long row = r0 + r;
-            sm_npg[q.a_off[l] + r * q.sa[l] + k] = row < a.n_rows ? a.cache[row * q.cache_w + q.cache_off[l] + k] : 0.f;
+            sm_npg[q.a_off[l] + r * q.sa[l] + k] = s_src[r] >= 0 ? a.cache[row * q.cache_w + q.cache_off[l] + k] : 0.f;
           }
         }
       }
@@ -246,11 +254,8 @@ npg_rows_kernel(const NpgConst q, const float* __restrict__ pack, const float* _
     {
       const int sdL = q.sd[L - 1];
       for (int r = threadIdx.x; r < R; r += blockDim.x) {
-        const long long row = r0 + r;
-        bool ok = row < a.n_rows;
-        long long src = row;
-        if (ok && a.idx) src = a.idx[row];
-        if (ok && a.valid) ok = a.valid[src] != 0;
+        const long long src = s_src[r];
+        const bool ok = src >= 0;
         float* y = sm_npg + q.d_off[L - 1] + r * sdL;
         float* e = E + r * q.se;
         for (int j = 0; j < A + kNpgExtra; ++j) e[j] = 0.f;

@@ -9,7 +9,9 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <map>
 #include <memory>
+#include <mutex>
 #include <string>
 #include <utility>
 #include <vector>
@@ -24,17 +26,34 @@
 #include "policy.cuh"
 #include "post_tma.cuh"
 #include "train.cuh"
+#include "launch.h"
+
+namespace simstep {
+
+std::atomic<long long> g_launches{0};
+
+cudaError_t raise_smem_limit(const void* kern, int device, size_t bytes) {
+  static std::mutex mu;
+  static std::map<std::pair<const void*, int>, size_t> limits;  // the limit set so far of (kernel, device)
+  std::lock_guard<std::mutex> lock(mu);
+  size_t& limit = limits[{kern, device}];
+  if (limit >= bytes) return cudaSuccess;
+  const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(bytes));
+  if (e == cudaSuccess) limit = bytes;
+  return e;
+}
+
+}  // namespace simstep
 
 using namespace simstep;
 
 namespace {
 
-std::atomic<long long> g_launches{0};
 thread_local std::string g_create_error;
 
 inline long long round_up(long long x, long long m) { return (x + m - 1) / m * m; }
 
-constexpr int kMaxDevices = 64;  // per-device bookkeeping of kernel attributes
+constexpr int kMaxDevices = 64;  // per-device bookkeeping of device attributes
 
 constexpr size_t kGuardBytes = 64 * 1024;
 using GuardList = std::vector<std::pair<void*, size_t>>;  // (user pointer, user bytes) of a handle's guarded buffers
@@ -203,21 +222,12 @@ int cuda_fail(simstep_handle* h, int code, const std::string& what, cudaError_t 
       return cuda_fail(h, SIMSTEP_ECUDA, #expr, e__, " (" __FILE__ ":" + std::to_string(__LINE__) + ")"); \
   } while (0)
 
-// Launch with programmatic stream serialization (see ptx::grid_dep_wait): the kernel may be scheduled while the
-// previous kernel of the stream drains; every kernel launched this way starts with grid_dep_wait().
+// launch_kernel (launch.h) from an entry point: a refused launch is reported as CU_TRY reports a failed call.
 template <typename... KArgs, typename... Args>
-cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
+int launch(simstep_handle* h, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, unsigned flags,
+           Args&&... args) {
+  const cudaError_t e = launch_kernel(kern, grid, block, smem, st, flags, std::forward<Args>(args)...);
+  return e == cudaSuccess ? SIMSTEP_OK : cuda_fail(h, SIMSTEP_ECUDA, "kernel launch", e);
 }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -260,39 +270,18 @@ int encode_operand(simstep_handle* h, CUtensorMap* map, int prec, void* base, lo
 template <typename E, int MODE, int EG>
 int launch_gemm_t(simstep_handle* h, const CUtensorMap& ax, const CUtensorMap& ah, const CUtensorMap& b,
                   const CUtensorMap& out, const GemmArgs& ga, int sm_count, cudaStream_t st) {
-  static bool attr_set[kMaxDevices] = {};  // function attributes are per device
   auto kern = gemm_tcgen05_kernel<E, MODE, EG>;
   using Plan = GemmPlan<EG, !epi_is_rff(MODE)>;
   constexpr size_t smem = Plan::smem_bytes();
   int dev = h ? h->device : 0;  // h is null for simstep_debug_gemm: use the calling thread's current device
   if (!h) CU_TRY(h, cudaGetDevice(&dev));
-  bool& attr_done = attr_set[dev % kMaxDevices];
-  if (!attr_done) {
-    CU_TRY(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    attr_done = true;
-  }
+  CU_TRY(h, raise_smem_limit(reinterpret_cast<const void*>(kern), dev, smem));
   const int total = ga.m_tiles * ga.n_tiles * ga.groups;
   if (total <= 0) return SIMSTEP_OK;
   // persistent: one CTA pair per tile slot, at most one CTA per SM
   const int n_inner = ga.n_inner > 1 ? ga.n_inner : 1;
   const int slots = std::min(total / n_inner, sm_count / 2);
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(unsigned(slots * 2));
-  cfg.blockDim = dim3(Plan::kThreads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 2;
-  CU_TRY(h, cudaLaunchKernelEx(&cfg, kern, ax, ah, b, out, ga));
-  g_launches++;
-  return SIMSTEP_OK;
+  return launch(h, kern, dim3(unsigned(slots * 2)), dim3(Plan::kThreads), smem, st, kPdl | kPair, ax, ah, b, out, ga);
 }
 
 template <int MODE>
@@ -302,18 +291,19 @@ int launch_gemm(simstep_handle* h, int prec, const CUtensorMap& ax, const CUtens
   // element, no store staging), and store modes whose whole K fits the shortened ring (the first layer).
   constexpr bool kStore = !epi_is_rff(MODE);
   const bool wide = MODE != kEpiFinal && (!kStore || ga.kb_x + ga.kb_h <= GemmPlan<2, true>::kStages);
-#define SIMSTEP_GEMM_CASE(ELEM)                                                                    \
-  if constexpr (MODE != kEpiFinal) {                                                               \
-    if (wide) return launch_gemm_t<ELEM, MODE, 2>(h, ax, ah, b, out, ga, sm_count, st);             \
-  }                                                                                                \
-  return launch_gemm_t<ELEM, MODE, 1>(h, ax, ah, b, out, ga, sm_count, st)
-  switch (prec) {
-    case SIMSTEP_PREC_TF32: SIMSTEP_GEMM_CASE(ElemTF32);
-    case SIMSTEP_PREC_FP16: SIMSTEP_GEMM_CASE(ElemF16);
-    case SIMSTEP_PREC_BF16: SIMSTEP_GEMM_CASE(ElemBF16);
-  }
-#undef SIMSTEP_GEMM_CASE
-  return fail(h, SIMSTEP_EINVAL, "unknown precision");
+  int rc = SIMSTEP_OK;
+  if (!with_elem(prec, [&](auto e) {
+        using E = decltype(e);
+        if constexpr (MODE != kEpiFinal) {
+          if (wide) {
+            rc = launch_gemm_t<E, MODE, 2>(h, ax, ah, b, out, ga, sm_count, st);
+            return;
+          }
+        }
+        rc = launch_gemm_t<E, MODE, 1>(h, ax, ah, b, out, ga, sm_count, st);
+      }))
+    return fail(h, SIMSTEP_EINVAL, "unknown precision");
+  return rc;
 }
 
 int grid_for(long long work_items, int threads, int sm_count) {
@@ -327,22 +317,14 @@ int grid_for(long long work_items, int threads, int sm_count) {
 int pack_matrix(simstep_handle* h, int prec, const float* src_dev, int src_pitch, int rows, void* dst,
                 long long dst_pitch, const PackSegs& segs, int mode, cudaStream_t st) {
   if (rows <= 0) return SIMSTEP_OK;
-  switch (prec) {
-    case SIMSTEP_PREC_TF32:
-      pack_weight_kernel<ElemTF32><<<rows, 128, 0, st>>>(src_dev, src_pitch, rows, static_cast<float*>(dst),
-                                                         dst_pitch, segs, mode);
-      break;
-    case SIMSTEP_PREC_FP16:
-      pack_weight_kernel<ElemF16><<<rows, 128, 0, st>>>(src_dev, src_pitch, rows, static_cast<__half*>(dst),
-                                                        dst_pitch, segs, mode);
-      break;
-    default:
-      pack_weight_kernel<ElemBF16><<<rows, 128, 0, st>>>(src_dev, src_pitch, rows, static_cast<__nv_bfloat16*>(dst),
-                                                         dst_pitch, segs, mode);
-  }
-  g_launches++;
-  CU_TRY(h, cudaGetLastError());
-  return SIMSTEP_OK;
+  int rc = SIMSTEP_OK;
+  if (!with_elem(prec, [&](auto e) {
+        using E = decltype(e);
+        rc = launch(h, pack_weight_kernel<E>, dim3(rows), dim3(128), 0, st, kPlain, src_dev, src_pitch, rows,
+                    static_cast<typename E::storage*>(dst), dst_pitch, segs, mode);
+      }))
+    return fail(h, SIMSTEP_EINVAL, "unknown precision");
+  return rc;
 }
 
 // Frees `out`, then allocates `bytes` of device memory into it.  guarded: a workspace buffer, which
@@ -423,18 +405,22 @@ int ensure_workspace(simstep_handle* h, long long rows) {
   return SIMSTEP_OK;
 }
 
-template <typename E>
-void launch_prep(simstep_handle* h, const float* s, const float* a, long long n, long long rows_pad,
-                 const float* w_src, cudaStream_t st) {
+int launch_prep(simstep_handle* h, const float* s, const float* a, long long n, long long rows_pad, const float* w_src,
+                cudaStream_t st) {
   const int grid = int(std::min<long long>(rows_pad, static_cast<long long>(h->sm_count) * 16));
   // column pairs are read with one 8-byte load when no pair straddles the state / action boundary
   const bool vec = h->S % 2 == 0 && h->A % 2 == 0 && reinterpret_cast<uintptr_t>(s) % 8 == 0 &&
                    reinterpret_cast<uintptr_t>(a) % 8 == 0;
-  auto kern = vec ? prep_input_kernel<E, true> : prep_input_kernel<E, false>;
-  launch_pdl(kern, dim3(grid), dim3(kPrepThreads), 0, st, s, a, h->S, h->A, h->XP, n, rows_pad,
-             h->cfg.transform ? h->tf_dev.get() : nullptr, static_cast<typename E::storage*>(h->xbuf.get()),
-             w_src, w_src ? h->rff_wpad.get() : nullptr, h->D, h->sat_dev.get());
-  g_launches++;
+  int rc = SIMSTEP_OK;
+  if (!with_elem(h->cfg.precision, [&](auto e) {
+        using E = decltype(e);
+        rc = launch(h, vec ? prep_input_kernel<E, true> : prep_input_kernel<E, false>, dim3(grid), dim3(kPrepThreads), 0,
+                    st, kPdl, s, a, h->S, h->A, h->XP, n, rows_pad, h->cfg.transform ? h->tf_dev.get() : nullptr,
+                    static_cast<typename E::storage*>(h->xbuf.get()), w_src, w_src ? h->rff_wpad.get() : nullptr, h->D,
+                    h->sat_dev.get());
+      }))
+    return fail(h, SIMSTEP_EINVAL, "unknown precision");
+  return rc;
 }
 
 // The column-fused forward pass (gemm_chain.cuh): every layer of a (member, 256-row env tile) on one CTA pair, the
@@ -521,7 +507,6 @@ int launch_chain(simstep_handle* h, long long rows_pad, cudaStream_t st) {
       }
   }
   CU_TRY(h, launch_ensemble_chain(h->cfg.precision, h->cfg.activation != SIMSTEP_ACT_RELU, cl, h->sm_count, h->device, st));
-  g_launches++;
   return SIMSTEP_OK;
 }
 
@@ -534,14 +519,9 @@ int run_ensemble_chunk(simstep_handle* h, const float* s, const float* a, long l
   if (last_layer == -2) last_layer = h->L;  // -1: input preparation only
   const long long rows_pad = round_up(n, h->row_align);
   {
-  ProfScope ps(h, SIMSTEP_PROF_PREP, st);
-  switch (h->cfg.precision) {
-    case SIMSTEP_PREC_TF32: launch_prep<ElemTF32>(h, s, a, n, rows_pad, w_stage, st); break;
-    case SIMSTEP_PREC_FP16: launch_prep<ElemF16>(h, s, a, n, rows_pad, w_stage, st); break;
-    default: launch_prep<ElemBF16>(h, s, a, n, rows_pad, w_stage, st);
+    ProfScope ps(h, SIMSTEP_PROF_PREP, st);
+    if (int rc = launch_prep(h, s, a, n, rows_pad, w_stage, st)) return rc;
   }
-  }
-  CU_TRY(h, cudaGetLastError());
   ProfScope ps(h, SIMSTEP_PROF_ENSEMBLE_GEMM, st);
   h->forward_was_chain = false;
   if (last_layer == h->L && chain_ok(h, rows_pad)) {
@@ -611,42 +591,32 @@ int launch_post(simstep_handle* h, const float* state, const int32_t* member, in
   // the chain kernel writes the deltas in row order: the last rows are the ones still in L2, so the rows are walked
   // backwards; the per-layer final GEMM itself runs backwards, its LAST rows are row 0's
   const int post_reverse = h->forward_was_chain ? 1 : 0;
-#define POST_TMA_LAUNCH(NM, ET)                                                                                \
-  do {                                                                                                         \
-    auto kern = h->S == 226 ? post_step_tma_kernel<NM, ET, 226> : post_step_tma_kernel<NM, ET, 0>;             \
-    static size_t attr_smem[kMaxDevices][2] = {};  /* function attributes are per device */                   \
-    size_t& attr_ref = attr_smem[h->device % kMaxDevices][h->S == 226 ? 1 : 0];                                                                               \
-    if (attr_ref < plan.smem) {                                                                                \
-      CU_TRY(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(plan.smem)));      \
-      attr_ref = plan.smem;                                                                                    \
-    }                                                                                                          \
-    const long long pairs = (n + 1) / 2;                                                                       \
-    const int grid = int(std::min<long long>((pairs + plan.rings - 1) / plan.rings, h->sm_count));             \
-    launch_pdl(kern, dim3(grid), dim3(plan.rings * 64), plan.smem, st, h->dws.get(), h->cap_rows, h->DP, state, member, \
-               num_steps, h->S, n, next_state, disc, done, h->term, rff, plan.stages, post_reverse);           \
-  } while (0)
-#define POST_CASE(NM)                                                                                          \
-  case NM:                                                                                                     \
-    if (tma) {                                                                                                 \
-      if (rff.out == nullptr || h->cfg.precision == SIMSTEP_PREC_FP16) POST_TMA_LAUNCH(NM, ElemF16);           \
-      else if (h->cfg.precision == SIMSTEP_PREC_TF32) POST_TMA_LAUNCH(NM, ElemTF32);                           \
-      else POST_TMA_LAUNCH(NM, ElemBF16);                                                                      \
-    } else if (vec2)                                                                                           \
-      launch_pdl(post_step_kernel<NM, 2>, dim3(blocks), dim3(kPostWarps * 32), smem, st, h->dws.get(), h->cap_rows, h->DP, \
-                 state, member, num_steps, h->S, n, next_state, disc, done, h->term, rff);                      \
-    else                                                                                                       \
-      launch_pdl(post_step_kernel<NM, 1>, dim3(blocks), dim3(kPostWarps * 32), smem, st, h->dws.get(), h->cap_rows, h->DP, \
-                 state, member, num_steps, h->S, n, next_state, disc, done, h->term, rff);                      \
-    break;
-  switch (h->N) {
-    POST_CASE(1) POST_CASE(2) POST_CASE(3) POST_CASE(4) POST_CASE(5) POST_CASE(6) POST_CASE(7) POST_CASE(8)
-    default: return fail(h, SIMSTEP_EINVAL, "n_models must be in [1, 8]");
-  }
-#undef POST_CASE
-#undef POST_TMA_LAUNCH
-  g_launches++;
-  CU_TRY(h, cudaGetLastError());
-  return SIMSTEP_OK;
+  int rc = SIMSTEP_OK;
+  if (!with_members(h->N, [&](auto nm) {
+        constexpr int NM = decltype(nm)::value;
+        if (!tma) {
+          rc = launch(h, vec2 ? post_step_kernel<NM, 2> : post_step_kernel<NM, 1>, dim3(blocks), dim3(kPostWarps * 32),
+                      smem, st, kPdl, h->dws.get(), h->cap_rows, h->DP, state, member, num_steps, h->S, n, next_state,
+                      disc, done, h->term, rff);
+          return;
+        }
+        // the element type only matters for the cost operand rows: without them the ElemF16 instantiation runs
+        const bool known = with_elem(rff.out == nullptr ? SIMSTEP_PREC_FP16 : h->cfg.precision, [&](auto e) {
+          using E = decltype(e);
+          auto kern = h->S == 226 ? post_step_tma_kernel<NM, E, 226> : post_step_tma_kernel<NM, E, 0>;
+          if (cudaError_t err = raise_smem_limit(reinterpret_cast<const void*>(kern), h->device, plan.smem)) {
+            rc = cuda_fail(h, SIMSTEP_ECUDA, "raise_smem_limit", err);
+            return;
+          }
+          const long long pairs = (n + 1) / 2;
+          const int grid = int(std::min<long long>((pairs + plan.rings - 1) / plan.rings, h->sm_count));
+          rc = launch(h, kern, dim3(grid), dim3(plan.rings * 64), plan.smem, st, kPdl, h->dws.get(), h->cap_rows, h->DP,
+                      state, member, num_steps, h->S, n, next_state, disc, done, h->term, rff, plan.stages, post_reverse);
+        });
+        if (!known) rc = fail(h, SIMSTEP_EINVAL, "unknown precision");
+      }))
+    return fail(h, SIMSTEP_EINVAL, "n_models must be in [1, 8]");
+  return rc;
 }
 
 int launch_rff_pack(simstep_handle* h, const RffSrc& src, long long n, cudaStream_t st) {
@@ -654,22 +624,14 @@ int launch_rff_pack(simstep_handle* h, const RffSrc& src, long long n, cudaStrea
   const long long rows_pad = round_up(n, h->row_align);
   const int grid = int(std::min<long long>(rows_pad, static_cast<long long>(h->sm_count) * 16));
   const int pitch = h->rff_split_cap ? 2 * h->RK : h->RK;
-  switch (h->cfg.precision) {
-    case SIMSTEP_PREC_TF32:
-      launch_pdl(rff_pack_kernel<ElemTF32>, dim3(grid), dim3(kPrepThreads), 0, st, src, h->RK, h->rff_split, pitch, n,
-                 rows_pad, static_cast<float*>(h->rffin.get()));
-      break;
-    case SIMSTEP_PREC_FP16:
-      launch_pdl(rff_pack_kernel<ElemF16>, dim3(grid), dim3(kPrepThreads), 0, st, src, h->RK, h->rff_split, pitch, n,
-                 rows_pad, static_cast<__half*>(h->rffin.get()));
-      break;
-    default:
-      launch_pdl(rff_pack_kernel<ElemBF16>, dim3(grid), dim3(kPrepThreads), 0, st, src, h->RK, h->rff_split, pitch, n,
-                 rows_pad, static_cast<__nv_bfloat16*>(h->rffin.get()));
-  }
-  g_launches++;
-  CU_TRY(h, cudaGetLastError());
-  return SIMSTEP_OK;
+  int rc = SIMSTEP_OK;
+  if (!with_elem(h->cfg.precision, [&](auto e) {
+        using E = decltype(e);
+        rc = launch(h, rff_pack_kernel<E>, dim3(grid), dim3(kPrepThreads), 0, st, kPdl, src, h->RK, h->rff_split, pitch,
+                    n, rows_pad, static_cast<typename E::storage*>(h->rffin.get()));
+      }))
+    return fail(h, SIMSTEP_EINVAL, "unknown precision");
+  return rc;
 }
 
 // What happens to a row's feature dot product (see CombineArgs).
@@ -1237,10 +1199,9 @@ int simstep_forward(simstep_handle* h, const float* state_dev, const float* acti
     const long long n = std::min<long long>(h->cap_rows, n_envs - r0);
     if ((rc = run_ensemble_chunk(h, state_dev + r0 * h->S, action_dev + r0 * h->A, n, st))) return rc;
     const long long total = static_cast<long long>(h->N) * n * h->S;
-    extract_delta_kernel<<<grid_for(total, 256, h->sm_count), 256, 0, st>>>(h->dws.get(), h->cap_rows, h->DP, h->N, h->S, n,
-                                                                            delta_dev, n_envs, r0);
-    g_launches++;
-    CU_TRY(h, cudaGetLastError());
+    if ((rc = launch(h, extract_delta_kernel, dim3(grid_for(total, 256, h->sm_count)), dim3(256), 0, st, kPlain,
+                     h->dws.get(), h->cap_rows, h->DP, h->N, h->S, n, delta_dev, n_envs, r0)))
+      return rc;
   }
   return SIMSTEP_OK;
 }
@@ -1343,10 +1304,11 @@ int simstep_rff_features(simstep_handle* h, const float* x_dev, int64_t n_rows, 
   if (phi_sum_dev) {
     const int nb = int(std::min<long long>(1024, std::max<long long>(1, (n_rows + 63) / 64)));
     const int rpb = int((n_rows + nb - 1) / nb);
-    colsum_partial_kernel<<<nb, 256, 0, st>>>(phi_dev, n_rows, h->D, rpb > 0 ? rpb : 1, h->colsum_partial.get());
-    colsum_final_kernel<<<(h->D + 255) / 256, 256, 0, st>>>(h->colsum_partial.get(), nb, h->D, phi_sum_dev, 0);
-    g_launches += 2;
-    CU_TRY(h, cudaGetLastError());
+    if ((rc = launch(h, colsum_partial_kernel, dim3(nb), dim3(256), 0, st, kPlain, phi_dev, n_rows, h->D,
+                     rpb > 0 ? rpb : 1, h->colsum_partial.get())))
+      return rc;
+    return launch(h, colsum_final_kernel, dim3((h->D + 255) / 256), dim3(256), 0, st, kPlain, h->colsum_partial.get(), nb,
+                  h->D, phi_sum_dev, 0);
   }
   return SIMSTEP_OK;
 }
@@ -1391,10 +1353,9 @@ int simstep_bonus_cost(simstep_handle* h, const float* x_dev, const float* disc_
 
 int simstep_reduce_max_sum(simstep_handle* h, const float* x_dev, int64_t n, double* out_dev, void* stream) {
   if (!h || !out_dev || n < 0 || (n > 0 && !x_dev)) return fail(h, SIMSTEP_EINVAL, "bad argument");
-  reduce_max_sum_kernel<<<1, 1024, 0, static_cast<cudaStream_t>(stream)>>>(x_dev, n, out_dev);
-  g_launches++;
-  CU_TRY(h, cudaGetLastError());
-  return SIMSTEP_OK;
+  if (int rc = check_device(h)) return rc;
+  return launch(h, reduce_max_sum_kernel, dim3(1), dim3(1024), 0, static_cast<cudaStream_t>(stream), kPlain, x_dev, n,
+                out_dev);
 }
 
 int simstep_profile_enable(simstep_handle* h, int32_t enable) {
@@ -1480,10 +1441,9 @@ int simstep_debug_gemm(int32_t precision, int32_t groups, int64_t m, int32_t n, 
   ga.out_col0 = 0;
   if (int rc = launch_gemm<kEpiFinal>(h, precision, ta, ta, tb, td, ga, prop.multiProcessorCount, st)) return rc;
   const long long total = static_cast<long long>(groups) * m * n;
-  extract_delta_kernel<<<grid_for(total, 256, prop.multiProcessorCount), 256, 0, st>>>(dp.get(), m_pad, int(n_pad), groups,
-                                                                                       n, m, d_dev, m, 0);
-  g_launches++;
-  CU_TRY(h, cudaGetLastError());
+  if (int rc = launch(h, extract_delta_kernel, dim3(grid_for(total, 256, prop.multiProcessorCount)), dim3(256), 0, st,
+                      kPlain, dp.get(), m_pad, int(n_pad), groups, n, m, d_dev, m, 0))
+    return rc;
   CU_TRY(h, cudaStreamSynchronize(st));  // the owners free the buffers on return
   return SIMSTEP_OK;
 }

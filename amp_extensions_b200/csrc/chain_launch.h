@@ -12,7 +12,7 @@ struct ChainLaunch {
 };
 
 // prec: SIMSTEP_PREC_*; tanh_act: hidden activation is tanh (ReLU otherwise).  Enqueues the launch on `st`
-// (programmatic stream serialization): min(units, sm_count / 2) CTA pairs.
+// (programmatic stream serialization): min(units, sm_count / 2) CTA pairs.  device: the calling thread's current device.
 cudaError_t launch_ensemble_chain(int prec, bool tanh_act, const ChainLaunch& cl, int sm_count, int device,
                                   cudaStream_t st);
 

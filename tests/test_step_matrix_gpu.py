@@ -533,8 +533,8 @@ def step_branches(c, prec, align, itype=None):
     vec2 = S % 2 == 0 and align % 8 == 0
     if post_tma_plan_ok(S, N) and vec2 and align % 16 == 0:
         b.add(("post tma", N))
-        b.add(("post tma S", 226 if S == 226 else 0))              # POST_TMA_LAUNCH: the S = 226 specialisation
-        # POST_CASE: the ElemF16 instantiation unless the kernel stores tf32 or bf16 cost rows
+        b.add(("post tma S", 226 if S == 226 else 0))              # the S = 226 specialisation
+        # the ElemF16 instantiation unless the kernel stores tf32 or bf16 cost rows
         b.add(("post tma cost rows", prec if fuse else None))
     else:
         b.add(("post float2" if vec2 else "post scalar", N))

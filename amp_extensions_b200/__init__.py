@@ -9,6 +9,7 @@ Host-side mirror of the reference's plugin surface for this one hot path:
   SimEnv / VecSimEnv                 (reference gym-simenv/gym_simenv/envs/sim_env.py)
   ImitationReward                    (reference DeepMimicCore/scenes/SceneImitate.cpp)
   sampler.get_samples / sample_points (reference milo/milo/sampler.py, batched on the device)
+  MLPBaseline / DeviceMLPBaseline     (reference mjrl/mjrl/baselines/mlp_baseline.py)
 
 All compute goes through libsimstep.so (include/simstep.h); there is no CPU fallback.
 """
@@ -24,6 +25,7 @@ from .character import Character, humanoid3d  # noqa: F401
 from .imitation import ImitationReward  # noqa: F401
 from .motion import MotionClip  # noqa: F401
 from . import sampler  # noqa: F401
+from .baseline import DeviceMLPBaseline, MLPBaseline  # noqa: F401
 
 
 def register_gym(env_id="simenv-v0"):

@@ -138,6 +138,13 @@ _SIGNATURES = {
     "simstep_npg_apply": (C.c_int, [_c_void_p, C.c_double, C.c_int32, _c_void_p]),
     "simstep_npg_diag": (C.c_int, [_c_void_p, _c_void_p, _c_void_p, _c_void_p, _c_void_p, C.c_int64, _c_void_p, _c_void_p]),
     "simstep_npg_scalars": (C.c_int, [_c_void_p, _c_void_p, _c_void_p]),
+    "simstep_baseline_init": (C.c_int, [_c_void_p, C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.c_float, C.c_float,
+                                        C.c_float, C.c_float, C.c_float, _c_void_p, _c_void_p, _c_void_p, C.c_int64]),
+    "simstep_baseline_state": (C.c_int, [_c_void_p, C.c_int32, _c_void_p, _c_void_p, _c_void_p, _c_void_p,
+                                         C.POINTER(C.c_int64)]),
+    "simstep_baseline_predict": (C.c_int, [_c_void_p, _c_void_p, _c_void_p, C.c_int64, _c_void_p, _c_void_p]),
+    "simstep_baseline_fit": (C.c_int, [_c_void_p, _c_void_p, _c_void_p, _c_void_p, C.c_int64, _c_void_p, C.c_int64,
+                                       C.c_int32, C.c_int32, _c_void_p]),
     "simstep_histogram": (C.c_int, [_c_void_p, _c_void_p, C.c_int64, C.c_double, C.c_double, C.c_int32, _c_void_p,
                                     _c_void_p]),
     "simstep_quantile_op": (C.c_int, [_c_void_p, C.c_int32, _c_void_p, C.c_int64, C.c_int32, _c_void_p, _c_void_p,

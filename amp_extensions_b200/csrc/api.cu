@@ -17,6 +17,7 @@
 #include <vector>
 
 #include "../../include/simstep.h"
+#include "baseline.cuh"
 #include "elementwise.cuh"
 #include "gemm_tcgen05.cuh"
 #include "chain_launch.h"
@@ -89,11 +90,12 @@ struct Layer {
   CUtensorMap tmap_w64;  // the same operand with a 64-row box (column halves of the chain kernel's shared units)
 };
 
-// Per-feature stores (imitation_api.inc, policy_api.inc, train_api.inc, npg_api.inc).
+// Per-feature stores (imitation_api.inc, policy_api.inc, train_api.inc, npg_api.inc, baseline_api.inc).
 struct ClipStore;
 struct PolicyStore;
 struct TrainStore;
 struct NpgStore;
+struct BaselineStore;
 
 }  // namespace
 
@@ -154,6 +156,7 @@ struct simstep_handle {
   std::unique_ptr<PolicyStore> policy;
   std::unique_ptr<TrainStore> train;
   std::unique_ptr<NpgStore> npg;
+  std::unique_ptr<BaselineStore> baseline;  // value baseline: independent of the ensemble and the policy
   bool train_raw = false;  // tf32 handle in training: parameters keep all fp32 bits (they are the master copy)
 
   // optional per-category device timing (simstep_profile_*)
@@ -1454,6 +1457,7 @@ int simstep_debug_gemm(int32_t precision, int32_t groups, int64_t m, int32_t n, 
 #include "policy_api.inc"
 #include "train_api.inc"
 #include "npg_api.inc"
+#include "baseline_api.inc"
 
 simstep_handle::~simstep_handle() {
   for (cudaEvent_t e : prof_ev) cudaEventDestroy(e);

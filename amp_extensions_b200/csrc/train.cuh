@@ -184,6 +184,7 @@ struct OptimArgs {
   float beta2;
   float eps;
   float grad_clip;   // 0: off; else clip_grad_norm_(max_norm) over one member's parameters
+  float weight_decay;  // L2 term added to the gradient, g + wd * w (torch.optim's weight_decay, not decoupled); 0: off
 };
 
 // Step-dependent optimiser quantities live on the device so that a captured CUDA graph of the training step can
@@ -192,16 +193,20 @@ struct OptimState {
   long long step;    // optimiser steps taken, including the current one
   float bc1, bc2;    // Adam bias corrections 1 - beta^step
   int first_step;    // SGD: the momentum buffer starts as the gradient itself
+  int skip;          // the update is a no-op (a replayed value-baseline step past the end of its epoch)
 };
 
+// One optimiser step begins: the step counter and the quantities derived from it.  Called by one thread.
+__device__ inline void optim_tick(OptimState* st, float beta1, float beta2) {
+  const long long t = st->step + 1;
+  st->step = t;
+  st->first_step = t == 1;
+  st->bc1 = static_cast<float>(1.0 - pow(static_cast<double>(beta1), static_cast<double>(t)));
+  st->bc2 = static_cast<float>(1.0 - pow(static_cast<double>(beta2), static_cast<double>(t)));
+}
+
 __global__ void train_tick_kernel(OptimState* st, float beta1, float beta2) {
-  if (threadIdx.x == 0 && blockIdx.x == 0) {
-    const long long t = st->step + 1;
-    st->step = t;
-    st->first_step = t == 1;
-    st->bc1 = static_cast<float>(1.0 - pow(static_cast<double>(beta1), static_cast<double>(t)));
-    st->bc2 = static_cast<float>(1.0 - pow(static_cast<double>(beta2), static_cast<double>(t)));
-  }
+  if (threadIdx.x == 0 && blockIdx.x == 0) optim_tick(st, beta1, beta2);
 }
 
 // Every parameter tensor of the ensemble in one launch: blockIdx.z = tensor, blockIdx.y = member.  Member g's
@@ -245,6 +250,7 @@ __global__ void train_optim_batch_kernel(const ParamDesc* __restrict__ descs, in
   const ParamDesc d = descs[blockIdx.z];
   const int gi = blockIdx.y;
   const OptimState os = *state;
+  if (os.skip) return;
   float coef = 1.f;
   if (a.grad_clip > 0.f) {
     const float c = a.grad_clip / (static_cast<float>(sqrt(sumsq[gi])) + 1e-6f);
@@ -254,8 +260,9 @@ __global__ void train_optim_batch_kernel(const ParamDesc* __restrict__ descs, in
   const long long gbase = gi * d.g_stride + d.g_off;
   for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < d.count;
        i += static_cast<long long>(gridDim.x) * blockDim.x) {
-    const float grad = d.g[gbase + i] * coef;
+    float grad = d.g[gbase + i] * coef;
     float w = pp[i];
+    if (a.weight_decay != 0.f) grad = fmaf(a.weight_decay, w, grad);
     if (a.kind == 0) {
       const float buf = os.first_step ? grad : fmaf(a.momentum, d.m[gbase + i], grad);
       d.m[gbase + i] = buf;

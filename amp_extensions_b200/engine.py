@@ -645,3 +645,58 @@ class Engine:
         with torch.cuda.device(self.device):
             self._check(self.lib.simstep_train_export(self._h, int(what), wp, bp))
         return ws, bs
+
+    # -- MLP value baseline (simstep_baseline_*) ---------------------------------------------
+    def baseline_init(self, sizes, batch_size, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0,
+                      exp_avg=None, exp_avg_sq=None, step=0):
+        """Load the baseline network (widths `sizes` = (obs_dim + 4, hidden..., 1)), its parameters (fp32 [P] in
+        model.parameters() order) and torch.optim.Adam's settings and state (None: a fresh optimiser)."""
+        sizes = [int(s) for s in sizes]
+        dims = (C.c_int32 * len(sizes))(*sizes)
+        vecs = [None if t is None else t.detach().to(self.device, torch.float32).contiguous().reshape(-1)
+                for t in (params, exp_avg, exp_avg_sq)]
+        with torch.cuda.device(self.device):
+            self._check(self.lib.simstep_baseline_init(self._h, len(sizes) - 1, dims, int(batch_size), float(lr),
+                                                       float(betas[0]), float(betas[1]), float(eps),
+                                                       float(weight_decay), *[_ptr(t) for t in vecs], int(step)))
+        self.baseline_n_params = int(vecs[0].numel())
+
+    def baseline_state(self, params=None, exp_avg=None, exp_avg_sq=None, step=None):
+        """Replace the given parts of the baseline's parameters and Adam state (synchronous)."""
+        vecs = [None if t is None else t.detach().to(self.device, torch.float32).contiguous().reshape(-1)
+                for t in (params, exp_avg, exp_avg_sq)]
+        st = None if step is None else C.c_int64(int(step))
+        with torch.cuda.device(self.device):
+            self._check(self.lib.simstep_baseline_state(self._h, 1, *[_ptr(t) for t in vecs], None,
+                                                        None if st is None else C.byref(st)))
+
+    def baseline_read(self):
+        """{params, exp_avg, exp_avg_sq, grad (of the last fit step), step} of the baseline (synchronous)."""
+        out = {k: torch.empty((self.baseline_n_params,), device=self.device, dtype=torch.float32)
+               for k in ("params", "exp_avg", "exp_avg_sq", "grad")}
+        st = C.c_int64(0)
+        with torch.cuda.device(self.device):
+            self._check(self.lib.simstep_baseline_state(self._h, 0, _ptr(out["params"]), _ptr(out["exp_avg"]),
+                                                        _ptr(out["exp_avg_sq"]), _ptr(out["grad"]), C.byref(st)))
+        out["step"] = int(st.value)
+        return out
+
+    def baseline_predict(self, obs, t, out=None):
+        """Baseline values [n] of obs rows [n, obs_dim] (fp32) with path step indices t [n] (int32)."""
+        n = obs.shape[0]
+        self._npg_rows(obs, "obs")
+        self._npg_rows(t, "t", torch.int32)
+        out = torch.empty((n,), device=self.device, dtype=torch.float32) if out is None else out
+        self._check(self.lib.simstep_baseline_predict(self._h, _ptr(obs), _ptr(t), n, _ptr(out), _stream(self.device)))
+        return out
+
+    def baseline_fit(self, obs, t, y, perm, n_steps, restart=True):
+        """Enqueue n_steps Adam steps on the minibatches perm[j*B:(j+1)*B] (int64 row indices into obs / t / y),
+        j continuing from the device cursor (restart: from 0).  Steps past the epoch's n_perm // B - 1 minibatches
+        do nothing.  No host synchronisation."""
+        self._npg_rows(obs, "obs")
+        self._npg_rows(t, "t", torch.int32)
+        self._npg_rows(y, "y")
+        self._npg_rows(perm, "perm", torch.int64)
+        self._check(self.lib.simstep_baseline_fit(self._h, _ptr(obs), _ptr(t), _ptr(y), obs.shape[0], _ptr(perm),
+                                                  perm.numel(), int(n_steps), int(bool(restart)), _stream(self.device)))

@@ -9,6 +9,8 @@ and mjrl/mjrl/algos/batch_reinforce.py:85-170, with the NPG update as an option)
   6. returns, GAE advantages, whitening, rollout statistics        (process_samples.py, batch_reinforce.py:135-141)
   7. with npg_steps > 0: that many rounds of collect -> advantages -> NPG policy step on the device (npg_cg.py,
      DeviceNPG.update)
+  8. with vf_epochs > 0: mjrl's MLPBaseline as the value baseline of the advantages, fitted for that many epochs to
+     the returns after each policy step (batch_reinforce.py:149-160 -> DeviceMLPBaseline); otherwise the baseline is 0
 
 Synthetic offline / expert data stand in for data/offline.pt and data/expert.pt (a download in the reference);
 initial states come from the spin-kick clip without the simulator.  Run:  python examples/milo_iteration.py
@@ -44,7 +46,8 @@ class GaussianMLP:
         self.log_std = torch.full((act_dim,), float(init_log_std))
 
 
-def main(num_envs=512, horizon=40, epochs=3, n_offline=4096, hidden=(128, 128), num_models=4, verbose=True, npg_steps=0):
+def main(num_envs=512, horizon=40, epochs=3, n_offline=4096, hidden=(128, 128), num_models=4, verbose=True, npg_steps=0,
+         vf_epochs=0):
     from amp_extensions_b200 import (AmpDataset, DynamicsEnsemble, ImitationReward, RBFLinearCost, VecSimEnv)
     from amp_extensions_b200.rollout import DeviceRollout
     S, A = 226, 28
@@ -74,8 +77,25 @@ def main(num_envs=512, horizon=40, epochs=3, n_offline=4096, hidden=(128, 128), 
     env.reset()
     batch = ro.collect(horizon, graph=True)
     ret = batch.returns(0.995)                                                          # 6
-    baseline = torch.zeros_like(ret)
-    adv = batch.normalize(batch.advantages(baseline, 0.995, 0.97))
+    vf = None
+    if vf_epochs > 0:                                                                  # 8
+        from amp_extensions_b200.baseline import DeviceMLPBaseline
+
+        class Spec:
+            observation_dim = S
+
+        torch.manual_seed(0)   # nn.Linear's initialisation
+        vf = DeviceMLPBaseline.from_spec(ro, Spec(), epochs=vf_epochs, seed=0)
+
+    def value(batch, ret):
+        return vf.predict_batch(batch) if vf is not None else torch.zeros_like(ret)
+
+    def fit_value(batch, ret):   # after the policy step, as batch_reinforce.py does
+        if vf is not None:
+            before, after = vf.fit_batch(batch, ret, return_errors=True)
+            out["vf_error_before"], out["vf_error_after"] = float(before), float(after)
+
+    adv = batch.normalize(batch.advantages(value(batch, ret), 0.995, 0.97))
     stats = batch.statistics()
     paths = batch.paths(include_partial=False)
     out = dict(train_loss_first=[f[1] for f in fit], train_loss_best=[f[0] for f in fit], threshold=ens.threshold, mmd=mmd,
@@ -89,11 +109,16 @@ def main(num_envs=512, horizon=40, epochs=3, n_offline=4096, hidden=(128, 128), 
         for _ in range(npg_steps):
             res = npg.update(batch, adv)
             out["npg"].append({k: float(v) for k, v in res.items()})
+            fit_value(batch, ret)
             env.reset()
             batch = ro.collect(horizon, graph=True)                                     # replays with the new policy
             ret = batch.returns(0.995)
-            adv = batch.normalize(batch.advantages(torch.zeros_like(ret), 0.995, 0.97))
+            adv = batch.normalize(batch.advantages(value(batch, ret), 0.995, 0.97))
         npg.export_params()
+    else:
+        fit_value(batch, ret)
+    if vf is not None:
+        vf.export()
     if verbose:
         for k, v in out.items():
             print(f"{k:18s} {v}")

@@ -440,6 +440,34 @@ int simstep_train_grads(simstep_handle* h, const float* state_dev, const float* 
                         int32_t batch_rows, double* loss_dev, void* stream);
 int simstep_train_export(simstep_handle* h, int32_t what, float* const* weights_host, float* const* biases_host);
 
+/* ---- MLP value baseline (mjrl/mjrl/baselines/mlp_baseline.py, mjrl/mjrl/utils/optimize_model.py: fit_data) ---- */
+
+/* nn.Sequential of n_layers Linear layers with ReLU between them, widths sizes[0 .. n_layers] = (obs_dim + 4,
+ * hidden..., 1), 1 <= n_layers <= 4, obs_dim in [1, 512], hidden widths in [1, 256].  The input of row i is
+ * [clip(obs_i, -10, 10) / 10, (t_i/1000)^1 .. (t_i/1000)^4] (fp64, rounded to fp32), t_i the int32 step index of
+ * the row within its path; features are formed on the fly, never stored.  The baseline lives in the handle beside
+ * (and independent of) the ensemble, the policy and their training state.
+ *   init:    parameters params_dev [P] fp32 in model.parameters() order (W_0 [out][in], b_0, W_1, ...), and
+ *            Adam(lr, beta1, beta2, eps, weight_decay: L2 term added to the gradient) with its state: first and
+ *            second moments m_dev / v_dev [P] (NULL: zeros) after `step` steps; batch_size in [1, 1024].  Synchronous.
+ *   state:   set != 0: the non-NULL vectors and *step (when step is non-NULL) replace the store's; set == 0: copies
+ *            them (and grad_dev [P], the gradient of the last fit step) out.  Synchronous.
+ *   predict: out_dev [n] fp32 = model(x_i) for rows i < n of obs_dev [n][obs_dim] and t_dev [n].
+ *   fit:     enqueues n_steps Adam steps of fit_data on the minibatches perm_dev[j*B .. (j+1)*B), j = the device
+ *            cursor of the epoch (restart != 0: set to 0 first), each with MSELoss(mean) against y_dev; an epoch
+ *            has n_perm / B - 1 minibatches, and steps past its end are no-ops, so a captured graph can be replayed
+ *            freely.  perm_dev entries index rows of obs_dev / t_dev / y_dev and must lie in [0, n).  No host
+ *            synchronisation. */
+int simstep_baseline_init(simstep_handle* h, int32_t n_layers, const int32_t* sizes, int32_t batch_size, float lr,
+                          float beta1, float beta2, float eps, float weight_decay, const float* params_dev,
+                          const float* m_dev, const float* v_dev, int64_t step);
+int simstep_baseline_state(simstep_handle* h, int32_t set, float* params_dev, float* m_dev, float* v_dev,
+                           float* grad_dev, int64_t* step);
+int simstep_baseline_predict(simstep_handle* h, const float* obs_dev, const int32_t* t_dev, int64_t n, float* out_dev,
+                             void* stream);
+int simstep_baseline_fit(simstep_handle* h, const float* obs_dev, const int32_t* t_dev, const float* y_dev, int64_t n,
+                         const int64_t* perm_dev, int64_t n_perm, int32_t n_steps, int32_t restart, void* stream);
+
 /* ---- reductions used by the multi-GPU host code ------------------------- */
 
 /* counts_dev[b] (int64, bins entries, overwritten) = number of x_dev[i] in [lo, hi] whose bin

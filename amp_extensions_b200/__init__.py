@@ -10,6 +10,7 @@ Host-side mirror of the reference's plugin surface for this one hot path:
   ImitationReward                    (reference DeepMimicCore/scenes/SceneImitate.cpp)
   sampler.get_samples / sample_points (reference milo/milo/sampler.py, batched on the device)
   MLPBaseline / DeviceMLPBaseline     (reference mjrl/mjrl/baselines/mlp_baseline.py)
+  BC / DeviceBC                       (reference mjrl/mjrl/algos/behavior_cloning.py)
 
 All compute goes through libsimstep.so (include/simstep.h); there is no CPU fallback.
 """
@@ -26,6 +27,7 @@ from .imitation import ImitationReward  # noqa: F401
 from .motion import MotionClip  # noqa: F401
 from . import sampler  # noqa: F401
 from .baseline import DeviceMLPBaseline, MLPBaseline  # noqa: F401
+from .bc import BC, DeviceBC  # noqa: F401
 
 
 def register_gym(env_id="simenv-v0"):

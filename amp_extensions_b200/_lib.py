@@ -145,6 +145,15 @@ _SIGNATURES = {
     "simstep_baseline_predict": (C.c_int, [_c_void_p, _c_void_p, _c_void_p, C.c_int64, _c_void_p, _c_void_p]),
     "simstep_baseline_fit": (C.c_int, [_c_void_p, _c_void_p, _c_void_p, _c_void_p, C.c_int64, _c_void_p, C.c_int64,
                                        C.c_int32, C.c_int32, _c_void_p]),
+    "simstep_bc_init": (C.c_int, [_c_void_p, C.c_int32, C.c_int32, C.c_float, C.c_float, C.c_float, C.c_float,
+                                  C.c_float, C.c_float, _c_void_p, _c_void_p, _c_void_p, C.c_int64,
+                                  C.POINTER(C.c_int64)]),
+    "simstep_bc_state": (C.c_int, [_c_void_p, C.c_int32, _c_void_p, _c_void_p, _c_void_p, _c_void_p,
+                                   C.POINTER(C.c_int64)]),
+    "simstep_bc_loss": (C.c_int, [_c_void_p, _c_void_p, _c_void_p, C.c_int64, _c_void_p, _c_void_p]),
+    "simstep_bc_fit": (C.c_int, [_c_void_p, _c_void_p, _c_void_p, C.c_int64, _c_void_p, C.c_int64, C.c_int32,
+                                 C.c_int32, _c_void_p]),
+    "simstep_bc_commit": (C.c_int, [_c_void_p, _c_void_p]),
     "simstep_histogram": (C.c_int, [_c_void_p, _c_void_p, C.c_int64, C.c_double, C.c_double, C.c_int32, _c_void_p,
                                     _c_void_p]),
     "simstep_quantile_op": (C.c_int, [_c_void_p, C.c_int32, _c_void_p, C.c_int64, C.c_int32, _c_void_p, _c_void_p,

@@ -18,6 +18,7 @@
 
 #include "../../include/simstep.h"
 #include "baseline.cuh"
+#include "bc.cuh"
 #include "elementwise.cuh"
 #include "gemm_tcgen05.cuh"
 #include "chain_launch.h"
@@ -90,12 +91,13 @@ struct Layer {
   CUtensorMap tmap_w64;  // the same operand with a 64-row box (column halves of the chain kernel's shared units)
 };
 
-// Per-feature stores (imitation_api.inc, policy_api.inc, train_api.inc, npg_api.inc, baseline_api.inc).
+// Per-feature stores (imitation_api.inc, policy_api.inc, train_api.inc, npg_api.inc, baseline_api.inc, bc_api.inc).
 struct ClipStore;
 struct PolicyStore;
 struct TrainStore;
 struct NpgStore;
 struct BaselineStore;
+struct BcStore;
 
 }  // namespace
 
@@ -157,6 +159,7 @@ struct simstep_handle {
   std::unique_ptr<TrainStore> train;
   std::unique_ptr<NpgStore> npg;
   std::unique_ptr<BaselineStore> baseline;  // value baseline: independent of the ensemble and the policy
+  std::unique_ptr<BcStore> bc;              // behaviour cloning of the policy: dropped by simstep_load_policy
   bool train_raw = false;  // tf32 handle in training: parameters keep all fp32 bits (they are the master copy)
 
   // optional per-category device timing (simstep_profile_*)
@@ -1458,6 +1461,7 @@ int simstep_debug_gemm(int32_t precision, int32_t groups, int64_t m, int32_t n, 
 #include "train_api.inc"
 #include "npg_api.inc"
 #include "baseline_api.inc"
+#include "bc_api.inc"
 
 simstep_handle::~simstep_handle() {
   for (cudaEvent_t e : prof_ev) cudaEventDestroy(e);

@@ -240,32 +240,36 @@ baseline_rows_kernel(const BlNet net, const float* __restrict__ theta, const flo
   }
 }
 
-// grad[p] for every parameter p: dW_l[o][k] = sum_i dz_l[i][o] a_l[i][k] (a_0 = x, a_l = h_{l-1}), db_l[o] =
-// sum_i dz_l[i][o]; rows i = 0 .. B-1 in order, fp64 accumulators.
+// The gradient of parameter p < net.P: dW_l[o][k] = sum_i dz_l[i][o] a_l[i][k] (a_0 = x, a_l = h_{l-1}), db_l[o] =
+// sum_i dz_l[i][o]; rows i = 0 .. B-1 in order, fp64 accumulator.  Shared with the behaviour-cloning step (bc.cuh).
+__device__ inline double bl_param_grad(const BlNet& net, int B, const BlWork& wk, long long p) {
+  int l = 0;
+  while (l + 1 < net.n_lin && p >= net.w_off[l + 1]) ++l;
+  const int din = net.dim[l], dout = net.dim[l + 1];
+  const float* __restrict__ dz = wk.dz[l];
+  double acc = 0.0;
+  if (p < net.b_off[l]) {
+    const long long q = p - net.w_off[l];
+    const int o = static_cast<int>(q / din), k = static_cast<int>(q - static_cast<long long>(o) * din);
+    const float* __restrict__ a = l == 0 ? wk.x : wk.h[l - 1];
+#pragma unroll 16
+    for (int i = 0; i < B; ++i)
+      acc = fma(static_cast<double>(dz[static_cast<long long>(i) * dout + o]), static_cast<double>(a[static_cast<long long>(i) * din + k]), acc);
+  } else {
+    const int o = static_cast<int>(p - net.b_off[l]);
+#pragma unroll 16
+    for (int i = 0; i < B; ++i) acc += static_cast<double>(dz[static_cast<long long>(i) * dout + o]);
+  }
+  return acc;
+}
+
+// grad[p] for every parameter p (bl_param_grad).
 __global__ void __launch_bounds__(256)
 baseline_wgrad_kernel(const BlNet net, const BlCtl* __restrict__ ctl, int B, BlWork wk, float* __restrict__ grad) {
   if (ctl->skip) return;
   for (long long p = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; p < net.P;
-       p += static_cast<long long>(gridDim.x) * blockDim.x) {
-    int l = 0;
-    while (l + 1 < net.n_lin && p >= net.w_off[l + 1]) ++l;
-    const int din = net.dim[l], dout = net.dim[l + 1];
-    const float* __restrict__ dz = wk.dz[l];
-    double acc = 0.0;
-    if (p < net.b_off[l]) {
-      const long long q = p - net.w_off[l];
-      const int o = static_cast<int>(q / din), k = static_cast<int>(q - static_cast<long long>(o) * din);
-      const float* __restrict__ a = l == 0 ? wk.x : wk.h[l - 1];
-#pragma unroll 16
-      for (int i = 0; i < B; ++i)
-        acc = fma(static_cast<double>(dz[static_cast<long long>(i) * dout + o]), static_cast<double>(a[static_cast<long long>(i) * din + k]), acc);
-    } else {
-      const int o = static_cast<int>(p - net.b_off[l]);
-#pragma unroll 16
-      for (int i = 0; i < B; ++i) acc += static_cast<double>(dz[static_cast<long long>(i) * dout + o]);
-    }
-    grad[p] = static_cast<float>(acc);
-  }
+       p += static_cast<long long>(gridDim.x) * blockDim.x)
+    grad[p] = static_cast<float>(bl_param_grad(net, B, wk, p));
 }
 
 }  // namespace simstep

@@ -482,8 +482,16 @@ npg_cg_kernel(int op, const double* __restrict__ sums, int P, double damping, do
   }
 }
 
-// theta (fp32, mjrl flat order) -> pack (transposed weights, biases) and tail std = float(exp(double(log_std)))
-// exactly as simstep_load_policy stores them.  APPLY (x != null) first forms the NPG step:
+// Flat entry i (mjrl order) of value t into the policy: pack_of[i] >= 0 is its place in the pack, else it is
+// log_std[i - ls0] and goes to std[i - ls0] = float(exp(double(t))), exactly as simstep_load_policy stores it.
+__device__ __forceinline__ void policy_store_flat(int i, float t, const int* __restrict__ pack_of, int ls0,
+                                                  float* __restrict__ pack, float* __restrict__ stdv) {
+  if (pack_of[i] >= 0) pack[pack_of[i]] = t;
+  else stdv[i - ls0] = static_cast<float>(exp(static_cast<double>(t)));
+}
+
+// theta (fp32, mjrl flat order) -> pack (transposed weights, biases) and tail std (policy_store_flat).  APPLY
+// (x != null) first forms the NPG step:
 //   alpha = const_lr ? lr : sqrt(|delta / (g.x + 1e-10)|),  theta <- float(theta + alpha x),
 //   log_std <- max(log_std, min_log_std) (MLP.set_param_values), and keeps the previous parameters in old_* for the
 //   diagnostics pass.
@@ -515,8 +523,7 @@ npg_write_kernel(float* __restrict__ theta, const int* __restrict__ pack_of, int
       if (i >= ls0) t = fmaxf(t, min_log_std);
       theta[i] = t;
     }
-    if (pack_of[i] >= 0) pack[pack_of[i]] = t;
-    else tail[tail_std0 + (i - ls0)] = static_cast<float>(exp(static_cast<double>(t)));
+    policy_store_flat(i, t, pack_of, ls0, pack, tail + tail_std0);
   }
   if (x && threadIdx.x == 0) *skip = 0;
 }

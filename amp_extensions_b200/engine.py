@@ -700,3 +700,67 @@ class Engine:
         self._npg_rows(perm, "perm", torch.int64)
         self._check(self.lib.simstep_baseline_fit(self._h, _ptr(obs), _ptr(t), _ptr(y), obs.shape[0], _ptr(perm),
                                                   perm.numel(), int(n_steps), int(bool(restart)), _stream(self.device)))
+
+    # -- behaviour cloning of the loaded policy (simstep_bc_*) --------------------------------
+    BC_LOSS = {"MSE": 0, "MLE": 1}
+
+    def bc_init(self, batch_size, loss_type, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0,
+                min_log_std=-3.0, exp_avg=None, exp_avg_sq=None, step=0):
+        """Allocate the behaviour-cloning state of the loaded policy: parameters (fp32 [P], mjrl's flat order),
+        torch.optim.Adam's settings and state (None: a fresh optimiser), loss_type "MSE" or "MLE".  Returns P."""
+        if loss_type not in self.BC_LOSS:
+            raise ValueError(f"loss_type must be 'MSE' or 'MLE', got {loss_type!r}")
+        vecs = [None if t is None else t.detach().to(self.device, torch.float32).contiguous().reshape(-1)
+                for t in (params, exp_avg, exp_avg_sq)]
+        n = C.c_int64(0)
+        with torch.cuda.device(self.device):
+            self._check(self.lib.simstep_bc_init(self._h, int(batch_size), self.BC_LOSS[loss_type], float(lr),
+                                                 float(betas[0]), float(betas[1]), float(eps), float(weight_decay),
+                                                 float(min_log_std), *[_ptr(t) for t in vecs], int(step), C.byref(n)))
+        self.bc_n_params = int(n.value)
+        if vecs[0].numel() != self.bc_n_params:
+            raise ValueError(f"{vecs[0].numel()} parameters given, the policy has {self.bc_n_params}")
+        return self.bc_n_params
+
+    def bc_state(self, params=None, exp_avg=None, exp_avg_sq=None, step=None):
+        """Replace the given parts of the behaviour-cloning parameters and Adam state (synchronous)."""
+        vecs = [None if t is None else t.detach().to(self.device, torch.float32).contiguous().reshape(-1)
+                for t in (params, exp_avg, exp_avg_sq)]
+        st = None if step is None else C.c_int64(int(step))
+        with torch.cuda.device(self.device):
+            self._check(self.lib.simstep_bc_state(self._h, 1, *[_ptr(t) for t in vecs], None,
+                                                  None if st is None else C.byref(st)))
+
+    def bc_read(self):
+        """{params, exp_avg, exp_avg_sq, grad (of the last fit step), step} of behaviour cloning (synchronous)."""
+        out = {k: torch.empty((self.bc_n_params,), device=self.device, dtype=torch.float32)
+               for k in ("params", "exp_avg", "exp_avg_sq", "grad")}
+        st = C.c_int64(0)
+        with torch.cuda.device(self.device):
+            self._check(self.lib.simstep_bc_state(self._h, 0, _ptr(out["params"]), _ptr(out["exp_avg"]),
+                                                  _ptr(out["exp_avg_sq"]), _ptr(out["grad"]), C.byref(st)))
+        out["step"] = int(st.value)
+        return out
+
+    def bc_loss(self, obs, act, out=None):
+        """{rows, sum of row losses, 0} (CUDA fp64 [3]) of obs [n, obs_dim] / act [n, act_dim] rows (fp32)."""
+        self._npg_rows(obs, "obs")
+        self._npg_rows(act, "act")
+        out = torch.empty((3,), device=self.device, dtype=torch.float64) if out is None else out
+        self._check(self.lib.simstep_bc_loss(self._h, _ptr(obs), _ptr(act), obs.shape[0], _ptr(out),
+                                             _stream(self.device)))
+        return out
+
+    def bc_fit(self, obs, act, idx, n_steps, restart=True):
+        """Enqueue n_steps Adam steps on the minibatches idx[j*B:(j+1)*B] (int64 row indices into obs / act), j
+        continuing from the device cursor (restart: from 0).  Steps past the epoch's idx.numel() // B minibatches do
+        nothing.  No host synchronisation."""
+        self._npg_rows(obs, "obs")
+        self._npg_rows(act, "act")
+        self._npg_rows(idx, "idx", torch.int64)
+        self._check(self.lib.simstep_bc_fit(self._h, _ptr(obs), _ptr(act), obs.shape[0], _ptr(idx), idx.numel(),
+                                            int(n_steps), int(bool(restart)), _stream(self.device)))
+
+    def bc_commit(self):
+        """Write the cloned parameters into the loaded policy in place (and into the NPG state, if any)."""
+        self._check(self.lib.simstep_bc_commit(self._h, _stream(self.device)))

@@ -11,6 +11,8 @@ and mjrl/mjrl/algos/batch_reinforce.py:85-170, with the NPG update as an option)
      DeviceNPG.update)
   8. with vf_epochs > 0: mjrl's MLPBaseline as the value baseline of the advantages, fitted for that many epochs to
      the returns after each policy step (batch_reinforce.py:149-160 -> DeviceMLPBaseline); otherwise the baseline is 0
+  9. with bc_epochs > 0: the policy is warm-started by behaviour cloning on the expert's (s, a) rows for that many
+     epochs before the first rollout, as run.py:195-226 does (mjrl's BC -> DeviceBC)
 
 Synthetic offline / expert data stand in for data/offline.pt and data/expert.pt (a download in the reference);
 initial states come from the spin-kick clip without the simulator.  Run:  python examples/milo_iteration.py
@@ -47,7 +49,7 @@ class GaussianMLP:
 
 
 def main(num_envs=512, horizon=40, epochs=3, n_offline=4096, hidden=(128, 128), num_models=4, verbose=True, npg_steps=0,
-         vf_epochs=0):
+         vf_epochs=0, bc_epochs=0):
     from amp_extensions_b200 import (AmpDataset, DynamicsEnsemble, ImitationReward, RBFLinearCost, VecSimEnv)
     from amp_extensions_b200.rollout import DeviceRollout
     S, A = 226, 28
@@ -70,6 +72,13 @@ def main(num_envs=512, horizon=40, epochs=3, n_offline=4096, hidden=(128, 128), 
     env.reset()
     policy = GaussianMLP(S, A)
     ro = DeviceRollout(env, policy, seed=0)
+    bc_log = {}
+    if bc_epochs > 0:                                                                  # 9
+        from amp_extensions_b200.bc import DeviceBC
+        bc = DeviceBC(ro, policy, expert_paths=[dict(observations=s[:1024].numpy(), actions=a[:1024].numpy())],
+                      epochs=bc_epochs, seed=0)
+        bc.train()                                                                      # the policy object follows
+        bc_log = dict(bc_loss_before=bc.log["loss_before"], bc_loss_after=bc.log["loss_after"])
     batch = ro.collect(horizon)                                                         # 4 (no cost yet: rewards 0)
     pi = torch.cat([batch.observations.reshape(-1, S), batch.next_observations.reshape(-1, S)], dim=1)
     mmd = cost.fit_cost(pi)                                                             # 5
@@ -101,7 +110,7 @@ def main(num_envs=512, horizon=40, epochs=3, n_offline=4096, hidden=(128, 128), 
     out = dict(train_loss_first=[f[1] for f in fit], train_loss_best=[f[0] for f in fit], threshold=ens.threshold, mmd=mmd,
                env_steps=int(batch.rewards.numel()), trajectories=len(stats["ep_len"]), complete_paths=len(paths),
                mean_cost=stats["mean_cost"], adv_mean=float(adv.mean()), adv_std=float(adv.std(unbiased=False)),
-               mean_return=float(ret[0].mean()), expert_cost=float(cost.get_expert_cost()))
+               mean_return=float(ret[0].mean()), expert_cost=float(cost.get_expert_cost()), **bc_log)
     if npg_steps > 0:                                                                  # 7
         from amp_extensions_b200.npg import DeviceNPG
         npg = DeviceNPG(ro, policy)

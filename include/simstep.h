@@ -468,6 +468,42 @@ int simstep_baseline_predict(simstep_handle* h, const float* obs_dev, const int3
 int simstep_baseline_fit(simstep_handle* h, const float* obs_dev, const int32_t* t_dev, const float* y_dev, int64_t n,
                          const int64_t* perm_dev, int64_t n_perm, int32_t n_steps, int32_t restart, void* stream);
 
+/* ---- behaviour cloning of the loaded policy (mjrl/mjrl/algos/behavior_cloning.py: BC.fit) ---- */
+
+/* Minibatch Adam on the policy loaded with simstep_load_policy, against expert (obs, action) rows in device memory.
+ * P and the flat order are simstep_npg_*'s (per layer W [out][in], b [out], then log_std [act]); the policy's
+ * transformations are used as loaded.  simstep_load_policy discards this state; loading an ensemble, a cost or a
+ * baseline leaves it alone.
+ *   init:    loss SIMSTEP_BC_MSE (MSELoss(mean) of the mean against the action; log_std is not trained and its Adam
+ *            moments stay as given) or SIMSTEP_BC_MLE (-mean log-likelihood; log_std is trained, unclamped, with the
+ *            rest), batch_size in [1, 1024], Adam(lr, beta1, beta2, eps, weight_decay: L2 term added to the gradient)
+ *            with its state: parameters params_dev [P] fp32, moments m_dev / v_dev [P] (NULL: zeros) after `step`
+ *            steps.  min_log_std is the clamp of commit.  *n_params_out = P (may be NULL).  Synchronous.
+ *   state:   set != 0: the non-NULL vectors and *step (when step is non-NULL) replace the store's; set == 0: copies
+ *            them (and grad_dev [P], the gradient of the last fit step) out.  Synchronous.
+ *   loss:    out_dev [3] fp64 = { n, sum over rows of the row loss, 0 } for rows 0 .. n-1 of obs_dev [n][obs_dim] and
+ *            act_dev [n][act_dim], with the store's parameters; the row loss is sum_j (mu_j - a_j)^2 (MSE: the loss is
+ *            sum / (n act_dim)) or -LL (MLE: the loss is sum / n).
+ *   fit:     enqueues n_steps Adam steps on the minibatches idx_dev[j*B .. (j+1)*B) (int64 rows in [0, n), repeats
+ *            allowed), j = the device cursor of the epoch (restart != 0: set to 0 first); an epoch has n_idx / B
+ *            minibatches and steps past its end are no-ops, so a captured graph can be replayed freely.  No host
+ *            synchronisation.
+ *   commit:  writes the parameters into the policy in place (log_std clamped at min_log_std first, as
+ *            MLP.set_param_values does; std = float(exp(double(log_std))) as simstep_load_policy stores it), and into
+ *            the NPG state's parameters when there is one.  Graphs that captured simstep_policy_act stay valid. */
+#define SIMSTEP_BC_MSE 0
+#define SIMSTEP_BC_MLE 1
+int simstep_bc_init(simstep_handle* h, int32_t batch_size, int32_t loss_type, float lr, float beta1, float beta2,
+                    float eps, float weight_decay, float min_log_std, const float* params_dev, const float* m_dev,
+                    const float* v_dev, int64_t step, int64_t* n_params_out);
+int simstep_bc_state(simstep_handle* h, int32_t set, float* params_dev, float* m_dev, float* v_dev, float* grad_dev,
+                     int64_t* step);
+int simstep_bc_loss(simstep_handle* h, const float* obs_dev, const float* act_dev, int64_t n, double* out_dev,
+                    void* stream);
+int simstep_bc_fit(simstep_handle* h, const float* obs_dev, const float* act_dev, int64_t n, const int64_t* idx_dev,
+                   int64_t n_idx, int32_t n_steps, int32_t restart, void* stream);
+int simstep_bc_commit(simstep_handle* h, void* stream);
+
 /* ---- reductions used by the multi-GPU host code ------------------------- */
 
 /* counts_dev[b] (int64, bins entries, overwritten) = number of x_dev[i] in [lo, hi] whose bin
